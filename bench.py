@@ -1,9 +1,11 @@
 #!/usr/bin/env python
 """Benchmark of the hot path on BASELINE.json's metric: QMIX train transitions/sec (B=32, T=200) + act-select.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
-One JSON line on stdout (rank 0).  A "step" is one QLearner.train() on one sampled batch of synthetic episodes
+One JSON line on stdout (rank 0).  `--dump-outputs DIR` also writes what the last timed step returned to its caller
+(statistics, gradient, updated parameters) as DIR/<name>.npy; the inputs are seeded, so two builds run with the same
+arguments can be compared output for output.  A "step" is one QLearner.train() on one sampled batch of synthetic episodes
 (SURVEY.md 8d).  `value` = transitions/s with the batch resident in HBM; `e2e` = the same through the public API
 with the batch in pinned HOST memory (H2D copy of the step's inputs + D2H read of the loss inside the timed region).
 Multi-GPU = league sharding: every rank owns an independent learner + replay buffer (weak scaling, no collective
@@ -276,6 +278,8 @@ def run_ours(a, rank, world, device):
     wall = dist_max(wall, world, device)
     ms_per_step = dev_ms / a.steps
     value = world * transitions / (ms_per_step * 1e-3)
+    if a.dump_outputs and rank == 0:                    # before the passes below train the learner further
+        dump_outputs(a.dump_outputs, learner)
 
     # ---------------- per-kernel profile (same steps again, CUDA events around every launch on its own stream)
     peak, peak_src = hbm_peak()
@@ -538,6 +542,22 @@ def run_ours(a, rank, world, device):
             "hbm_kernels": hbm}
     line.update(extra)
     return line
+
+
+def dump_outputs(out_dir, learner):
+    """What QLearner.train() leaves its caller after a step, as float32 .npy files: the logged statistics (mask sum,
+    loss, |td| mean, q_taken mean, target mean, grad norm), the clipped gradient (p.grad) and the updated parameters."""
+    from ma_league_b200 import _native as nat
+    flat = lambda ts: th.cat([t.detach().reshape(-1) for t in ts])      # noqa: E731
+    arrays = {"train_stats": learner.scalars()[nat.SC_MASK_SUM:nat.SC_GRAD_NORM + 1],
+              "grad": flat(p.grad for p in learner.parameters()),
+              "agent_params": flat(learner.mac.parameters())}
+    mixer_params = list(learner.mixer.parameters())                    # VDN has none
+    if mixer_params:
+        arrays["mixer_params"] = flat(mixer_params)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def measure_m1_prime(a, M, learner, buf, B, TT, world, device):
@@ -821,7 +841,11 @@ def main():
     ap.add_argument("--dp-leg", action="store_true", help="run the config-5 leg also at one GPU (its single-GPU step time)")
     ap.add_argument("--dp-steps", dest="dp_steps", type=int, default=10)
     ap.add_argument("--opt", action="append", default=[], help="library switch name=int (mal_set_option), e.g. reduce_tc=0")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     a.warmup = max(a.warmup, 3)
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
