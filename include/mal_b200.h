@@ -12,6 +12,12 @@
  *
  * Fixed model constants of the path: rnn_hidden_dim == MAL_HID (config/default.yaml:45),
  * n_actions <= MAL_MAX_ACTIONS, mixing_embed_dim <= MAL_MAX_EMBED (config/algs/qmix.yaml:21).
+ *
+ * Agent input (basic_controller.py:80-101): the columns of fc1's input are
+ *   [obs | one-hot(a_{t-1}) if obs_last_action | one-hot(agent id) if obs_agent_id]   (config/default.yaml:46-47),
+ * d_in = OBS + A * obs_last_action + N * obs_agent_id.  The learner (mal_learner_cfg_t.agent_input), the fused
+ * act-select (the dense_input argument of mal_agent_step / mal_dqn_step) and the rollout step
+ * (mal_rollout_io_t.agent_input) take the two switches as MAL_IN_* bits; 0 = both on, the reference's default.
  */
 #ifndef MAL_B200_H
 #define MAL_B200_H
@@ -22,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MAL_ABI_VERSION 3
+#define MAL_ABI_VERSION 4
 #define MAL_HID 64
 #define MAL_MAX_ACTIONS 32
 #define MAL_MAX_EMBED 32
@@ -51,6 +57,9 @@ typedef struct mal_batch {
 
 enum { MAL_MIXER_VDN = 0, MAL_MIXER_QMIX2 = 1, MAL_MIXER_QMIX1 = 2 };
 
+/* agent-input switches: a set bit leaves that column block out of fc1's input */
+enum { MAL_IN_NO_LAST_ACTION = 1 /* obs_last_action = False */, MAL_IN_NO_AGENT_ID = 2 /* obs_agent_id = False */ };
+
 /* Hyper-parameters read by QLearner / Learner (marl/learners/q_learner.py:18-24,70,86,104;
  * marl/learners/learner.py:25-31) and QMixer (marl/modules/mixers/qmix.py:12-21). */
 typedef struct mal_learner_cfg {
@@ -66,6 +75,7 @@ typedef struct mal_learner_cfg {
                                          no agent gradient is computed, its grad slice is zero and left out of the clip norm,
                                          and clip + RMSprop skip its parameters and square_avg (only the mixer trains) */
     int32_t agent_kind;               /* MAL_AGENT_RNN (drqn_agent.py) or MAL_AGENT_DQN (dqn_agent.py: fc1 -> ReLU -> fc2) */
+    int32_t agent_input;              /* MAL_IN_* bits (0: obs | last action | agent id); sets d_in and n_agent_params */
 } mal_learner_cfg_t;
 enum { MAL_AGENT_RNN = 0, MAL_AGENT_DQN = 1 };
 
@@ -191,8 +201,10 @@ int mal_agent_step(const float *agent, int32_t rows, int32_t n_agents, int32_t o
                    int32_t dense_input, const float *obs, int64_t obs_sb, const float *last_onehot,
                    int64_t onehot_sb, const float *h_in, float *h_out, float *q, const mal_select_t *sel,
                    void *stream);
-/* dense_input != 0: `obs` is the already assembled agent input [rows, obs_dim] with row stride obs_sb
- * (DRQNAgentNetwork.forward(inputs, hidden_state), drqn_agent.py:29-35); obs_dim is then the full input width. */
+/* dense_input bit 0 set: `obs` is the already assembled agent input [rows, obs_dim] with row stride obs_sb
+ * (DRQNAgentNetwork.forward(inputs, hidden_state), drqn_agent.py:29-35); obs_dim is then the full input width.
+ * Bit 0 clear (fused input assembly): bits 1..2 are the agent-input switches, MAL_IN_* << 1 (last_onehot is not read
+ * when MAL_IN_NO_LAST_ACTION is set).  Other bits are rejected. */
 
 /* The same for the feed-forward DQNAgentNetwork (marl/modules/agents/dqn_agent.py:9-37: q = fc2(relu(fc1(inputs))), the
  * hidden state is passed through untouched); flat parameters fc1.weight | fc1.bias | fc2.weight | fc2.bias. */
@@ -226,9 +238,11 @@ typedef struct mal_rollout_io {
     const float *onehot_tm1; int64_t onehot_tm1_sb;       /* actions_onehot[:, t-1] (agent input), NULL at t == 0 */
     float *reward_tm1; int64_t reward_sb;
     uint8_t *term_tm1; int64_t term_sb;
+    int32_t agent_input;                                  /* MAL_IN_* bits of the agent's input (0: the default layout) */
 } mal_rollout_io_t;
 
-/* `sel` is required (sel->avail / avail_sb are ignored: the environment's avail rows of `io` are used). */
+/* `sel` is required (sel->avail / avail_sb are ignored: the environment's avail rows of `io` are used).
+ * onehot_t is written whatever io->agent_input says (actions_onehot is part of the batch scheme). */
 int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
                      const mal_rollout_io_t *io, const float *h_in, float *h_out, float *q, const mal_select_t *sel,
                      void *stream);

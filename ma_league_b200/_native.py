@@ -14,10 +14,12 @@ import sys
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmal_b200.so")
 SRC = os.path.join(_HERE, "csrc", "mal_b200.cu")
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 MIXER_VDN, MIXER_QMIX2, MIXER_QMIX1 = 0, 1, 2
 AGENT_RNN, AGENT_DQN = 0, 1
+IN_NO_LAST_ACTION, IN_NO_AGENT_ID = 1, 2     # agent-input switches (mal_learner_cfg_t.agent_input, mal_rollout_io_t.agent_input)
+STEP_DENSE = 1                               # dense_input of mal_agent_step / mal_dqn_step: bit 0; bits 1..2 = IN_* << 1
 SC_MASK_SUM, SC_LOSS, SC_TD_ABS, SC_Q_TAKEN, SC_TARGET, SC_GRAD_NORM, SC_MASK_COUNT, SC_STATUS = range(8)
 SC_RAW0 = 8     # raw sums: sum mtd^2, sum |mtd|, sum q_tot*m, sum targets*m, sum m, count
 HID = 64
@@ -43,7 +45,7 @@ class LearnerCfg(C.Structure):
     _fields_ = [("mixer", C.c_int32), ("double_q", C.c_int32), ("embed", C.c_int32), ("hyper_embed", C.c_int32),
                 ("gamma", C.c_float), ("lr", C.c_float), ("alpha", C.c_float), ("eps", C.c_float),
                 ("clip", C.c_float), ("save_q", C.c_int32), ("unnormalized", C.c_int32), ("freeze_agent", C.c_int32),
-                ("agent_kind", C.c_int32)]
+                ("agent_kind", C.c_int32), ("agent_input", C.c_int32)]
 
 
 _PLAN_FIELDS = ["total_bytes", "n_agent_params", "n_mixer_params", "x_on", "x_tg", "gi_on", "gi_tg", "h_on", "h_tg",
@@ -70,7 +72,8 @@ class RolloutIO(C.Structure):
                 ("avail_sb", C.c_int64), ("obs_t", C.c_void_p), ("obs_sb", C.c_int64), ("filled_t", C.c_void_p),
                 ("filled_sb", C.c_int64), ("actions_t", C.c_void_p), ("actions_sb", C.c_int64), ("onehot_t", C.c_void_p),
                 ("onehot_sb", C.c_int64), ("onehot_tm1", C.c_void_p), ("onehot_tm1_sb", C.c_int64),
-                ("reward_tm1", C.c_void_p), ("reward_sb", C.c_int64), ("term_tm1", C.c_void_p), ("term_sb", C.c_int64)]
+                ("reward_tm1", C.c_void_p), ("reward_sb", C.c_int64), ("term_tm1", C.c_void_p), ("term_sb", C.c_int64),
+                ("agent_input", C.c_int32)]
 
 
 class WireLayout(C.Structure):
@@ -204,6 +207,11 @@ def check(rc: int, what: str = ""):
 # ---------------------------------------------------------------------------------------------------------
 # torch <-> ABI helpers (torch is plumbing: device memory + current stream)
 # ---------------------------------------------------------------------------------------------------------
+def agent_input_flags(obs_last_action: bool, obs_agent_id: bool) -> int:
+    """IN_* bits of the agent input [obs | one-hot(a_{t-1}) | one-hot(agent id)] (basic_controller.py:80-101)."""
+    return (0 if obs_last_action else IN_NO_LAST_ACTION) | (0 if obs_agent_id else IN_NO_AGENT_ID)
+
+
 def require_cuda(t, what="tensor"):
     if not t.is_cuda:
         raise MalError("%s must live on a CUDA device: the B200 path has no CPU fallback" % what)

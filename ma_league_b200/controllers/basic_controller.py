@@ -72,6 +72,7 @@ class BasicMAC(MultiAgentController):
         status = th.zeros(1, dtype=th.int32, device=dev) if sel.validate else None
         s, keep = make_select_struct(avail, eps, out[0], out[1], status, u, e)
         io = nat.RolloutIO()
+        io.agent_input = self._input_flags()
         io.state_dim = state.shape[-1]
         io.env_state, io.env_state_sb = state.data_ptr(), state.stride(0)
         io.env_avail, io.env_avail_sb = avail.data_ptr(), avail.stride(0)
@@ -199,8 +200,11 @@ class BasicMAC(MultiAgentController):
     def _fusable(self):
         cls = type(self)
         return (cls._build_inputs is BasicMAC._build_inputs and cls._compute_agent_outputs is BasicMAC._compute_agent_outputs
-                and isinstance(self.agent, (DRQNAgentNetwork, DQNAgentNetwork)) and self.args.obs_last_action
-                and self.args.obs_agent_id and self.agent_output_type == "q")
+                and isinstance(self.agent, (DRQNAgentNetwork, DQNAgentNetwork)) and self.agent_output_type == "q")
+
+    def _input_flags(self):
+        """IN_* bits of the agent input the kernels assemble (obs_last_action / obs_agent_id, basic_controller.py:80-101)."""
+        return nat.agent_input_flags(self.args.obs_last_action, self.args.obs_agent_id)
 
     def _rollout_fusable(self):
         return self._fusable() and isinstance(self.agent, DRQNAgentNetwork)
@@ -214,8 +218,9 @@ class BasicMAC(MultiAgentController):
         if obs_all.stride(3) != 1 or obs_all.stride(2) != OBS or obs_all.dtype != th.float32:
             raise nat.MalError("obs must be float32 with contiguous [N, OBS] rows")
         obs_ptr = obs_all.data_ptr() + 4 * t * obs_all.stride(1)
+        flags = self._input_flags()
         last_ptr, last_sb = None, 0
-        if t > 0:
+        if t > 0 and self.args.obs_last_action:
             oh = ep_batch["actions_onehot"]
             if oh.stride(3) != 1 or oh.stride(2) != A or oh.dtype != th.float32:
                 raise nat.MalError("actions_onehot must be float32 with contiguous [N, A] rows")
@@ -227,7 +232,7 @@ class BasicMAC(MultiAgentController):
             flat = self.agent.flat_params()
             with nat.on_device(dev):
                 nat.check(nat.lib().mal_dqn_step(
-                    flat.data_ptr(), rows, N, OBS, A, 0, obs_ptr, obs_all.stride(0), last_ptr, last_sb, q.data_ptr(),
+                    flat.data_ptr(), rows, N, OBS, A, flags << 1, obs_ptr, obs_all.stride(0), last_ptr, last_sb, q.data_ptr(),
                     C.byref(select_struct) if select_struct is not None else None, nat.current_stream(dev)), "mal_dqn_step")
             return q
         h_in = self.hidden_states
@@ -244,7 +249,7 @@ class BasicMAC(MultiAgentController):
         flat = self.agent.flat_params()
         with nat.on_device(dev):
             nat.check(nat.lib().mal_agent_step(
-                flat.data_ptr(), rows, N, OBS, A, 0, obs_ptr, obs_all.stride(0), last_ptr, last_sb, h_ptr,
+                flat.data_ptr(), rows, N, OBS, A, flags << 1, obs_ptr, obs_all.stride(0), last_ptr, last_sb, h_ptr,
                 h_out.data_ptr(), q.data_ptr(), C.byref(select_struct) if select_struct is not None else None,
                 nat.current_stream(dev)), "mal_agent_step")
         self.hidden_states = h_out

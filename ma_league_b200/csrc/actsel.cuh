@@ -192,6 +192,7 @@ struct AgentStepArgs {
     int kind;                                   // MAL_AGENT_RNN | MAL_AGENT_DQN (feed-forward: no hidden state; stream kernel only)
     int rows, N, OBS, A;
     int dense;                                  // 1: obs is the full [rows, d_in] agent input (row stride obs_sb)
+    AgentInput in;                              // fc1 input columns of the fused input assembly (dense: last = id = 0)
     const float *obs; int64_t obs_sb;
     const float *onehot; int64_t onehot_sb;     // NULL at t == 0
     const float *h_in;                          // NULL -> zeros
@@ -207,8 +208,8 @@ struct AgentStepArgs {
 #define AS_FC1_MAXK 7    // ceil(224 / 32): obs+action columns handled per lane
 __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
     extern __shared__ float as_smem[];
-    const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.A + a.N, a.A);
-    const int Kin = a.dense ? a.OBS : a.OBS + a.A;
+    const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.in.last + a.in.id, a.A);
+    const int Kin = a.dense ? a.OBS : a.OBS + a.in.last;   // [obs | last action]: the agent-id block is a bias gather
     const int ldin = Kin + 1;
     float *in_s = as_smem;                       // [8][ldin]
     float *x_s = in_s + AS_ROWS * ldin;          // [8][64]
@@ -239,7 +240,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
         for (int c = 0; c < AS_FC1_MAXK; ++c) w1[i][c] = (lane + 32 * c < Kin) ? __ldg(w + lane + 32 * c) : 0.0f;
         const int row = r0 + (lane >> 2);
         const int n = row < a.rows ? row % a.N : 0;
-        b1x[i] = __ldg(P + L.fc1_b + j) + (a.dense ? 0.0f : __ldg(w + Kin + n));
+        b1x[i] = __ldg(P + L.fc1_b + j) + (a.in.id ? __ldg(w + Kin + n) : 0.0f);
     }
     float2 w2[MAL_MAX_ACTIONS / AS_WARPS];
     float b2[MAL_MAX_ACTIONS / AS_WARPS];
@@ -407,8 +408,8 @@ __device__ __forceinline__ void load_a_frag(float (&av)[4], const float *W, int6
 
 __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs a) {
     extern __shared__ float as_smem[];
-    const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.A + a.N, a.A);
-    const int Kin = a.dense ? a.OBS : a.OBS + a.A;
+    const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.in.last + a.in.id, a.A);
+    const int Kin = a.dense ? a.OBS : a.OBS + a.in.last;   // [obs | last action]: the agent-id block is a bias gather
     const int ldin = ((Kin + 7) & ~7) + 4;       // zero-padded to whole k-steps; +4: the 8 rows of a B fragment hit different banks
     float *in_s = as_smem;                       // [8][ldin]
     float *x_s = in_s + AS_ROWS * ldin;          // [8][68]
@@ -441,7 +442,7 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
         for (int i = 0; i < 4; ++i) {
             const int j = 16 * warp + g + 8 * (i >> 1), row = r0 + 2 * tig + (i & 1);
             const int n = row < a.rows ? row % a.N : 0;
-            fb[i] = __ldg(P + L.fc1_b + j) + (a.dense ? 0.0f : __ldg(P + L.fc1_w + (int64_t)j * L.d_in + Kin + n));
+            fb[i] = __ldg(P + L.fc1_b + j) + (a.in.id ? __ldg(P + L.fc1_w + (int64_t)j * L.d_in + Kin + n) : 0.0f);
         }
         if (warp < 2) {
 #pragma unroll
@@ -571,9 +572,9 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
 // instead of being parked in 255 registers per thread.
 __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs a) {
     extern __shared__ float as_smem[];
-    const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.A + a.N, a.A, a.kind);
+    const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.in.last + a.in.id, a.A, a.kind);
     const bool rnn = a.kind == MAL_AGENT_RNN;
-    const int Kin = a.dense ? a.OBS : a.OBS + a.A;
+    const int Kin = a.dense ? a.OBS : a.OBS + a.in.last;   // [obs | last action]: the agent-id block is a bias gather
     const int ldin = Kin + 1;
     float *in_s = as_smem;                       // [8][ldin]
     float *x_s = in_s + AS_ROWS * ldin;          // [8][64]
@@ -620,7 +621,7 @@ __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs 
         if ((lane & 3) == 0) {
             int r = lane >> 2, row = r0 + r;
             int n = row < a.rows ? row % a.N : 0;
-            s += __ldg(P + L.fc1_b + j) + (a.dense ? 0.0f : __ldg(w + Kin + n));
+            s += __ldg(P + L.fc1_b + j) + (a.in.id ? __ldg(w + Kin + n) : 0.0f);
             x_s[r * HID + j] = fmaxf(s, 0.0f);
         }
     }

@@ -44,6 +44,10 @@ struct AgentInArgs {
     BatchView bv;
 };
 
+// DEFAULT_IN: the input layout is [obs | last action | agent id] (both switches on), compiled in; otherwise the column
+// bounds come from a.bv.in at run time.  A template parameter rather than a branch: the kernel sits at its register cap
+// (128 at 512 threads), and the default instance keeps the exact code of the fixed layout (DESIGN.md section 4).
+template <bool DEFAULT_IN>
 __global__ void __launch_bounds__(AI_THREADS, 1) k_agent_in_tc(const __grid_constant__ AgentInArgs a) {
     extern __shared__ __align__(1024) uint8_t tc_smem[];
     __shared__ __align__(8) uint64_t mma_bar;
@@ -56,10 +60,12 @@ __global__ void __launch_bounds__(AI_THREADS, 1) k_agent_in_tc(const __grid_cons
     const int n_mtiles = (int)((a.m_end - a.m_begin + TC_M - 1) / TC_M);
     if ((int)blockIdx.x >= n_mtiles) return;
     const BatchView &bv = a.bv;
-    const int K1f = bv.OBS + bv.A;                      // the agent-id columns are a bias gather in the epilogue
+    const int K1f = bv.OBS + (DEFAULT_IN ? bv.A : bv.in.last);   // the agent-id columns are a bias gather in the epilogue
+    const bool has_id = DEFAULT_IN || bv.in.id;
     // A short remainder past the last full 64-column chunk (20v20: 194 = 3 x 64 + 2) would cost a whole extra load / stage /
     // MMA / wait round for a handful of columns: those columns (of the one-hot part) join the agent-id term as rank-1
-    // updates in epilogue 1 instead, and the MMA runs over K1 = the full chunks only
+    // updates in epilogue 1 instead, and the MMA runs over K1 = the full chunks only.  Obs columns never do: without the
+    // last-action block K1f = OBS, and the remainder rule requires K1 >= OBS.
     const int rem1 = (K1f > TC_KC && (K1f % TC_KC) != 0 && (K1f % TC_KC) <= AI_REM_MAX && K1f - (K1f % TC_KC) >= bv.OBS) ? K1f % TC_KC : 0;
     const int K1 = K1f - rem1;
     const int nkc1 = (K1 + TC_KC - 1) / TC_KC;
@@ -244,10 +250,10 @@ __global__ void __launch_bounds__(AI_THREADS, 1) k_agent_in_tc(const __grid_cons
             tmem_ld16_nowait(tl + AI_COL_X2, d2);
             int agent = 0, t_r = 0, b_r = 0;
             if (m < M) { int rr; fast_divmod((int)m, bv.R, invR, t_r, rr); fast_divmod(rr, bv.N, invN, b_r, agent); }
-            const float *wid = P + L.fc1_w + K1f + agent;         // fc1.weight[n, K1f + agent]
+            const float *wid = P + L.fc1_w + K1f + agent;         // fc1.weight[n, K1f + agent] (when has_id)
             float wa[16];
 #pragma unroll
-            for (int e = 0; e < 16; ++e) wa[e] = __ldg(wid + (int64_t)(cgp * 16 + e) * a.d_in);   // in flight under the TMEM load
+            for (int e = 0; e < 16; ++e) wa[e] = has_id ? __ldg(wid + (int64_t)(cgp * 16 + e) * a.d_in) : 0.0f;   // in flight under the TMEM load
             if (rem1 > 0) {                                       // remainder columns K1 .. K1f-1 (one-hot part): x += in[k] W1[n, k]
                 const float *oh = (m < M && t_r > 0) ? field_ptr<float>(bv.onehot, b_r, t_r - 1) + (int64_t)agent * bv.A + (K1 - bv.OBS) : nullptr;
 #pragma unroll

@@ -63,6 +63,7 @@ __global__ void __launch_bounds__(256) k_peer_allreduce_grad(const __grid_consta
 struct BatchView {
     int B, TT, T, N, A, OBS, S, R;
     mal_field_t obs, onehot, state, actions;
+    AgentInput in;        // column layout of the A_AGENT_IN rows
 };
 
 enum { A_DENSE = 0, A_AGENT_IN = 1, A_STATE = 2 };
@@ -93,13 +94,13 @@ __device__ __forceinline__ RowSrc resolve_row(int kind, const BatchView &bv, con
     return r;
 }
 
-// element k of the logical input row; for A_AGENT_IN: [obs | last-action one-hot | agent-id one-hot]
+// element k < d_in of the logical input row; for A_AGENT_IN: [obs | last-action one-hot | agent-id one-hot] (bv.in)
 __device__ __forceinline__ float row_elem(int kind, const BatchView &bv, const RowSrc &r, int k) {
     if (kind != A_AGENT_IN) return r.p0[k];
     if (k < bv.OBS) return r.p0[k];
     k -= bv.OBS;
-    if (k < bv.A) return r.p1 ? r.p1[k] : 0.0f;
-    return (k - bv.A) == r.agent ? 1.0f : 0.0f;
+    if (k < bv.in.last) return r.p1 ? r.p1[k] : 0.0f;
+    return (k - bv.in.last) == r.agent ? 1.0f : 0.0f;
 }
 
 // =============================================================================================
@@ -308,7 +309,7 @@ __global__ void __launch_bounds__(256) k_reduce_group(const __grid_constant__ Re
                 const float *ap = field_ptr<float>(bv.state, b, t + p.shift) + k0;
                 ra[2 * u] = (ok && k_ok0) ? __ldg(ap + c0) : 0.0f;
                 ra[2 * u + 1] = (ok && k_ok1) ? __ldg(ap + c1) : 0.0f;
-            } else {   // [obs | last-action one-hot | agent-id one-hot]
+            } else {   // [obs | last-action one-hot | agent-id one-hot], bounds from bv.in (K = d_in)
                 const int t = (int)((unsigned)m / (unsigned)bv.R), rr = (int)m - t * bv.R;   // rows < 2^31 (host-checked): 32-bit division
                 const int b = rr / bv.N, n = rr - b * bv.N;
                 const float *po = field_ptr<float>(bv.obs, b, t) + (int64_t)n * bv.OBS;
@@ -319,8 +320,8 @@ __global__ void __launch_bounds__(256) k_reduce_group(const __grid_constant__ Re
                     float v = 0.0f;
                     if (ok && k < p.K) {
                         if (k < bv.OBS) v = __ldg(po + k);
-                        else if (k < bv.OBS + bv.A) v = t > 0 ? __ldg(ph + (k - bv.OBS)) : 0.0f;
-                        else v = (k - bv.OBS - bv.A) == n ? 1.0f : 0.0f;
+                        else if (k < bv.OBS + bv.in.last) v = t > 0 ? __ldg(ph + (k - bv.OBS)) : 0.0f;
+                        else v = (k - bv.OBS - bv.in.last) == n ? 1.0f : 0.0f;
                     }
                     ra[2 * u + h] = v;
                 }

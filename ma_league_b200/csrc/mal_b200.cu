@@ -382,7 +382,8 @@ extern "C" int mal_eps_greedy_select(const float *q, int64_t q_ld, int32_t rows,
 }
 
 static thread_local int g_actsel_lat = 1;    // 1: mma.sync latency kernel for rollout-sized launches; 0: lanes-along-k register kernel
-static int launch_agent_step(AgentStepArgs &a, int Kin, cudaStream_t stream) {
+static int launch_agent_step(AgentStepArgs &a, cudaStream_t stream) {
+    const int Kin = a.in.last_end();
     const size_t smem = sizeof(float) * (size_t)(AS_ROWS * (Kin + 1) + AS_ROWS * HID * 3 + AS_ROWS * 2 * G3 + AS_ROWS * 32);
     MAL_REQUIRE(smem <= 200 * 1024 && Kin <= 32 * AS_FC1_MAXK, "mal_agent_step: input width %d too large (max %d)", Kin,
                 32 * AS_FC1_MAXK);
@@ -410,6 +411,17 @@ static int launch_agent_step(AgentStepArgs &a, int Kin, cudaStream_t stream) {
     return 0;
 }
 
+// dense_input of mal_agent_step / mal_dqn_step: bit 0 = the caller assembled the input (obs_dim columns, nothing to
+// gather); otherwise bits 1..2 are the MAL_IN_* switches of the fused input assembly
+static int step_input(int32_t dense_input, AgentStepArgs *a) {
+    MAL_REQUIRE((dense_input & ~7) == 0 && !((dense_input & 1) && (dense_input >> 1)),
+                "dense_input %d: bit 0 (dense) or the agent-input bits 1..2, nothing else", dense_input);
+    a->dense = dense_input & 1;
+    if (a->dense) { a->in.obs = a->in.d_in = a->OBS; a->in.last = a->in.id = 0; }
+    else a->in = agent_input(a->OBS, a->A, a->N, dense_input >> 1);
+    return 0;
+}
+
 extern "C" int mal_agent_step(const float *agent, int32_t rows, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
                               int32_t dense_input, const float *obs, int64_t obs_sb, const float *last_onehot,
                               int64_t onehot_sb, const float *h_in, float *h_out, float *q, const mal_select_t *sel,
@@ -420,11 +432,11 @@ extern "C" int mal_agent_step(const float *agent, int32_t rows, int32_t n_agents
     AgentStepArgs a;
     memset(&a, 0, sizeof(a));
     a.params = agent; a.rows = rows; a.N = n_agents; a.OBS = obs_dim; a.A = n_actions;
-    a.dense = dense_input ? 1 : 0;
-    a.obs = obs; a.obs_sb = obs_sb; a.onehot = dense_input ? nullptr : last_onehot; a.onehot_sb = onehot_sb;
+    if (int rc = step_input(dense_input, &a)) return rc;
+    a.obs = obs; a.obs_sb = obs_sb; a.onehot = a.in.last > 0 ? last_onehot : nullptr; a.onehot_sb = onehot_sb;
     a.h_in = h_in; a.h_out = h_out; a.q = q; a.do_select = sel ? 1 : 0;
     if (sel) if (int rc = fill_select(sel, rows, n_agents, n_actions, &a.sel)) return rc;
-    return launch_agent_step(a, dense_input ? obs_dim : obs_dim + n_actions, (cudaStream_t)stream);
+    return launch_agent_step(a, (cudaStream_t)stream);
 }
 
 // DQNAgentNetwork.forward (dqn_agent.py:34-37: q = fc2(relu(fc1(inputs))), no hidden state) through BasicMAC's input
@@ -438,11 +450,11 @@ extern "C" int mal_dqn_step(const float *agent, int32_t rows, int32_t n_agents, 
     AgentStepArgs a;
     memset(&a, 0, sizeof(a));
     a.params = agent; a.kind = MAL_AGENT_DQN; a.rows = rows; a.N = n_agents; a.OBS = obs_dim; a.A = n_actions;
-    a.dense = dense_input ? 1 : 0;
-    a.obs = obs; a.obs_sb = obs_sb; a.onehot = dense_input ? nullptr : last_onehot; a.onehot_sb = onehot_sb;
+    if (int rc = step_input(dense_input, &a)) return rc;
+    a.obs = obs; a.obs_sb = obs_sb; a.onehot = a.in.last > 0 ? last_onehot : nullptr; a.onehot_sb = onehot_sb;
     a.h_in = nullptr; a.h_out = nullptr; a.q = q; a.do_select = sel ? 1 : 0;
     if (sel) if (int rc = fill_select(sel, rows, n_agents, n_actions, &a.sel)) return rc;
-    return launch_agent_step(a, dense_input ? obs_dim : obs_dim + n_actions, (cudaStream_t)stream);
+    return launch_agent_step(a, (cudaStream_t)stream);
 }
 
 extern "C" int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
@@ -454,10 +466,12 @@ extern "C" int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents
     MAL_REQUIRE(io->env_state && io->env_avail && io->env_obs && io->state_t && io->avail_t && io->obs_t && io->filled_t &&
                     io->actions_t && io->onehot_t, "mal_rollout_step: environment / batch pointers missing");
     MAL_REQUIRE(!io->prev_reward || (io->prev_done && io->reward_tm1 && io->term_tm1), "mal_rollout_step: previous-step fields missing");
+    MAL_REQUIRE((io->agent_input & ~3) == 0, "mal_rollout_step: unknown agent_input bits %d", io->agent_input);
     AgentStepArgs a;
     memset(&a, 0, sizeof(a));
     const int rows = bs * n_agents;
     a.params = agent; a.rows = rows; a.N = n_agents; a.OBS = obs_dim; a.A = n_actions; a.dense = 0;
+    a.in = agent_input(obs_dim, n_actions, n_agents, io->agent_input);
     a.obs = io->env_obs; a.obs_sb = io->env_obs_sb; a.onehot = io->onehot_tm1; a.onehot_sb = io->onehot_tm1_sb;
     a.h_in = h_in; a.h_out = h_out; a.q = q; a.do_select = 1;
     mal_select_t s2 = *sel;
@@ -471,7 +485,7 @@ extern "C" int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents
     r.obs_t = io->obs_t; r.obs_sb = io->obs_sb; r.filled_t = (long long *)io->filled_t; r.filled_sb = io->filled_sb;
     r.actions_t = (long long *)io->actions_t; r.actions_sb = io->actions_sb; r.onehot_t = io->onehot_t; r.onehot_sb = io->onehot_sb;
     r.reward_tm1 = io->reward_tm1; r.reward_sb = io->reward_sb; r.term_tm1 = io->term_tm1; r.term_sb = io->term_sb;
-    return launch_agent_step(a, obs_dim + n_actions, (cudaStream_t)stream);
+    return launch_agent_step(a, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -479,6 +493,7 @@ extern "C" int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents
 // ---------------------------------------------------------------------------------------------
 struct Dims {
     int B, TT, T, N, A, OBS, S, R, E, HE, d_in, mixer, two, kind;
+    AgentInput in;                  // fc1 input layout (d_in = in.d_in)
     int64_t M1, BT;
     int ld1, ld2;
 };
@@ -493,7 +508,9 @@ static int get_dims(const mal_batch_t *b, const mal_learner_cfg_t *c, Dims *d) {
     d->B = b->B; d->TT = b->TT; d->T = b->TT - 1; d->N = b->N; d->A = b->A; d->OBS = b->OBS; d->S = b->S;
     MAL_REQUIRE(c->agent_kind == MAL_AGENT_RNN || c->agent_kind == MAL_AGENT_DQN, "agent kind %d not recognised", c->agent_kind);
     d->kind = c->agent_kind;
-    d->R = b->B * b->N; d->d_in = b->OBS + b->A + b->N; d->mixer = c->mixer;
+    MAL_REQUIRE((c->agent_input & ~3) == 0, "agent_input %d: only MAL_IN_NO_LAST_ACTION | MAL_IN_NO_AGENT_ID", c->agent_input);
+    d->in = agent_input(b->OBS, b->A, b->N, c->agent_input);
+    d->R = b->B * b->N; d->d_in = d->in.d_in; d->mixer = c->mixer;
     d->E = c->embed; d->HE = c->hyper_embed; d->two = (c->mixer == MAL_MIXER_QMIX2);
     if (c->mixer != MAL_MIXER_VDN) {
         MAL_REQUIRE(d->E >= 1 && d->E <= MAL_MAX_EMBED, "mixing_embed_dim must be in [1, %d]", MAL_MAX_EMBED);
@@ -637,6 +654,7 @@ static BatchView make_view(const mal_batch_t *b, const Dims &d) {
     BatchView v;
     v.B = d.B; v.TT = d.TT; v.T = d.T; v.N = d.N; v.A = d.A; v.OBS = d.OBS; v.S = d.S; v.R = d.R;
     v.obs = b->obs; v.onehot = b->onehot; v.state = b->state; v.actions = b->actions;
+    v.in = d.in;
     return v;
 }
 
@@ -759,7 +777,8 @@ static int launch_linear_tc(const LinGroup &g0, int64_t maxM, cudaStream_t st, c
     }
     const int64_t tiles = ceil_div64(maxM, TC_M);
     const int ak = dense ? TCA_VEC_DENSE : (state ? TCA_VEC_STATE : TCA_GENERIC);
-    bool agent_vec = ek == TCE_FC1 && maxM < (1 << 24);   // float4 loads over the obs part of the fc1 input rows
+    // float4 loads over the obs part of the fc1 input rows (TCE_BIAS_ACT: an input without the agent-id block)
+    bool agent_vec = (ek == TCE_FC1 || ek == TCE_BIAS_ACT) && maxM < (1 << 24);
     for (int i = 0; i < g.n; ++i)
         agent_vec = agent_vec && g.p[i].a_kind == A_AGENT_IN && (g.bv.OBS & 3) == 0 && (g.bv.obs.sb & 3) == 0 &&
             (g.bv.obs.st & 3) == 0 && aligned16(g.bv.obs.ptr);
@@ -775,7 +794,8 @@ static int launch_linear_tc(const LinGroup &g0, int64_t maxM, cudaStream_t st, c
         if (ak == TCA_VEC_DENSE && ek == TCE_BIAS_ACT) return launch_tc2_inst<TCA_VEC_DENSE, TCE_BIAS_ACT>(g, grid1, st, tag, g_next_pdl);
         if (ak == TCA_VEC_DENSE && ek == TCE_MASKPOS) return launch_tc2_inst<TCA_VEC_DENSE, TCE_MASKPOS>(g, grid1, st, tag, g_next_pdl);
         if (ak == TCA_VEC_STATE && ek == TCE_BIAS_ACT) return launch_tc2_inst<TCA_VEC_STATE, TCE_BIAS_ACT>(g, grid1, st, tag, g_next_pdl);
-        if (agent_vec) return launch_tc2_inst<TCA_AGENT, TCE_FC1>(g, grid1, st, tag, g_next_pdl);
+        if (agent_vec) return ek == TCE_FC1 ? launch_tc2_inst<TCA_AGENT, TCE_FC1>(g, grid1, st, tag, g_next_pdl)
+                                            : launch_tc2_inst<TCA_AGENT, TCE_BIAS_ACT>(g, grid1, st, tag, g_next_pdl);
         if (ek == TCE_FC1) return launch_tc2_inst<TCA_GENERIC, TCE_FC1>(g, grid1, st, tag, g_next_pdl);
         if (ek == TCE_MASKPOS) return launch_tc2_inst<TCA_GENERIC, TCE_MASKPOS>(g, grid1, st, tag, g_next_pdl);
         return launch_tc2_inst<TCA_GENERIC, TCE_BIAS_ACT>(g, grid1, st, tag, g_next_pdl);
@@ -785,7 +805,8 @@ static int launch_linear_tc(const LinGroup &g0, int64_t maxM, cudaStream_t st, c
     if (ak == TCA_VEC_DENSE && ek == TCE_BIAS_ACT) return launch_tc_inst<TCA_VEC_DENSE, TCE_BIAS_ACT>(g, grid, st, tag, g_next_pdl);
     if (ak == TCA_VEC_DENSE && ek == TCE_MASKPOS) return launch_tc_inst<TCA_VEC_DENSE, TCE_MASKPOS>(g, grid, st, tag, g_next_pdl);
     if (ak == TCA_VEC_STATE && ek == TCE_BIAS_ACT) return launch_tc_inst<TCA_VEC_STATE, TCE_BIAS_ACT>(g, grid, st, tag, g_next_pdl);
-    if (agent_vec) return launch_tc_inst<TCA_AGENT, TCE_FC1>(g, grid, st, tag, g_next_pdl);
+    // (no TCA_AGENT instance with the plain epilogue here: at the two-CTA register cap it spills; the generic loader serves)
+    if (agent_vec && ek == TCE_FC1) return launch_tc_inst<TCA_AGENT, TCE_FC1>(g, grid, st, tag, g_next_pdl);
     if (ek == TCE_FC1) return launch_tc_inst<TCA_GENERIC, TCE_FC1>(g, grid, st, tag, g_next_pdl);
     if (ek == TCE_MASKPOS) return launch_tc_inst<TCA_GENERIC, TCE_MASKPOS>(g, grid, st, tag, g_next_pdl);
     return launch_tc_inst<TCA_GENERIC, TCE_BIAS_ACT>(g, grid, st, tag, g_next_pdl);
@@ -933,9 +954,10 @@ extern "C" int mal_learner_forward(const mal_batch_t *batch, const mal_learner_c
     // tensor-core recurrence (k_gru_fwd_tc) for large row counts: gi then leaves k_agent_in_tc in the tiled layout
     const bool rec_tc = rec_tc_selected(d, bv);
     if (fused_in) {
-        const size_t ai_smem = ai_smem_bytes(bv.OBS + bv.A);
-        static size_t attr[MAL_MAX_DEV];
-        if (int rc = ensure_dyn_smem(k_agent_in_tc, ai_smem, attr)) return rc;
+        const size_t ai_smem = ai_smem_bytes(d.in.last_end());
+        const bool default_in = d.in.last == d.A && d.in.id;
+        static size_t attr[MAL_MAX_DEV], attr_g[MAL_MAX_DEV];
+        if (int rc = default_in ? ensure_dyn_smem(k_agent_in_tc<true>, ai_smem, attr) : ensure_dyn_smem(k_agent_in_tc<false>, ai_smem, attr_g)) return rc;
         ++g_stat_agent_in_fused;
         auto launch_in = [&](int tb, int te, cudaStream_t s_) -> int {
             AgentInArgs a;
@@ -945,7 +967,11 @@ extern "C" int mal_learner_forward(const mal_batch_t *batch, const mal_learner_c
             const int64_t tiles = ceil_div64(a.m_end - a.m_begin, TC_M);
             int64_t per = sms / 2; if (per < 1) per = 1;
             dim3 grid((unsigned)(tiles < per ? tiles : per), 2);
-            { ProfScope _ps("k_agent_in_tc", s_); k_agent_in_tc<<<grid, AI_THREADS, ai_smem, s_>>>(a); }
+            {
+                ProfScope _ps("k_agent_in_tc", s_);
+                if (default_in) k_agent_in_tc<true><<<grid, AI_THREADS, ai_smem, s_>>>(a);
+                else k_agent_in_tc<false><<<grid, AI_THREADS, ai_smem, s_>>>(a);
+            }
             MAL_LAUNCH_CHECK("k_agent_in_tc");
             return 0;
         };
@@ -958,9 +984,9 @@ extern "C" int mal_learner_forward(const mal_batch_t *batch, const mal_learner_c
     {
         LinGroup g; g.n = 2; g.bv = bv;
         for (int net = 0; net < 2; ++net)
-            g.p[net] = lin(d.M1, d.OBS + d.A, HID, A_AGENT_IN, 0, nullptr, 0, ap[net] + AL.fc1_w, d.d_in, 0,
-                           ap[net] + AL.fc1_b, EPI_FC1, nullptr, 0, dqn ? hh[net] : x[net], HID);   // DQN: the "hidden state" IS relu(fc1)
-        if (int rc = launch_linear(g, d.M1, d.OBS + d.A, st, "k_linear_group:fc1")) return rc;
+            g.p[net] = lin(d.M1, d.in.last_end(), HID, A_AGENT_IN, 0, nullptr, 0, ap[net] + AL.fc1_w, d.d_in, 0, ap[net] + AL.fc1_b,
+                           d.in.id ? EPI_FC1 : EPI_RELU, nullptr, 0, dqn ? hh[net] : x[net], HID);   // DQN: the "hidden state" IS relu(fc1)
+        if (int rc = launch_linear(g, d.M1, d.in.last_end(), st, "k_linear_group:fc1")) return rc;
     }
     // gi = W_ih x + b_ih
     if (!dqn) {

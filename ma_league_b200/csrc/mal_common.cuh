@@ -70,6 +70,27 @@ __host__ __device__ inline AgentLayout agent_layout(int d_in, int n_actions, int
     return L;
 }
 
+// Column layout of fc1's input, basic_controller.py:80-101:  [obs | one-hot(a_{t-1}) | one-hot(agent id)], the last two
+// blocks switched by obs_last_action / obs_agent_id.  Every loader and epilogue that touches fc1's input takes its
+// column bounds from here: obs columns [0, obs), last-action columns [obs, obs + last), agent-id columns
+// [obs + last, d_in).  The blocks are given as widths so that the kernels keep the arithmetic of the fixed layout, with
+// `last` / `id` where they read n_actions / n_agents.
+struct AgentInput {
+    int obs;        // OBS
+    int last;       // width of the last-action block: A * obs_last_action
+    int id;         // width of the agent-id block: N * obs_agent_id
+    int d_in;       // fc1 input width, obs + last + id
+    __host__ __device__ int last_end() const { return obs + last; }
+};
+__host__ __device__ inline AgentInput agent_input(int OBS, int A, int N, int flags) {   // flags: MAL_IN_* bits
+    AgentInput in;
+    in.obs = OBS;
+    in.last = (flags & MAL_IN_NO_LAST_ACTION) ? 0 : A;
+    in.id = (flags & MAL_IN_NO_AGENT_ID) ? 0 : N;
+    in.d_in = OBS + in.last + in.id;
+    return in;
+}
+
 struct MixerLayout {   // qmix.py:16-39 (layers == 2: Linear-ReLU-Linear hypernets; == 1: single Linear)
     int S, N, E, HE, layers;
     int64_t w1a_w, w1a_b, w1b_w, w1b_b;   // hyper_w_1.{0,2}  (layers==1: only w1b = hyper_w_1, K = S)

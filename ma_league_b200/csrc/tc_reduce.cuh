@@ -246,8 +246,8 @@ __global__ void __launch_bounds__(256, 1) k_reduce_tc(const __grid_constant__ Re
                 for (int e = 0; e < 4; ++e) {
                     const int kk = k + e;
                     if (kk < bv.OBS) cp_async4(dst + 4 * e, ob + kk);
-                    else if (kk < bv.OBS + bv.A) cp_async4(dst + 4 * e, oh ? oh + (kk - bv.OBS) : p.dY, oh ? 4 : 0);
-                    else *reinterpret_cast<float *>(dst + 4 * e) = (kk < p.K && kk - bv.OBS - bv.A == n) ? 1.0f : 0.0f;   // computed, not loaded
+                    else if (kk < bv.OBS + bv.in.last) cp_async4(dst + 4 * e, oh ? oh + (kk - bv.OBS) : p.dY, oh ? 4 : 0);
+                    else *reinterpret_cast<float *>(dst + 4 * e) = (kk < p.K && kk - bv.OBS - bv.in.last == n) ? 1.0f : 0.0f;   // computed, not loaded
                 }
             }
         };
@@ -600,8 +600,8 @@ __global__ void __launch_bounds__(RT3_THREADS, 1) k_reduce_tc3(const __grid_cons
                 float *d = reinterpret_cast<float *>(dst + 4 * e);
                 if (kk >= p.K) *d = 0.0f;
                 else if (AK != A_AGENT_IN || kk < bv.OBS) cp_async4_plain(d, src + kk);
-                else if (kk < bv.OBS + bv.A) { if (oh) cp_async4_plain(d, oh + (kk - bv.OBS)); else *d = 0.0f; }
-                else *d = (kk - bv.OBS - bv.A == agent) ? 1.0f : 0.0f;               // agent-id one-hot: computed, not loaded
+                else if (kk < bv.OBS + bv.in.last) { if (oh) cp_async4_plain(d, oh + (kk - bv.OBS)); else *d = 0.0f; }
+                else *d = (kk - bv.OBS - bv.in.last == agent) ? 1.0f : 0.0f;         // agent-id one-hot: computed, not loaded
             }
         } else zero16(dst);
     };
@@ -970,7 +970,7 @@ __global__ void __launch_bounds__(RT3_THREADS, 1) k_reduce_fc1(const __grid_cons
     const uint32_t tmem_base = tmem_base_s;
 
     // ---- this thread's pieces of a block: row `warp`; input pieces `lane` and `lane + 32`, d_x piece `lane` (lanes 0-15)
-    const int KA = bv.OBS + bv.A;                        // first agent-id column
+    const int KA = bv.OBS + bv.in.last;                  // first agent-id column (columns < d_in only)
     const bool obs_vec = (bv.OBS & 3) == 0 && (bv.obs.sb & 3) == 0 && (bv.obs.st & 3) == 0 && ((reinterpret_cast<uintptr_t>(bv.obs.ptr) & 15) == 0);
     uint32_t off_in[2];
     int col_in[2], cls_in[2];                            // class 0: zero, 1: one 16-byte copy from the obs row, 2: element-wise

@@ -78,7 +78,8 @@ class QLearner(Learner):
         return nat.LearnerCfg(self._mixer_kind(), int(bool(a.double_q)), self.mixer.embed_dim if qm else 0,
                               self.mixer.hypernet_embed if qm else 0, a.gamma, a.lr, a.optim_alpha, a.optim_eps,
                               a.grad_norm_clip, int(self.save_q), int(self._dp_world() > 1), int(self._agent_frozen()),
-                              getattr(self.mac.agent, "mal_kind", nat.AGENT_RNN))
+                              getattr(self.mac.agent, "mal_kind", nat.AGENT_RNN),
+                              nat.agent_input_flags(getattr(a, "obs_last_action", True), getattr(a, "obs_agent_id", True)))
 
     def _agent_frozen(self):
         """`freeze_agent_weights()` (multi_agent_controller.py:74-76, `args.freeze_native`): in the reference a frozen
