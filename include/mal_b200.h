@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MAL_ABI_VERSION 4
+#define MAL_ABI_VERSION 5
 #define MAL_HID 64
 #define MAL_MAX_ACTIONS 32
 #define MAL_MAX_EMBED 32
@@ -55,7 +55,9 @@ typedef struct mal_batch {
     mal_field_t filled;               /* i64 [B,TT,1] */
 } mal_batch_t;
 
-enum { MAL_MIXER_VDN = 0, MAL_MIXER_QMIX2 = 1, MAL_MIXER_QMIX1 = 2 };
+/* MAL_MIXER_NONE: independent Q-learners (IQL, `mixer: None`): no mixing network, every agent has its own TD error
+ * against the transition's reward and the [B,T] mask broadcast over agents (q_learner.py:81-98 with self.mixer = None). */
+enum { MAL_MIXER_VDN = 0, MAL_MIXER_QMIX2 = 1, MAL_MIXER_QMIX1 = 2, MAL_MIXER_NONE = 3 };
 
 /* agent-input switches: a set bit leaves that column block out of fc1's input */
 enum { MAL_IN_NO_LAST_ACTION = 1 /* obs_last_action = False */, MAL_IN_NO_AGENT_ID = 2 /* obs_agent_id = False */ };
@@ -80,7 +82,9 @@ typedef struct mal_learner_cfg {
 enum { MAL_AGENT_RNN = 0, MAL_AGENT_DQN = 1 };
 
 /* Byte offsets of every intermediate inside the caller-owned workspace (filled by mal_learner_plan).
- * Row index of the [TT*R, .] arrays is m = t*R + b*N + n; of the [B*T, .] arrays m = b*T + t. */
+ * Row index of the [TT*R, .] arrays is m = t*R + b*N + n; of the [B*T, .] arrays m = b*T + t.
+ * MAL_MIXER_NONE: n_mixer_params = 0, y1 / a2 / d_a2 / d_y1 are empty and q_tot / target_q_tot / targets / td hold
+ * [B,T,N] (one TD error per agent); mask stays [B,T]. */
 typedef struct mal_plan {
     int64_t total_bytes;
     int64_t n_agent_params, n_mixer_params;
@@ -94,7 +98,7 @@ typedef struct mal_plan {
     int64_t mask;                     /* f32 [B,T] */
     int64_t y1_on, y1_tg;             /* f32 [B*T, 2*HE+2*E]  h1|hf|b1|v1 */
     int64_t a2_on, a2_tg;             /* f32 [B*T, E*N+E]     a1|af (pre-abs) */
-    int64_t q_tot, target_q_tot, targets, td;   /* f32 [B*T] */
+    int64_t q_tot, target_q_tot, targets, td;   /* f32 [B*T] ([B*T*N] for MAL_MIXER_NONE: chosen / target_max per agent) */
     int64_t d_a2, d_y1;               /* f32 like a2 / y1 */
     int64_t d_chosen;                 /* f32 [B,T,N] */
     int64_t d_g;                      /* f32 [TT*R,256]  d(gi_r)|d(gi_z)|d(gi_n)|d(gh_n) */
@@ -139,7 +143,11 @@ int mal_learner_plan(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, mal
 
 /* QLearner.train forward half, marl/learners/q_learner.py:36-98: unroll of the online and target
  * RNN agents, chosen-action gather, masked (double-Q) target max, mixers, TD error, masked loss.
- * Parameters are flat fp32 buffers in state_dict order. Results land in the workspace (plan offsets). */
+ * Parameters are flat fp32 buffers in state_dict order. Results land in the workspace (plan offsets).
+ * mixer / target_mixer may be NULL for MAL_MIXER_VDN and MAL_MIXER_NONE (no mixer parameters).
+ * MAL_MIXER_NONE: the loss normaliser and every statistic use the mask expanded to [B,T,N] (q_learner.py:92,117-124):
+ * scalars[MAL_SC_MASK_SUM] = N * mask.sum(), MAL_SC_MASK_COUNT counts N per live transition, and q_taken / target means
+ * divide by that sum times N, as the reference's lines do. */
 int mal_learner_forward(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
                         const float *agent, const float *target_agent, const float *mixer,
                         const float *target_mixer, void *workspace, void *stream);
@@ -249,7 +257,8 @@ int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents, int32_t o
 
 /* Launch counters per kernel flavour since process start, for tests that assert which variant the launch heuristics
  * picked: "linear_tc2" (pipelined tcgen05 GEMM), "linear_tc", "reduce_tc", "reduce_tc_swap", "reduce_ffma",
- * "agent_in_fused".  Unknown names return 0. */
+ * "agent_in_fused", "rec_tc", "rec_tc_bwd", "reduce_fc1", "gru_balanced" (forward recurrence as 2 x SMs equal workers).
+ * Unknown names return 0. */
 uint64_t mal_stat(const char *name);
 
 /* Library options (experiment switches; the defaults are the measured best).  They are PER CALLING THREAD, like the
@@ -263,7 +272,7 @@ uint64_t mal_stat(const char *name);
  *   "pdl"           1 (default): programmatic dependent launch along the main kernel chain; 0: full serialisation
  *   "time_chunks"   1 (default) / 2: time-chunked forward (input projection of the 2nd half beside the 1st half's recurrence)
  *   "gru_balance"   a forward recurrence of more than 2 and at most 3 chains per SM can run as 2 x SMs equal workers (a chain
- *                   may change workers once): 1 (default) when nothing runs beside it (VDN), 2 always, 0 never
+ *                   may change workers once): 1 (default) when nothing runs beside it (VDN, no mixer), 2 always, 0 never
  *   "rec_carveout"  bit 0 / bit 1 (default 2 = backward only): the forward / backward recurrence kernel prefers the largest shared-memory
  *                   carve-out, so that the tcgen05 GEMMs of the side streams can be resident beside it (an SM keeps its L1 /
  *                   shared split while CTAs are resident); bit 2: the small kernels of the step too; 0: default carve-outs
@@ -276,7 +285,8 @@ int mal_debug_linear(int32_t M, int32_t K, int32_t Nout, const float *A, int64_t
                      int32_t w_trans, const float *bias, int32_t epi, const float *aux, int64_t ld_aux, float *Y,
                      int64_t ldy, int32_t use_tc, void *stream);
 
-/* QMixer.forward / VDNMixer.forward outside the learner, qmix.py:41-59 / vdn.py:9-10.
+/* QMixer.forward / VDNMixer.forward outside the learner, qmix.py:41-59 / vdn.py:9-10 (MAL_MIXER_NONE is rejected:
+ * there is no mixer module to run).
  * agent_qs [B*T,N] contiguous, states [B,T,S] with strides in elements, scratch >= B*T*(2*HE+2*E + E*N+E)
  * floats (unused for VDN), q_tot [B*T]. */
 int mal_mixer_forward(int32_t mixer, int32_t B, int32_t T, int32_t N, int32_t S, int32_t E, int32_t HE,

@@ -14,9 +14,9 @@ import sys
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmal_b200.so")
 SRC = os.path.join(_HERE, "csrc", "mal_b200.cu")
-ABI_VERSION = 4
+ABI_VERSION = 5
 
-MIXER_VDN, MIXER_QMIX2, MIXER_QMIX1 = 0, 1, 2
+MIXER_VDN, MIXER_QMIX2, MIXER_QMIX1, MIXER_NONE = 0, 1, 2, 3    # MIXER_NONE: independent Q-learners (IQL)
 AGENT_RNN, AGENT_DQN = 0, 1
 IN_NO_LAST_ACTION, IN_NO_AGENT_ID = 1, 2     # agent-input switches (mal_learner_cfg_t.agent_input, mal_rollout_io_t.agent_input)
 STEP_DENSE = 1                               # dense_input of mal_agent_step / mal_dqn_step: bit 0; bits 1..2 = IN_* << 1

@@ -593,6 +593,9 @@ __global__ void __launch_bounds__(128, 3) k_q_head(HeadArgs a) {
 // fc2/gather backward injection d h_t += d_chosen * W2[a_t].   One warp per (b,t); lane = embed index.
 //                                            q_learner.py:40-42,81-98, qmix.py:41-59, vdn.py:9-10
 // All seeds are UN-normalised (without the 1/mask.sum() factor); k_grad_reduce applies it once at the end.
+// No mixer (IQL): lane n is agent n's own transition: its TD error against the shared reward, its q_tot / targets / td
+// entry [m*N + n], its seed, and its share of the statistics, so that the block sums come out over the mask expanded to
+// [B,T,N] (q_learner.py:92): sum m and the count are N times the per-transition values.
 // =============================================================================================
 #define MIX_NSTAT 6   // sum mtd^2, sum |mtd|, sum q_tot*m, sum targets*m, sum m, count(m != 0)
 struct MixArgs {
@@ -650,7 +653,7 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
     float st[MIX_NSTAT] = {0, 0, 0, 0, 0, 0};
     float dv2w = 0, dv2b = 0;
     float v2w_o = 0.0f, v2w_t = 0.0f, v2b_o = 0.0f, v2b_t = 0.0f;
-    if (a.mixer != MAL_MIXER_VDN) {
+    if (mixer_has_hypernet(a.mixer)) {
         v2w_o = act ? __ldg(a.mparams[0] + ML.v2_w + lane) : 0.0f;
         v2w_t = act ? __ldg(a.mparams[1] + ML.v2_w + lane) : 0.0f;
         v2b_o = __ldg(a.mparams[0] + ML.v2_b);
@@ -670,8 +673,11 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
         const float term = (float)(*field_ptr<unsigned char>(a.terminated, b, t));
         float y, ty, pre = 0, hidden = 0, wf = 0, v1 = 0;
         const float *a2o = a.a2[0] + m * ld2;
+        const bool iql = a.mixer == MAL_MIXER_NONE;       // warp-uniform
         if (a.mixer == MAL_MIXER_VDN) {
             y = warp_sum(qc); ty = warp_sum(qt);
+        } else if (iql) {
+            y = qc; ty = qt;                             // lane n: agent n's chosen / target Q (lanes >= N carry zeros)
         } else {
             // online and target mixer rows side by side (lane = embed unit): hidden = elu(q . |w1| + b1), y = hidden . |w_f| + V(s)
             const float *a2t = a.a2[1] + m * ld2;
@@ -698,7 +704,15 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
         const float tdv = y - target;
         const float mtd = tdv * mk;
         const float gseed = 2.0f * mtd * mk;   // (d loss / d q_tot) * mask.sum()
-        if (lane == 0) {
+        if (iql) {
+            if (lane == 0) a.mask[m] = mk;
+            if (lane < a.N) {
+                const int64_t e = m * a.N + lane;
+                a.q_tot[e] = y; a.target_q_tot[e] = ty; a.targets[e] = target; a.td[e] = tdv;
+                st[0] += mtd * mtd; st[1] += fabsf(mtd); st[2] += y * mk; st[3] += target * mk;
+                st[4] += mk; st[5] += (mk != 0.0f) ? 1.0f : 0.0f;
+            }
+        } else if (lane == 0) {
             a.mask[m] = mk;
             a.q_tot[m] = y; a.target_q_tot[m] = ty; a.targets[m] = target; a.td[m] = tdv;
             st[0] += mtd * mtd; st[1] += fabsf(mtd); st[2] += y * mk; st[3] += target * mk;
@@ -722,8 +736,8 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
                 reinterpret_cast<float2 *>(dh + (int64_t)n * HID)[lane] = v;
             }
         };
-        if (a.mixer == MAL_MIXER_VDN) {
-            if (lane < a.N) a.d_chosen[m * a.N + lane] = gseed;   // d q_tot / d q_n = 1
+        if (!mixer_has_hypernet(a.mixer)) {
+            if (lane < a.N) a.d_chosen[m * a.N + lane] = gseed;   // VDN: d q_tot / d q_n = 1; IQL: lane n's own seed
             head_inject(gseed);
             continue;
         }
@@ -754,9 +768,11 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
         head_inject(dq_mine);
     }
     // ---- deterministic block partials
+    if (a.mixer == MAL_MIXER_NONE)                // IQL: every lane holds its agent's sums (fixed shuffle order)
+        for (int k = 0; k < MIX_NSTAT; ++k) st[k] = warp_sum(st[k]);
     if (lane == 0)
         for (int k = 0; k < MIX_NSTAT; ++k) s_stats[warp][k] = st[k];
-    if (a.mixer != MAL_MIXER_VDN) {
+    if (mixer_has_hypernet(a.mixer)) {
         if (lane < a.E) s_v2[warp][lane] = dv2w;
         if (lane == 0) s_v2[warp][a.E] = dv2b;
     }
@@ -767,7 +783,7 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
         for (int w = 0; w < 8; ++w) s += s_stats[w][tid];
         a.part_stats[blockIdx.x * MIX_NSTAT + tid] = s;
     }
-    if (a.mixer != MAL_MIXER_VDN && tid <= a.E) {
+    if (mixer_has_hypernet(a.mixer) && tid <= a.E) {
         float s = 0;
         for (int w = 0; w < 8; ++w) s += s_v2[w][tid];
         a.part_v2[(int64_t)blockIdx.x * (a.E + 1) + tid] = s;

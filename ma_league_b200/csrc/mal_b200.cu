@@ -503,8 +503,8 @@ static int get_dims(const mal_batch_t *b, const mal_learner_cfg_t *c, Dims *d) {
     MAL_REQUIRE(b->B >= 1 && b->TT >= 2 && b->N >= 1 && b->OBS >= 1 && b->S >= 1, "bad batch dims (need TT >= 2)");
     MAL_REQUIRE(b->A >= 1 && b->A <= MAL_MAX_ACTIONS, "n_actions must be in [1, %d]", MAL_MAX_ACTIONS);
     MAL_REQUIRE(b->N <= MAL_MAX_ACTIONS, "n_agents must be <= %d", MAL_MAX_ACTIONS);
-    MAL_REQUIRE(c->mixer == MAL_MIXER_VDN || c->mixer == MAL_MIXER_QMIX2 || c->mixer == MAL_MIXER_QMIX1,
-                "Mixer %d not recognised.", c->mixer);
+    MAL_REQUIRE(c->mixer == MAL_MIXER_VDN || c->mixer == MAL_MIXER_QMIX2 || c->mixer == MAL_MIXER_QMIX1 ||
+                c->mixer == MAL_MIXER_NONE, "Mixer %d not recognised.", c->mixer);
     d->B = b->B; d->TT = b->TT; d->T = b->TT - 1; d->N = b->N; d->A = b->A; d->OBS = b->OBS; d->S = b->S;
     MAL_REQUIRE(c->agent_kind == MAL_AGENT_RNN || c->agent_kind == MAL_AGENT_DQN, "agent kind %d not recognised", c->agent_kind);
     d->kind = c->agent_kind;
@@ -512,15 +512,15 @@ static int get_dims(const mal_batch_t *b, const mal_learner_cfg_t *c, Dims *d) {
     d->in = agent_input(b->OBS, b->A, b->N, c->agent_input);
     d->R = b->B * b->N; d->d_in = d->in.d_in; d->mixer = c->mixer;
     d->E = c->embed; d->HE = c->hyper_embed; d->two = (c->mixer == MAL_MIXER_QMIX2);
-    if (c->mixer != MAL_MIXER_VDN) {
+    if (mixer_has_hypernet(c->mixer)) {
         MAL_REQUIRE(d->E >= 1 && d->E <= MAL_MAX_EMBED, "mixing_embed_dim must be in [1, %d]", MAL_MAX_EMBED);
         if (d->two) MAL_REQUIRE(d->HE >= 1, "hypernet_embed must be >= 1");
     } else { d->E = 0; d->HE = 0; }
     d->M1 = (int64_t)d->TT * d->R;
     d->BT = (int64_t)d->B * d->T;
     MAL_REQUIRE(d->M1 < ((int64_t)1 << 31), "batch too large: (T+1)*B*N must be < 2^31 (row indices are 32-bit in the kernels)");
-    d->ld1 = d->mixer == MAL_MIXER_VDN ? 0 : (d->two ? 2 * d->HE + 2 * d->E : 2 * d->E);
-    d->ld2 = d->mixer == MAL_MIXER_VDN ? 0 : d->E * d->N + d->E;
+    d->ld1 = !mixer_has_hypernet(d->mixer) ? 0 : (d->two ? 2 * d->HE + 2 * d->E : 2 * d->E);
+    d->ld2 = !mixer_has_hypernet(d->mixer) ? 0 : d->E * d->N + d->E;
     return 0;
 }
 
@@ -596,7 +596,7 @@ static PartLayout part_layout(const Dims &d, int sms) {
     p.whhb_w = take((int64_t)p.nc_a * 64 * HID);  p.whhb_b = take((int64_t)p.nc_a * 64);
     p.fc1_w = take((int64_t)p.nc_f1 * HID * d.d_in); p.fc1_b = take((int64_t)p.nc_f1 * HID);
     p.fc2_w = take((int64_t)p.nc_f2 * d.A * HID);    p.fc2_b = take((int64_t)p.nc_f2 * d.A);
-    if (d.mixer != MAL_MIXER_VDN) {
+    if (mixer_has_hypernet(d.mixer)) {
         p.m_l2a_w = take((int64_t)p.nc_m2 * d.E * d.N * K2); p.m_l2a_b = take((int64_t)p.nc_m2 * d.E * d.N);
         p.m_l2b_w = take((int64_t)p.nc_m2 * d.E * K2);       p.m_l2b_b = take((int64_t)p.nc_m2 * d.E);
         p.m_l1_w = take((int64_t)p.nc_m1 * d.ld1 * d.S);     p.m_l1_b = take((int64_t)p.nc_m1 * d.ld1);
@@ -632,8 +632,9 @@ extern "C" int mal_learner_plan(const mal_batch_t *batch, const mal_learner_cfg_
     plan->mask = take(d.BT, 4);
     plan->y1_on = take(d.BT * d.ld1, 4); plan->y1_tg = take(d.BT * d.ld1, 4);
     plan->a2_on = take(d.BT * d.ld2, 4); plan->a2_tg = take(d.BT * d.ld2, 4);
-    plan->q_tot = take(d.BT, 4); plan->target_q_tot = take(d.BT, 4);
-    plan->targets = take(d.BT, 4); plan->td = take(d.BT, 4);
+    const int64_t nq_tot = d.mixer == MAL_MIXER_NONE ? d.BT * d.N : d.BT;   // IQL: one TD error per agent
+    plan->q_tot = take(nq_tot, 4); plan->target_q_tot = take(nq_tot, 4);
+    plan->targets = take(nq_tot, 4); plan->td = take(nq_tot, 4);
     plan->d_a2 = take(d.BT * d.ld2, 4); plan->d_y1 = take(d.BT * d.ld1, 4);
     plan->d_chosen = take(d.BT * d.N, 4);
     plan->d_g = take(d.M1 * 4 * HID, 4);
@@ -663,7 +664,7 @@ static thread_local int g_tc_dbg = 0;
 // k_gru_fwd9 may run a chain count between 2 and 3 per SM as 2 * SMs equal workers (GruFwdArgs.bal_D): 87 -> 66 us alone at
 // 5v5 / B = 32.  Every worker is then on the critical path, so GEMMs that move in beside it (the mixer hypernets) cost more
 // than the balance gains (0.322 vs 0.313 ms per step): 1 (default) balances only when nothing runs beside the forward
-// recurrence (VDN), 2 always, 0 never.
+// recurrence (VDN, no mixer), 2 always, 0 never.
 static thread_local int g_gru_balance = 1;
 static thread_local int g_gru_balance_pdl = 0;
 static thread_local int g_gru_variant = 9;     // recurrences: 9 = 64-thread CTAs, time loop unrolled over the ring slots; 7 = the same before the trimming; 8 = one chain per 128-thread CTA
@@ -675,7 +676,7 @@ static thread_local int g_tc_pipelined = 1;   // software-pipelined k_linear_tc2
 static thread_local int g_rec_tc = 1;         // tensor-core recurrence k_gru_fwd_tc: 0 off, 1 when both nets have >= REC_TC_MIN_ROWS chains, 2 whenever R % 32 == 0
 #define REC_TC_MIN_ROWS 8192                  // chains (both nets) from which a 128-chain MMA tile per SM beats one FFMA CTA per chain
 static thread_local int g_rec_tc_bwd = 0;     // tensor-core BPTT k_gru_bwd_tc beside k_gru_fwd_tc (A operand in tensor memory): correct, but measured slower than k_gru_bwd9 (4.16 vs 3.08 ms at 20v20); 1: on
-static uint64_t g_stat_rec_tc = 0, g_stat_rec_tc_bwd = 0, g_stat_reduce_fc1 = 0;
+static uint64_t g_stat_rec_tc = 0, g_stat_rec_tc_bwd = 0, g_stat_reduce_fc1 = 0, g_stat_gru_balanced = 0;
 static thread_local int g_fc1_fused = 1;      // fc1 weight gradient over the full input width on one CTA per row chunk (k_reduce_fc1); 0: 128-column tiles of k_reduce_tc3
 
 // Launch counters per kernel flavour since process start (tests check which variant the heuristics picked).
@@ -690,6 +691,7 @@ extern "C" uint64_t mal_stat(const char *name) {
     if (strcmp(name, "rec_tc") == 0) return g_stat_rec_tc;
     if (strcmp(name, "rec_tc_bwd") == 0) return g_stat_rec_tc_bwd;
     if (strcmp(name, "reduce_fc1") == 0) return g_stat_reduce_fc1;
+    if (strcmp(name, "gru_balanced") == 0) return g_stat_gru_balanced;
     return 0;
 }
 extern "C" int mal_set_option(const char *name, int value) {
@@ -848,6 +850,7 @@ static int launch_gru_fwd(const GruFwdArgs &a_in, int nets, int sms, int *chain_
         a.bal_chains = chains;
         a.bal_D = (int)ceil_div64((int64_t)chains * a.TT, workers);
         a.chain_flags = chain_flags;
+        ++g_stat_gru_balanced;
         // NOT as a programmatic dependent launch: the workers must find all SMs free.  Launched early they are packed three
         // and four deep onto the SMs that the predecessor (k_agent_in_tc: one CTA per SM, ragged last round) vacates first,
         // and the point of the balance -- two workers per SM -- is lost (graph replay: 0.322 vs 0.313 ms per step)
@@ -919,7 +922,7 @@ extern "C" int mal_learner_forward(const mal_batch_t *batch, const mal_learner_c
     Dims d;
     if (int rc = get_dims(batch, cfg, &d)) return rc;
     MAL_REQUIRE(plan && workspace && agent && target_agent, "mal_learner_forward: null argument");
-    MAL_REQUIRE(d.mixer == MAL_MIXER_VDN || (mixer && target_mixer), "mal_learner_forward: mixer parameters missing");
+    MAL_REQUIRE(!mixer_has_hypernet(d.mixer) || (mixer && target_mixer), "mal_learner_forward: mixer parameters missing");
     MAL_REQUIRE(d.M1 * 4 * HID < (int64_t)1 << 40, "problem too large");
     MAL_REQUIRE(d.M1 < 2147483647LL && d.BT < 2147483647LL, "row count overflows int32");
     int sms, tps;
@@ -1007,8 +1010,9 @@ extern "C" int mal_learner_forward(const mal_batch_t *batch, const mal_learner_c
     // When the forward recurrence may run balanced (nothing else beside it: VDN) the transposes start AFTER it: a dozen
     // CTAs that hold SMs (or just their default carve-out) when the 2 x SMs workers are placed push a third worker onto
     // some SMs, and the whole balanced schedule then runs at the three-per-SM pace (graph replay: 0.300 vs 0.285 ms).
+    // No mixer (IQL) has nothing beside the recurrence either.
     cudaStream_t sx = g_overlap ? ss->s[1] : st;
-    const bool rec_alone = d.mixer == MAL_MIXER_VDN;
+    const bool rec_alone = !mixer_has_hypernet(d.mixer);
     auto launch_transposes = [&]() -> int {
         if (fork_to(st, sx, ss->aux_fork_ev)) return 2;
         TransArgs ta;
@@ -1118,7 +1122,7 @@ extern "C" int mal_learner_forward(const mal_batch_t *batch, const mal_learner_c
         // stream (the backward joins that stream before k_grad_reduce) and leaves the critical path
         cudaStream_t sf = (g_defer_stats && g_overlap) ? ss->s[0] : st;
         if (fork_to(st, sf, ss->fork_ev[3])) return 2;
-        { ProfScope _ps("k_stats_finalize", sf); k_stats_finalize<<<1 + (d.mixer != MAL_MIXER_VDN ? (d.E + 1 + 7) / 8 : 0), 256, 0, sf>>>(
+        { ProfScope _ps("k_stats_finalize", sf); k_stats_finalize<<<1 + (mixer_has_hypernet(d.mixer) ? (d.E + 1 + 7) / 8 : 0), 256, 0, sf>>>(
                                                        parts + pl.mix_stats, pl.nblk_mix, d.N, scalars, parts + pl.mix_v2,
                                                        d.E + 1, parts + pl.mix_v2_sum); }
         MAL_LAUNCH_CHECK("k_stats_finalize");
@@ -1161,7 +1165,7 @@ extern "C" int mal_mixer_forward(int32_t mixer, int32_t B, int32_t T, int32_t N,
     a.mixer = mixer; a.B = B; a.T = T; a.N = N; a.E = E; a.HE = HE; a.S = S;
     a.chosen = agent_qs; a.q_tot = q_tot;
     const int64_t BT = (int64_t)B * T;
-    if (mixer != MAL_MIXER_VDN) {
+    if (mixer_has_hypernet(mixer)) {
         MAL_REQUIRE(params && states && scratch && S > 0, "mal_mixer_forward: params/states/scratch missing");
         MAL_REQUIRE(E >= 1 && E <= MAL_MAX_EMBED, "mixing_embed_dim must be in [1, %d]", MAL_MAX_EMBED);
         const MixerLayout ML = mixer_layout(mixer, S, N, E, HE);
@@ -1289,7 +1293,7 @@ extern "C" int mal_learner_backward(const mal_batch_t *batch, const mal_learner_
     Dims d;
     if (int rc = get_dims(batch, cfg, &d)) return rc;
     MAL_REQUIRE(plan && workspace && agent && grad, "mal_learner_backward: null argument");
-    MAL_REQUIRE(d.mixer == MAL_MIXER_VDN || mixer, "mal_learner_backward: mixer parameters missing");
+    MAL_REQUIRE(!mixer_has_hypernet(d.mixer) || mixer, "mal_learner_backward: mixer parameters missing");
     int sms, tps;
     if (device_sm_count(&sms, &tps)) return 2;
     cudaStream_t st = (cudaStream_t)stream;
@@ -1436,7 +1440,7 @@ extern "C" int mal_learner_backward(const mal_batch_t *batch, const mal_learner_
         seg(AL.fc2_w, (int64_t)d.A * HID, parts + pl.fc2_w, pl.nc_f2, (int64_t)d.A * HID);
         seg(AL.fc2_b, d.A, parts + pl.fc2_b, pl.nc_f2, d.A);
         const int64_t o = AL.total;
-        if (d.mixer != MAL_MIXER_VDN) {
+        if (mixer_has_hypernet(d.mixer)) {
             const int K2 = d.two ? d.HE : d.S;
             const int64_t l1w = (int64_t)d.ld1 * d.S;
             const int b1row = d.two ? 2 * d.HE : 0;

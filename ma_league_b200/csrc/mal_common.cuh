@@ -91,6 +91,10 @@ __host__ __device__ inline AgentInput agent_input(int OBS, int A, int N, int fla
     return in;
 }
 
+// QMIX (1- or 2-layer hypernetworks) is the only mixer with parameters, hypernet intermediates and a mixer backward;
+// VDN and the absent mixer (IQL, MAL_MIXER_NONE) have none.  Every "is there a hypernetwork" branch tests this.
+__host__ __device__ inline bool mixer_has_hypernet(int mixer) { return mixer == MAL_MIXER_QMIX2 || mixer == MAL_MIXER_QMIX1; }
+
 struct MixerLayout {   // qmix.py:16-39 (layers == 2: Linear-ReLU-Linear hypernets; == 1: single Linear)
     int S, N, E, HE, layers;
     int64_t w1a_w, w1a_b, w1b_w, w1b_b;   // hyper_w_1.{0,2}  (layers==1: only w1b = hyper_w_1, K = S)
@@ -101,7 +105,7 @@ __host__ __device__ inline MixerLayout mixer_layout(int mixer, int S, int N, int
     MixerLayout L;
     L.S = S; L.N = N; L.E = E; L.HE = HE; L.layers = (mixer == MAL_MIXER_QMIX2) ? 2 : 1;
     int64_t o = 0;
-    if (mixer == MAL_MIXER_VDN) { L.total = 0; L.layers = 0; return L; }
+    if (!mixer_has_hypernet(mixer)) { L.total = 0; L.layers = 0; return L; }
     if (L.layers == 2) {
         L.w1a_w = o; o += (int64_t)HE * S;  L.w1a_b = o; o += HE;
         L.w1b_w = o; o += (int64_t)E * N * HE; L.w1b_b = o; o += E * N;

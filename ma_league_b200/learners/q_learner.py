@@ -1,4 +1,5 @@
-"""Q-learning learner for VDN / QMIX with the reference's API (marl/learners/q_learner.py:11-147).
+"""Q-learning learner for VDN / QMIX / independent Q-learners (`mixer: None`) with the reference's API
+(marl/learners/q_learner.py:11-147).
 
 `train()` is one call into libmal_b200 (`mal_learner_step`): online + target RNN unroll, chosen-Q gather, masked
 double-Q target max, mixers, TD loss, full backward (mixer + BPTT), clip_grad_norm_ and RMSprop.  Nothing is read
@@ -46,7 +47,8 @@ class QLearner(Learner):
                 raise ValueError("Mixer {} not recognised.".format(args.mixer))
             self.target_mixer = copy.deepcopy(self.mixer)
         else:
-            raise ValueError("mixer=None (IQL) is broken in the reference (q_learner.py:32) and not supported")
+            # IQL: every agent learns from its own TD error; there is no mixer and no target mixer
+            self.target_mixer = None
         self.target_mac = copy.deepcopy(mac)
         self._ws = None
         self._ws_key = None
@@ -65,11 +67,21 @@ class QLearner(Learner):
         self.n_graph_replays = self.n_graph_captures = self.n_eager_steps = 0   # accounting (bench.py reports them)
         self.dp_profile = None   # set to [] to collect (start, end) CUDA events around the data-parallel exchange
 
+    def build_optimizer(self):
+        if self.mixer is None:
+            self._agent_frozen()           # a frozen agent without a mixer leaves nothing to train: raise here already
+        super().build_optimizer()
+
     def parameters(self):
+        # q_learner.py:30-32 returns [] without a mixer (an operator-precedence slip); the agent's parameters are meant
+        if self.mixer is None:
+            return list(self.mac.parameters())
         return list(self.mac.parameters()) + list(self.mixer.parameters())
 
     # ------------------------------------------------------------------ ABI marshalling
     def _mixer_kind(self):
+        if self.mixer is None:
+            return nat.MIXER_NONE
         return self.mixer.mal_kind if isinstance(self.mixer, QMixer) else nat.MIXER_VDN
 
     def _cfg(self):
@@ -89,6 +101,11 @@ class QLearner(Learner):
         n_req = sum(1 for p in ap if p.requires_grad)
         if 0 < n_req < len(ap):
             raise nat.MalError("partially frozen agents are not supported: freeze all agent parameters or none")
+        if self.mixer is None:
+            if len(ap) > 0 and n_req == 0:
+                raise nat.MalError("the agent is frozen (args.freeze_native) and there is no mixer: "
+                                   "independent Q-learners (mixer=None) would have no parameter to train")
+            return False
         mp = getattr(self.mixer, "_mal_params", None) or list(self.mixer.parameters())
         if not all(p.requires_grad for p in mp):
             raise nat.MalError("frozen mixer parameters are not supported by the fused learner step")
@@ -152,8 +169,10 @@ class QLearner(Learner):
             if self._ws is None or self._ws.numel() < self._plan.total_bytes or self._ws.device != dev:
                 self._ws = th.empty(self._plan.total_bytes, dtype=th.uint8, device=dev)
             self._ws_key = key
+        no_mixer = self.mixer is None
         flats = dict(agent=ensure_flat(self.mac.agent), tagent=ensure_flat(self.target_mac.agent),
-                     mixer=ensure_flat(self.mixer), tmixer=ensure_flat(self.target_mixer))
+                     mixer=None if no_mixer else ensure_flat(self.mixer),
+                     tmixer=None if no_mixer else ensure_flat(self.target_mixer))
         n_total = self._plan.n_agent_params + self._plan.n_mixer_params
         if flats["agent"].numel() != self._plan.n_agent_params or \
                 (flats["mixer"].numel() if flats["mixer"] is not None else 0) != self._plan.n_mixer_params:
@@ -417,18 +436,20 @@ class QLearner(Learner):
         return self._grad
 
     def intermediates(self, batch):
-        """Views of the workspace arrays produced by the last forward for `batch`'s shape."""
+        """Views of the workspace arrays produced by the last forward for `batch`'s shape (q_tot / target_q_tot /
+        targets / td are [B,T,N] without a mixer: one TD error per agent)."""
         p = self._plan
         B, TT = batch.batch_size, batch.max_seq_length
         N, A, T = self.args.n_agents, self.args.n_actions, TT - 1
+        Q = N if self.mixer is None else 1
         out = dict(chosen=self._ws_f32(p.chosen, B * T * N).view(B, T, N),
                    target_max=self._ws_f32(p.target_max, B * T * N).view(B, T, N),
                    argmax=self._ws[p.argmax:p.argmax + 4 * B * T * N].view(th.int32).view(B, T, N),
                    mask=self._ws_f32(p.mask, B * T).view(B, T, 1),
-                   q_tot=self._ws_f32(p.q_tot, B * T).view(B, T, 1),
-                   target_q_tot=self._ws_f32(p.target_q_tot, B * T).view(B, T, 1),
-                   targets=self._ws_f32(p.targets, B * T).view(B, T, 1),
-                   td=self._ws_f32(p.td, B * T).view(B, T, 1),
+                   q_tot=self._ws_f32(p.q_tot, B * T * Q).view(B, T, Q),
+                   target_q_tot=self._ws_f32(p.target_q_tot, B * T * Q).view(B, T, Q),
+                   targets=self._ws_f32(p.targets, B * T * Q).view(B, T, Q),
+                   td=self._ws_f32(p.td, B * T * Q).view(B, T, Q),
                    hout=self._ws_f32(p.h_on, TT * B * N * nat.HID).view(TT, B * N, nat.HID),
                    # relu(fc1): its own array for the recurrent agent, the "hidden state" itself for the feed-forward one
                    x=self._ws_f32(p.h_on if getattr(self.mac.agent, "mal_kind", nat.AGENT_RNN) == nat.AGENT_DQN else p.x_on,
@@ -447,8 +468,9 @@ class QLearner(Learner):
 
     def update_targets(self):
         """q_learner.py:127-131: online -> target copy (one flat device copy per network)."""
-        pairs = [(ensure_flat(self.target_mac.agent), ensure_flat(self.mac.agent)),
-                 (ensure_flat(self.target_mixer), ensure_flat(self.mixer))]
+        pairs = [(ensure_flat(self.target_mac.agent), ensure_flat(self.mac.agent))]
+        if self.mixer is not None:
+            pairs.append((ensure_flat(self.target_mixer), ensure_flat(self.mixer)))
         for dst, src in pairs:
             if dst is None:
                 continue
