@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MAL_ABI_VERSION 5
+#define MAL_ABI_VERSION 6
 #define MAL_HID 64
 #define MAL_MAX_ACTIONS 32
 #define MAL_MAX_EMBED 32
@@ -292,6 +292,37 @@ int mal_debug_linear(int32_t M, int32_t K, int32_t Nout, const float *A, int64_t
 int mal_mixer_forward(int32_t mixer, int32_t B, int32_t T, int32_t N, int32_t S, int32_t E, int32_t HE,
                       const float *params, const float *agent_qs, const float *states, int64_t state_sb,
                       int64_t state_st, float *scratch, float *q_tot, void *stream);
+
+/* Autograd backward of the stand-alone module calls (BasicMAC.forward / DRQNAgentNetwork.forward / DQNAgentNetwork.forward for
+ * one step, QMixer.forward), for callers that train through the modules with torch autograd instead of QLearner.train.
+ * Both recompute what they need from the forward's inputs, write gradients (no accumulation: the caller adds them up) and
+ * use no float atomics: two identical calls return bit-identical results.  Gradients with respect to obs / assembled inputs
+ * and states are not computed.  The workspace queries are host-only (no device needed); they return the size in bytes,
+ * or -1 (mal_last_error set) for arguments the backward rejects.
+ *
+ * mal_agent_step_backward: one step of mal_agent_step (agent_kind MAL_AGENT_RNN) or mal_dqn_step (MAL_AGENT_DQN).  agent,
+ * rows ... onehot_sb and h_in mean exactly what they mean there (dense_input bit 0 = assembled input, bits 1..2 = MAL_IN_*
+ * << 1; h_in NULL = zeros).  Upstream gradients: d_q [rows,A] and d_h_out [rows,64], either may be NULL (zeros).  Outputs:
+ * d_h_in [rows,64] (NULL: not wanted) and d_agent, the step's gradient of the flat parameters in state_dict order (NULL:
+ * frozen agent, only d_h_in is computed).  The feed-forward agent has no hidden state: h_in, d_h_out and d_h_in must be
+ * NULL (its hidden state passes through, so is its gradient).  All outputs contiguous. */
+int64_t mal_agent_step_backward_workspace(int32_t agent_kind, int32_t rows, int32_t n_agents, int32_t obs_dim,
+                                          int32_t n_actions, int32_t dense_input);
+int mal_agent_step_backward(int32_t agent_kind, const float *agent, int32_t rows, int32_t n_agents, int32_t obs_dim,
+                            int32_t n_actions, int32_t dense_input, const float *obs, int64_t obs_sb,
+                            const float *last_onehot, int64_t onehot_sb, const float *h_in, const float *d_q,
+                            const float *d_h_out, float *d_h_in, float *d_agent, void *workspace, void *stream);
+
+/* mal_mixer_backward: QMixer.forward backward for MAL_MIXER_QMIX2 / MAL_MIXER_QMIX1 (VDN's is d q_tot broadcast over the agents
+ * and needs no kernel; other mixers are rejected).  Arguments as in mal_mixer_forward; `scratch` is the buffer that the
+ * matching mal_mixer_forward call filled (raw hypernet outputs), d_q_tot [B*T].  Writes d_agent_qs [B*T,N] and d_params, the
+ * gradient of the flat mixer parameters in state_dict order.  The derivative of abs() is the sign of the raw value (0 at 0),
+ * as torch takes it. */
+int64_t mal_mixer_backward_workspace(int32_t mixer, int32_t B, int32_t T, int32_t N, int32_t S, int32_t E, int32_t HE);
+int mal_mixer_backward(int32_t mixer, int32_t B, int32_t T, int32_t N, int32_t S, int32_t E, int32_t HE,
+                       const float *params, const float *agent_qs, const float *states, int64_t state_sb,
+                       int64_t state_st, const float *scratch, const float *d_q_tot, float *d_agent_qs, float *d_params,
+                       void *workspace, void *stream);
 
 /* EpsilonGreedyActionSelector.select on existing Q-values, marl/components/action_selectors.py:44-62. */
 int mal_eps_greedy_select(const float *q, int64_t q_ld, int32_t rows, int32_t n_agents, int32_t n_actions,

@@ -14,7 +14,7 @@ import sys
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmal_b200.so")
 SRC = os.path.join(_HERE, "csrc", "mal_b200.cu")
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 MIXER_VDN, MIXER_QMIX2, MIXER_QMIX1, MIXER_NONE = 0, 1, 2, 3    # MIXER_NONE: independent Q-learners (IQL)
 AGENT_RNN, AGENT_DQN = 0, 1
@@ -120,6 +120,13 @@ _PROTOS = {
                                    C.c_void_p, C.c_void_p, C.POINTER(Select), C.c_void_p]),
     "mal_mixer_forward": (C.c_int, [C.c_int32] * 7 + [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                                                       C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mal_agent_step_backward_workspace": (C.c_int64, [C.c_int32] * 6),
+    "mal_agent_step_backward": (C.c_int, [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                          C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mal_mixer_backward_workspace": (C.c_int64, [C.c_int32] * 7),
+    "mal_mixer_backward": (C.c_int, [C.c_int32] * 7 + [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mal_eps_greedy_select": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(Select),
                                         C.c_void_p]),
     "mal_select_philox_advance": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(C.c_uint64)]),

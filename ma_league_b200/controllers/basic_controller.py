@@ -7,6 +7,7 @@ served through them (dense-input kernel) instead of the fused path.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 
 import torch as th
@@ -14,6 +15,7 @@ import torch as th
 from .. import _native as nat
 from ..components.action_selectors import make_select_struct
 from ..exceptions import HiddenStateNotInitialized
+from ..modules import autograd as ag
 from ..modules.agents import REGISTRY as agent_REGISTRY
 from ..modules.agents.drqn_agent import DRQNAgentNetwork
 from ..modules.agents.dqn_agent import DQNAgentNetwork
@@ -41,7 +43,8 @@ class BasicMAC(MultiAgentController):
                 raise ValueError("Expected at least one available action per agent (Categorical probs are all zero)")
             return out[0], out[1]
         avail_actions = ep_batch["avail_actions"][:, t_ep]
-        agent_outs = self.forward(ep_batch, t_ep, test_mode=test_mode)
+        with self._no_recording():    # acting never records an autograd node, whatever args.autograd_forward says
+            agent_outs = self.forward(ep_batch, t_ep, test_mode=test_mode)
         return self.action_selector.select(agent_outs[bs], avail_actions[bs], t_env, test_mode, u=u, e=e)
 
     def rollout_step(self, ep_batch, t_ep, t_env, pre, prev=None, alive=None, test_mode=False, u=None, e=None):
@@ -128,7 +131,12 @@ class BasicMAC(MultiAgentController):
         return out[0], out[1]
 
     def forward(self, ep_batch, t, test_mode=False):
+        """Q-values [bs, N, A] of timestep t.  Under `args.autograd_forward` (grad mode on, agent parameters or the hidden
+        state requiring grad) the step records an autograd node (modules/autograd.py), so that a loss over the outputs can
+        be back-propagated into the agent's parameters through time."""
         if self._fusable():
+            if self.hidden_states is not None and ag.recording(self, self.hidden_states, *self.agent.parameters()):
+                return self._step_recorded(ep_batch, t)
             return self._step(ep_batch, t, None)
         agent_inputs = self._build_inputs(ep_batch, t)
         if self.hidden_states is None:
@@ -209,22 +217,56 @@ class BasicMAC(MultiAgentController):
     def _rollout_fusable(self):
         return self._fusable() and isinstance(self.agent, DRQNAgentNetwork)
 
-    def _step(self, ep_batch, t, select_struct):
-        if self.hidden_states is None:
-            raise HiddenStateNotInitialized()
+    def _no_recording(self):
+        return th.no_grad() if getattr(self.args, "autograd_forward", False) else contextlib.nullcontext()
+
+    def _step_inputs(self, ep_batch, t):
+        """Pointers of the fused input assembly at timestep t: (obs [B, T+1, N, OBS], obs_ptr, last-action one-hot
+        [B, T+1, N, A] or None, last_ptr, last_sb)."""
         obs_all = nat.require_cuda(ep_batch["obs"], "ep_batch")        # [B, T+1, N, OBS] (strided view of the records)
-        B, _, N, OBS = obs_all.shape
+        OBS = obs_all.shape[3]
         A = self.n_actions
         if obs_all.stride(3) != 1 or obs_all.stride(2) != OBS or obs_all.dtype != th.float32:
             raise nat.MalError("obs must be float32 with contiguous [N, OBS] rows")
         obs_ptr = obs_all.data_ptr() + 4 * t * obs_all.stride(1)
-        flags = self._input_flags()
-        last_ptr, last_sb = None, 0
+        oh, last_ptr, last_sb = None, None, 0
         if t > 0 and self.args.obs_last_action:
             oh = ep_batch["actions_onehot"]
             if oh.stride(3) != 1 or oh.stride(2) != A or oh.dtype != th.float32:
                 raise nat.MalError("actions_onehot must be float32 with contiguous [N, A] rows")
             last_ptr, last_sb = oh.data_ptr() + 4 * (t - 1) * oh.stride(1), oh.stride(0)
+        return obs_all, obs_ptr, oh, last_ptr, last_sb
+
+    def _step_recorded(self, ep_batch, t):
+        """`_step` without selection as an autograd node: the same kernel launch, plus the backward of
+        modules/autograd.py.  The obs / one-hot views it reads and h_in are saved for the version check."""
+        obs_all, obs_ptr, oh, last_ptr, last_sb = self._step_inputs(ep_batch, t)
+        B, _, N, OBS = obs_all.shape
+        A = self.n_actions
+        rows = B * N
+        cfg = dict(rows=rows, N=N, OBS=OBS, A=A, dense_input=self._input_flags() << 1, obs_ptr=obs_ptr,
+                   obs_sb=obs_all.stride(0), last_ptr=last_ptr, last_sb=last_sb)
+        obs_v = obs_all[:, t]
+        oh_v = oh[:, t - 1] if oh is not None else None
+        with nat.on_device(obs_all.device):
+            if isinstance(self.agent, DQNAgentNetwork):
+                return ag.agent_step(self.agent, cfg, obs_v, oh_v, None).view(B, N, A)
+            h_in = self.hidden_states
+            if h_in.dim() == 3 and h_in.stride(0) == 0 and h_in.stride(1) == 0 and not h_in.requires_grad:
+                h_in = None                                                # fresh init_hidden(): zeros
+            else:
+                h_in = h_in.reshape(rows, nat.HID).contiguous()
+            q, h_out = ag.agent_step(self.agent, cfg, obs_v, oh_v, h_in)
+        self.hidden_states = h_out
+        return q.view(B, N, A)
+
+    def _step(self, ep_batch, t, select_struct):
+        if self.hidden_states is None:
+            raise HiddenStateNotInitialized()
+        obs_all, obs_ptr, _, last_ptr, last_sb = self._step_inputs(ep_batch, t)
+        B, _, N, OBS = obs_all.shape
+        A = self.n_actions
+        flags = self._input_flags()
         rows = B * N
         dev = obs_all.device
         if isinstance(self.agent, DQNAgentNetwork):      # feed-forward agent: no hidden state to read or write

@@ -13,6 +13,7 @@ from typing import Dict
 
 import torch as th
 
+from .._native import MalError
 from ..exceptions import HiddenStateNotInitialized
 from .basic_controller import BasicMAC
 
@@ -33,12 +34,16 @@ class EnsembleMAC(BasicMAC):
             self.native_hidden_states = self.hidden_states
             return out
         avail_actions = ep_batch["avail_actions"][:, t_ep]
-        agent_outs = self.forward(ep_batch, t_ep, test_mode=test_mode)
+        with self._no_recording():
+            agent_outs = self.forward(ep_batch, t_ep, test_mode=test_mode)
         return self.action_selector.select(agent_outs[bs], avail_actions[bs], t_env, test_mode, u=u, e=e)
 
     def forward(self, ep_batch, t, test_mode=False):
         if self.native_hidden_states is None:
             raise HiddenStateNotInitialized()
+        if self.ensemble and getattr(self.args, "autograd_forward", False) and th.is_grad_enabled():
+            raise MalError("EnsembleMAC.forward does not record autograd nodes for ensemble agents (a fixed-policy opponent); "
+                           "call it under torch.no_grad() or switch args.autograd_forward off")
         self.hidden_states = self.native_hidden_states
         agent_outs = super().forward(ep_batch, t, test_mode=test_mode)          # [B, N, A], native net for everyone
         self.native_hidden_states = self.hidden_states

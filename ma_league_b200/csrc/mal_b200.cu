@@ -12,6 +12,7 @@
 #include "gru_rec_tc.cuh"
 #include "agent_in_gemm.cuh"
 #include "tc_reduce.cuh"
+#include "autograd.cuh"
 
 // ---------------------------------------------------------------------------------------------
 static thread_local char g_err[512] = "";
@@ -1288,6 +1289,43 @@ static int launch_reduce(RedGroup &g, cudaStream_t st, const char *tag) {
     return 0;
 }
 
+// QMIX hypernet backward from the element-wise seeds d_a2 / d_y1: for two-layer hypernets the layer-2 input gradients
+//   d h1 = (d a1 . W_1.2) * (h1 > 0),  d hf = (d af . W_f.2) * (hf > 0)   (written into the h1 | hf columns of d_y1),
+// then the layer-2 and layer-1 weight-gradient split reductions into per-chunk partials.  Shared by the learner's backward and
+// mal_mixer_backward.  wt1 / wtf: hyper_w_1.2.weight / hyper_w_final.2.weight as GEMM operands W(n,k) (LinProb's w_trans).
+struct HyperBwd {
+    int mixer, two, N, E, HE, S, ld1, ld2;
+    int64_t BT;
+    const float *d_a2; float *d_y1; const float *y1;
+    const float *wt1, *wtf; int64_t ldw1, ldwf; int w_trans;
+    float *l2a_w, *l2a_b, *l2b_w, *l2b_b, *l1_w, *l1_b;
+    int nc_m2, nc_m1; int64_t rpc_m2, rpc_m1;
+};
+static void hyper_bwd_dims(const Dims &d, HyperBwd *h) {
+    h->mixer = d.mixer; h->two = d.two; h->N = d.N; h->E = d.E; h->HE = d.HE; h->S = d.S; h->ld1 = d.ld1; h->ld2 = d.ld2;
+    h->BT = d.BT;
+}
+static int launch_hyper_bwd(const HyperBwd &h, const BatchView &bv, cudaStream_t s1) {
+    if (h.mixer == MAL_MIXER_QMIX2) {
+        LinGroup g; g.n = 2; g.bv = bv;   // d h1 = (d a1 . W12) * (h1 > 0) ; d hf = (d af . Wf2) * (hf > 0)
+        g.p[0] = lin(h.BT, h.E * h.N, h.HE, A_DENSE, 0, h.d_a2, h.ld2, h.wt1, h.ldw1, h.w_trans, nullptr, EPI_MASKPOS, h.y1, h.ld1, h.d_y1, h.ld1);
+        g.p[1] = lin(h.BT, h.E, h.HE, A_DENSE, 0, h.d_a2 + h.E * h.N, h.ld2, h.wtf, h.ldwf, h.w_trans, nullptr, EPI_MASKPOS, h.y1 + h.HE, h.ld1, h.d_y1 + h.HE, h.ld1);
+        if (int rc = launch_linear(g, h.BT, h.E * h.N, s1, "k_linear_group:mixer_bwd_dh")) return rc;
+        RedGroup r; r.n = 3; r.bv = bv;
+        r.p[0] = red(h.BT, h.HE, h.E * h.N, h.d_a2, h.ld2, A_DENSE, 0, h.y1, h.ld1, h.l2a_w, h.l2a_b, h.nc_m2, h.rpc_m2);
+        r.p[1] = red(h.BT, h.HE, h.E, h.d_a2 + h.E * h.N, h.ld2, A_DENSE, 0, h.y1 + h.HE, h.ld1, h.l2b_w, h.l2b_b, h.nc_m2, h.rpc_m2);
+        r.p[2] = red(h.BT, h.S, h.ld1, h.d_y1, h.ld1, A_STATE, 0, nullptr, 0, h.l1_w, h.l1_b, h.nc_m1, h.rpc_m1);
+        if (int rc = launch_reduce(r, s1, "k_reduce_group:mixer")) return rc;
+    } else if (h.mixer == MAL_MIXER_QMIX1) {
+        RedGroup r; r.n = 3; r.bv = bv;
+        r.p[0] = red(h.BT, h.S, h.E * h.N, h.d_a2, h.ld2, A_STATE, 0, nullptr, 0, h.l2a_w, h.l2a_b, h.nc_m2, h.rpc_m2);
+        r.p[1] = red(h.BT, h.S, h.E, h.d_a2 + h.E * h.N, h.ld2, A_STATE, 0, nullptr, 0, h.l2b_w, h.l2b_b, h.nc_m2, h.rpc_m2);
+        r.p[2] = red(h.BT, h.S, h.ld1, h.d_y1, h.ld1, A_STATE, 0, nullptr, 0, h.l1_w, h.l1_b, h.nc_m1, h.rpc_m1);
+        if (int rc = launch_reduce(r, s1, "k_reduce_group:mixer")) return rc;
+    }
+    return 0;
+}
+
 extern "C" int mal_learner_backward(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
                                     const float *agent, const float *mixer, void *workspace, float *grad, void *stream) {
     Dims d;
@@ -1315,23 +1353,16 @@ extern "C" int mal_learner_backward(const mal_batch_t *batch, const mal_learner_
     if (fork_to(st, s2, ss->fork_ev[1])) return 2;
 
     // ---- side stream 1: mixer hypernet backward (independent of the agent BPTT)
-    if (d.mixer == MAL_MIXER_QMIX2) {
-        LinGroup g; g.n = 2; g.bv = bv;   // d h1 = (d a1 . W12) * (h1 > 0) ; d hf = (d af . Wf2) * (hf > 0)
-        const float *wt1 = F(plan->w_t) + (int64_t)HID * G3, *wtf = wt1 + (int64_t)d.HE * d.E * d.N;   // transposed by the forward call
-        g.p[0] = lin(d.BT, d.E * d.N, d.HE, A_DENSE, 0, d_a2, d.ld2, wt1, d.E * d.N, 0, nullptr, EPI_MASKPOS, y1, d.ld1, d_y1, d.ld1);
-        g.p[1] = lin(d.BT, d.E, d.HE, A_DENSE, 0, d_a2 + d.E * d.N, d.ld2, wtf, d.E, 0, nullptr, EPI_MASKPOS, y1 + d.HE, d.ld1, d_y1 + d.HE, d.ld1);
-        if (int rc = launch_linear(g, d.BT, d.E * d.N, s1, "k_linear_group:mixer_bwd_dh")) return rc;
-        RedGroup r; r.n = 3; r.bv = bv;
-        r.p[0] = red(d.BT, d.HE, d.E * d.N, d_a2, d.ld2, A_DENSE, 0, y1, d.ld1, parts + pl.m_l2a_w, parts + pl.m_l2a_b, pl.nc_m2, pl.rpc_m2);
-        r.p[1] = red(d.BT, d.HE, d.E, d_a2 + d.E * d.N, d.ld2, A_DENSE, 0, y1 + d.HE, d.ld1, parts + pl.m_l2b_w, parts + pl.m_l2b_b, pl.nc_m2, pl.rpc_m2);
-        r.p[2] = red(d.BT, d.S, d.ld1, d_y1, d.ld1, A_STATE, 0, nullptr, 0, parts + pl.m_l1_w, parts + pl.m_l1_b, pl.nc_m1, pl.rpc_m1);
-        if (int rc = launch_reduce(r, s1, "k_reduce_group:mixer")) return rc;
-    } else if (d.mixer == MAL_MIXER_QMIX1) {
-        RedGroup r; r.n = 3; r.bv = bv;
-        r.p[0] = red(d.BT, d.S, d.E * d.N, d_a2, d.ld2, A_STATE, 0, nullptr, 0, parts + pl.m_l2a_w, parts + pl.m_l2a_b, pl.nc_m2, pl.rpc_m2);
-        r.p[1] = red(d.BT, d.S, d.E, d_a2 + d.E * d.N, d.ld2, A_STATE, 0, nullptr, 0, parts + pl.m_l2b_w, parts + pl.m_l2b_b, pl.nc_m2, pl.rpc_m2);
-        r.p[2] = red(d.BT, d.S, d.ld1, d_y1, d.ld1, A_STATE, 0, nullptr, 0, parts + pl.m_l1_w, parts + pl.m_l1_b, pl.nc_m1, pl.rpc_m1);
-        if (int rc = launch_reduce(r, s1, "k_reduce_group:mixer")) return rc;
+    if (mixer_has_hypernet(d.mixer)) {
+        HyperBwd h;
+        hyper_bwd_dims(d, &h);
+        h.d_a2 = d_a2; h.d_y1 = d_y1; h.y1 = y1;
+        h.wt1 = F(plan->w_t) + (int64_t)HID * G3; h.wtf = h.wt1 + (int64_t)d.HE * d.E * d.N;   // transposed by the forward call
+        h.ldw1 = d.E * d.N; h.ldwf = d.E; h.w_trans = 0;
+        h.l2a_w = parts + pl.m_l2a_w; h.l2a_b = parts + pl.m_l2a_b; h.l2b_w = parts + pl.m_l2b_w; h.l2b_b = parts + pl.m_l2b_b;
+        h.l1_w = parts + pl.m_l1_w; h.l1_b = parts + pl.m_l1_b;
+        h.nc_m2 = pl.nc_m2; h.rpc_m2 = pl.rpc_m2; h.nc_m1 = pl.nc_m1; h.rpc_m1 = pl.rpc_m1;
+        if (int rc = launch_hyper_bwd(h, bv, s1)) return rc;
     }
     const bool frozen = cfg->freeze_agent != 0;   // multi_agent_controller.py:74-76: the agent gets no gradient at all
     // ---- side stream 2: fc2 gradients only need d_chosen and h (both forward products)
@@ -1473,6 +1504,257 @@ extern "C" int mal_learner_backward(const mal_batch_t *batch, const mal_learner_
         { ProfScope _ps("k_grad_reduce", st); launch_k(k_grad_reduce, dim3(pl.nblk_norm), dim3(256), 0, st, true, a); }   // stream predecessor: the fc1 reduction
         MAL_LAUNCH_CHECK("k_grad_reduce");
     }
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// autograd backward of the stand-alone module calls (one agent step, one QMixer.forward)
+// ---------------------------------------------------------------------------------------------
+// Chunk counts of the row reductions are a fixed function of the shapes (planned for a 148-SM B200), so that the workspace
+// size queries need no device and a gradient does not depend on the GPU it was computed on.
+#define MAL_BWD_SMS 148
+
+struct AgentBwdPlan {
+    AgentInput in;
+    int dense, ldi, nc;
+    int64_t rpc;
+    int64_t xin, x1, hp, hn, dq, d_g, d_x;                                            // bytes
+    int64_t fc1_w, fc1_b, wih_w, wih_b, whha_w, whha_b, whhb_w, whhb_b, fc2_w, fc2_b, norm;   // floats inside `parts`
+    int64_t parts, total;                                                             // bytes
+};
+
+static int agent_bwd_plan(int32_t kind, int32_t rows, int32_t N, int32_t OBS, int32_t A, int32_t dense_input, AgentBwdPlan *p) {
+    MAL_REQUIRE(kind == MAL_AGENT_RNN || kind == MAL_AGENT_DQN, "agent kind %d not recognised", kind);
+    MAL_REQUIRE(rows > 0 && N >= 1 && OBS >= 1, "mal_agent_step_backward: bad dims");
+    MAL_REQUIRE(A >= 1 && A <= MAL_MAX_ACTIONS, "n_actions must be in [1, %d]", MAL_MAX_ACTIONS);
+    MAL_REQUIRE((dense_input & ~7) == 0 && !((dense_input & 1) && (dense_input >> 1)),
+                "dense_input %d: bit 0 (dense) or the agent-input bits 1..2, nothing else", dense_input);
+    memset(p, 0, sizeof(*p));
+    p->dense = dense_input & 1;
+    if (p->dense) { p->in.obs = p->in.d_in = OBS; p->in.last = p->in.id = 0; }
+    else p->in = agent_input(OBS, A, N, dense_input >> 1);
+    MAL_REQUIRE(agent_bwd_smem(p->in.d_in) <= 200 * 1024, "mal_agent_step_backward: input width %d too large", p->in.d_in);
+    const bool rnn = kind == MAL_AGENT_RNN;
+    const int d_in = p->in.d_in;
+    p->ldi = (int)align_up64(d_in, 4);
+    int64_t o = 0;
+    auto take = [&](int64_t n_floats) { int64_t r = o; o += align_up64(n_floats * 4, 256); return r; };
+    p->xin = take(p->dense ? 0 : (int64_t)rows * p->ldi);
+    p->x1 = take((int64_t)rows * HID);
+    p->hp = take(rnn ? (int64_t)rows * HID : 0);
+    p->hn = take(rnn ? (int64_t)rows * HID : 0);
+    p->dq = take((int64_t)rows * A);
+    p->d_g = take(rnn ? (int64_t)rows * 4 * HID : 0);
+    p->d_x = take((int64_t)rows * HID);
+    int tiles = tiles_of(HID, d_in) + tiles_of(A, HID);
+    if (rnn) tiles += tiles_of(G3, HID) + tiles_of(128, HID) + tiles_of(64, HID);
+    chunking(rows, tiles, MAL_BWD_SMS, &p->nc, &p->rpc);
+    int64_t q = 0;
+    auto part = [&](int64_t n) { int64_t r = q; q += align_up64(n, 64); return r; };
+    p->fc1_w = part((int64_t)p->nc * HID * d_in); p->fc1_b = part((int64_t)p->nc * HID);
+    if (rnn) {
+        p->wih_w = part((int64_t)p->nc * G3 * HID);   p->wih_b = part((int64_t)p->nc * G3);
+        p->whha_w = part((int64_t)p->nc * 128 * HID); p->whha_b = part((int64_t)p->nc * 128);
+        p->whhb_w = part((int64_t)p->nc * 64 * HID);  p->whhb_b = part((int64_t)p->nc * 64);
+    }
+    p->fc2_w = part((int64_t)p->nc * A * HID); p->fc2_b = part((int64_t)p->nc * A);
+    p->norm = part(ceil_div64(agent_layout(d_in, A, kind).total, GRED_EPB));
+    p->parts = take(q);
+    p->total = o;
+    return 0;
+}
+
+extern "C" int64_t mal_agent_step_backward_workspace(int32_t agent_kind, int32_t rows, int32_t n_agents, int32_t obs_dim,
+                                                     int32_t n_actions, int32_t dense_input) {
+    AgentBwdPlan p;
+    if (agent_bwd_plan(agent_kind, rows, n_agents, obs_dim, n_actions, dense_input, &p)) return -1;
+    return p.total;
+}
+
+extern "C" int mal_agent_step_backward(int32_t agent_kind, const float *agent, int32_t rows, int32_t n_agents, int32_t obs_dim,
+                                       int32_t n_actions, int32_t dense_input, const float *obs, int64_t obs_sb,
+                                       const float *last_onehot, int64_t onehot_sb, const float *h_in, const float *d_q,
+                                       const float *d_h_out, float *d_h_in, float *d_agent, void *workspace, void *stream) {
+    AgentBwdPlan p;
+    if (int rc = agent_bwd_plan(agent_kind, rows, n_agents, obs_dim, n_actions, dense_input, &p)) return rc;
+    MAL_REQUIRE(agent && obs && workspace, "mal_agent_step_backward: agent, obs and workspace are required");
+    const bool rnn = agent_kind == MAL_AGENT_RNN;
+    MAL_REQUIRE(rnn || (!h_in && !d_h_out && !d_h_in), "mal_agent_step_backward: the feed-forward agent has no hidden state");
+    cudaStream_t st = (cudaStream_t)stream;
+    uint8_t *ws = (uint8_t *)workspace;
+    auto F = [&](int64_t off) { return reinterpret_cast<float *>(ws + off); };
+    AgentBwdArgs a;
+    memset(&a, 0, sizeof(a));
+    a.params = agent; a.kind = agent_kind; a.rows = rows; a.N = n_agents; a.OBS = obs_dim; a.A = n_actions; a.dense = p.dense;
+    a.in = p.in; a.obs = obs; a.obs_sb = obs_sb; a.onehot = p.in.last > 0 ? last_onehot : nullptr; a.onehot_sb = onehot_sb;
+    a.h_in = h_in; a.d_q = d_q; a.d_h_out = d_h_out;
+    a.xin = p.dense ? nullptr : F(p.xin); a.ldi = p.ldi;
+    a.x1 = F(p.x1); a.hp = rnn ? F(p.hp) : nullptr; a.hn = rnn ? F(p.hn) : nullptr; a.dq = F(p.dq);
+    a.d_g = rnn ? F(p.d_g) : nullptr; a.d_x = F(p.d_x); a.d_h_in = d_h_in;
+    const size_t smem = agent_bwd_smem(p.in.d_in);
+    static size_t attr[MAL_MAX_DEV];
+    if (smem > 48 * 1024) if (int rc = ensure_dyn_smem(k_agent_step_bwd, smem, attr)) return rc;
+    { ProfScope _ps("k_agent_step_bwd", st); k_agent_step_bwd<<<(unsigned)ceil_div64(rows, ABR_ROWS), ABR_THREADS, smem, st>>>(a); }
+    MAL_LAUNCH_CHECK("k_agent_step_bwd");
+    if (!d_agent) return 0;                      // frozen agent: only d h_in
+
+    // weight gradients: row reductions of the learner (one launch, dense loaders), then the fixed-order gather
+    const int d_in = p.in.d_in;
+    const AgentLayout AL = agent_layout(d_in, n_actions, agent_kind);
+    float *parts = F(p.parts);
+    const float *xin = p.dense ? obs : F(p.xin);
+    const int64_t ldx = p.dense ? obs_sb : p.ldi;
+    const float *hp = h_in ? h_in : F(p.hp);
+    BatchView bv;
+    memset(&bv, 0, sizeof(bv));
+    RedGroup r; r.n = 0; r.bv = bv;
+    r.p[r.n++] = red(rows, d_in, HID, F(p.d_x), HID, A_DENSE, 0, xin, ldx, parts + p.fc1_w, parts + p.fc1_b, p.nc, p.rpc);
+    if (rnn) {
+        const float *dg = F(p.d_g);
+        r.p[r.n++] = red(rows, HID, G3, dg, 4 * HID, A_DENSE, 0, F(p.x1), HID, parts + p.wih_w, parts + p.wih_b, p.nc, p.rpc);
+        r.p[r.n++] = red(rows, HID, 128, dg, 4 * HID, A_DENSE, 0, hp, HID, parts + p.whha_w, parts + p.whha_b, p.nc, p.rpc);
+        r.p[r.n++] = red(rows, HID, 64, dg + 3 * HID, 4 * HID, A_DENSE, 0, hp, HID, parts + p.whhb_w, parts + p.whhb_b, p.nc, p.rpc);
+    }
+    r.p[r.n++] = red(rows, HID, n_actions, F(p.dq), n_actions, A_DENSE, 0, rnn ? F(p.hn) : F(p.x1), HID, parts + p.fc2_w,
+                     parts + p.fc2_b, p.nc, p.rpc);
+    if (int rc = launch_reduce(r, st, "k_reduce_group:agent_step_bwd")) return rc;
+    GradReduceArgs g;
+    memset(&g, 0, sizeof(g));
+    int n = 0;
+    auto seg = [&](int64_t off, int64_t count, const float *part, int64_t stride) {
+        g.s[n].grad_off = off; g.s[n].count = (int)count; g.s[n].part = part; g.s[n].n_chunks = p.nc; g.s[n].chunk_stride = stride; ++n;
+    };
+    seg(AL.fc1_w, (int64_t)HID * d_in, parts + p.fc1_w, (int64_t)HID * d_in);
+    seg(AL.fc1_b, HID, parts + p.fc1_b, HID);
+    if (rnn) {
+        seg(AL.w_ih, (int64_t)G3 * HID, parts + p.wih_w, (int64_t)G3 * HID);
+        seg(AL.w_hh, 128 * HID, parts + p.whha_w, 128 * HID);
+        seg(AL.w_hh + 128 * HID, 64 * HID, parts + p.whhb_w, 64 * HID);
+        seg(AL.b_ih, G3, parts + p.wih_b, G3);
+        seg(AL.b_hh, 128, parts + p.whha_b, 128);
+        seg(AL.b_hh + 128, 64, parts + p.whhb_b, 64);
+    }
+    seg(AL.fc2_w, (int64_t)n_actions * HID, parts + p.fc2_w, (int64_t)n_actions * HID);
+    seg(AL.fc2_b, n_actions, parts + p.fc2_b, n_actions);
+    g.n = n; g.total = AL.total; g.grad = d_agent; g.norm_part = parts + p.norm; g.scalars = nullptr; g.unnormalized = 1;
+    { ProfScope _ps("k_grad_reduce", st); launch_k(k_grad_reduce, dim3((unsigned)ceil_div64(AL.total, GRED_EPB)), dim3(256), 0, st, false, g); }
+    MAL_LAUNCH_CHECK("k_grad_reduce");
+    return 0;
+}
+
+struct MixerBwdPlan {
+    int two, ld1, ld2, nblk, nc_m2, nc_m1;
+    int64_t rpc_m2, rpc_m1;
+    int64_t d_a2, d_y1, parts, total;                                         // bytes
+    int64_t l2a_w, l2a_b, l2b_w, l2b_b, l1_w, l1_b, v2, norm;                 // floats inside `parts`
+};
+
+static int mixer_bwd_plan(int32_t mixer, int32_t B, int32_t T, int32_t N, int32_t S, int32_t E, int32_t HE, MixerBwdPlan *p) {
+    MAL_REQUIRE(mixer_has_hypernet(mixer), "mal_mixer_backward: mixer %d has no kernel backward (VDN: d q_tot broadcast over agents)", mixer);
+    MAL_REQUIRE(B > 0 && T > 0 && N > 0 && N <= MAL_MAX_ACTIONS && S > 0, "mal_mixer_backward: bad dims");
+    MAL_REQUIRE(E >= 1 && E <= MAL_MAX_EMBED, "mixing_embed_dim must be in [1, %d]", MAL_MAX_EMBED);
+    MAL_REQUIRE(mixer != MAL_MIXER_QMIX2 || HE >= 1, "hypernet_embed must be >= 1");
+    memset(p, 0, sizeof(*p));
+    const int64_t BT = (int64_t)B * T;
+    p->two = mixer == MAL_MIXER_QMIX2;
+    p->ld1 = p->two ? 2 * HE + 2 * E : 2 * E;
+    p->ld2 = E * N + E;
+    const int K2 = p->two ? HE : S;
+    if (p->two) {   // the learner's chunking (part_layout)
+        chunking(BT, tiles_of(E * N, K2) + tiles_of(E, K2), MAL_BWD_SMS, &p->nc_m2, &p->rpc_m2);
+        chunking(BT, tiles_of(p->ld1, S), MAL_BWD_SMS, &p->nc_m1, &p->rpc_m1);
+    } else {
+        chunking(BT, tiles_of(E * N, K2) + tiles_of(E, K2) + tiles_of(p->ld1, S), MAL_BWD_SMS, &p->nc_m2, &p->rpc_m2);
+        p->nc_m1 = p->nc_m2; p->rpc_m1 = p->rpc_m2;
+    }
+    int64_t nb = ceil_div64(BT, 8); if (nb > MAL_BWD_SMS * 4) nb = MAL_BWD_SMS * 4;
+    p->nblk = (int)nb;
+    int64_t o = 0;
+    auto take = [&](int64_t n_floats) { int64_t r = o; o += align_up64(n_floats * 4, 256); return r; };
+    p->d_a2 = take(BT * p->ld2);
+    p->d_y1 = take(BT * p->ld1);
+    int64_t q = 0;
+    auto part = [&](int64_t n) { int64_t r = q; q += align_up64(n, 64); return r; };
+    p->l2a_w = part((int64_t)p->nc_m2 * E * N * K2); p->l2a_b = part((int64_t)p->nc_m2 * E * N);
+    p->l2b_w = part((int64_t)p->nc_m2 * E * K2);     p->l2b_b = part((int64_t)p->nc_m2 * E);
+    p->l1_w = part((int64_t)p->nc_m1 * p->ld1 * S);  p->l1_b = part((int64_t)p->nc_m1 * p->ld1);
+    p->v2 = part((int64_t)p->nblk * (E + 1));
+    p->norm = part(ceil_div64(mixer_layout(mixer, S, N, E, HE).total, GRED_EPB));
+    p->parts = take(q);
+    p->total = o;
+    return 0;
+}
+
+extern "C" int64_t mal_mixer_backward_workspace(int32_t mixer, int32_t B, int32_t T, int32_t N, int32_t S, int32_t E, int32_t HE) {
+    MixerBwdPlan p;
+    if (mixer_bwd_plan(mixer, B, T, N, S, E, HE, &p)) return -1;
+    return p.total;
+}
+
+extern "C" int mal_mixer_backward(int32_t mixer, int32_t B, int32_t T, int32_t N, int32_t S, int32_t E, int32_t HE,
+                                  const float *params, const float *agent_qs, const float *states, int64_t state_sb,
+                                  int64_t state_st, const float *scratch, const float *d_q_tot, float *d_agent_qs,
+                                  float *d_params, void *workspace, void *stream) {
+    MixerBwdPlan p;
+    if (int rc = mixer_bwd_plan(mixer, B, T, N, S, E, HE, &p)) return rc;
+    MAL_REQUIRE(params && agent_qs && states && scratch && d_q_tot && d_agent_qs && d_params && workspace,
+                "mal_mixer_backward: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    uint8_t *ws = (uint8_t *)workspace;
+    auto F = [&](int64_t off) { return reinterpret_cast<float *>(ws + off); };
+    const int64_t BT = (int64_t)B * T;
+    const MixerLayout ML = mixer_layout(mixer, S, N, E, HE);
+    const float *y1 = scratch, *a2 = scratch + BT * p.ld1;      // mal_mixer_forward's scratch layout
+    float *d_a2 = F(p.d_a2), *d_y1 = F(p.d_y1), *parts = F(p.parts);
+    MixBwdArgs m;
+    m.mixer = mixer; m.B = B; m.T = T; m.N = N; m.E = E; m.HE = HE; m.S = S;
+    m.params = params; m.agent_qs = agent_qs; m.y1 = y1; m.a2 = a2; m.d_q_tot = d_q_tot;
+    m.d_agent_qs = d_agent_qs; m.d_a2 = d_a2; m.d_y1 = d_y1; m.part_v2 = parts + p.v2;
+    { ProfScope _ps("k_mix_bwd", st); k_mix_bwd<<<p.nblk, 256, 0, st>>>(m); }
+    MAL_LAUNCH_CHECK("k_mix_bwd");
+    BatchView bv;
+    memset(&bv, 0, sizeof(bv));
+    bv.B = B; bv.T = T; bv.TT = T; bv.N = N; bv.S = S; bv.R = B * N;
+    bv.state.ptr = states; bv.state.sb = state_sb; bv.state.st = state_st;
+    HyperBwd h;
+    h.mixer = mixer; h.two = p.two; h.N = N; h.E = E; h.HE = HE; h.S = S; h.ld1 = p.ld1; h.ld2 = p.ld2; h.BT = BT;
+    h.d_a2 = d_a2; h.d_y1 = d_y1; h.y1 = y1;
+    h.wt1 = params + ML.w1b_w; h.wtf = params + ML.wfb_w; h.ldw1 = HE; h.ldwf = HE; h.w_trans = 1;   // W(n,k) = W_2[k, n]
+    h.l2a_w = parts + p.l2a_w; h.l2a_b = parts + p.l2a_b; h.l2b_w = parts + p.l2b_w; h.l2b_b = parts + p.l2b_b;
+    h.l1_w = parts + p.l1_w; h.l1_b = parts + p.l1_b;
+    h.nc_m2 = p.nc_m2; h.rpc_m2 = p.rpc_m2; h.nc_m1 = p.nc_m1; h.rpc_m1 = p.rpc_m1;
+    if (int rc = launch_hyper_bwd(h, bv, st)) return rc;
+    GradReduceArgs g;
+    memset(&g, 0, sizeof(g));
+    int n = 0;
+    auto seg = [&](int64_t off, int64_t count, const float *part, int n_chunks, int64_t stride) {
+        g.s[n].grad_off = off; g.s[n].count = (int)count; g.s[n].part = part; g.s[n].n_chunks = n_chunks; g.s[n].chunk_stride = stride; ++n;
+    };
+    const int K2 = p.two ? HE : S;
+    const int64_t l1w = (int64_t)p.ld1 * S;
+    const int b1row = p.two ? 2 * HE : 0;
+    const float *pl1w = parts + p.l1_w, *pl1b = parts + p.l1_b;
+    if (p.two) {
+        seg(ML.w1a_w, (int64_t)HE * S, pl1w, p.nc_m1, l1w);
+        seg(ML.w1a_b, HE, pl1b, p.nc_m1, p.ld1);
+    }
+    seg(ML.w1b_w, (int64_t)E * N * K2, parts + p.l2a_w, p.nc_m2, (int64_t)E * N * K2);
+    seg(ML.w1b_b, E * N, parts + p.l2a_b, p.nc_m2, E * N);
+    if (p.two) {
+        seg(ML.wfa_w, (int64_t)HE * S, pl1w + (int64_t)HE * S, p.nc_m1, l1w);
+        seg(ML.wfa_b, HE, pl1b + HE, p.nc_m1, p.ld1);
+    }
+    seg(ML.wfb_w, (int64_t)E * K2, parts + p.l2b_w, p.nc_m2, (int64_t)E * K2);
+    seg(ML.wfb_b, E, parts + p.l2b_b, p.nc_m2, E);
+    seg(ML.b1_w, (int64_t)E * S, pl1w + (int64_t)b1row * S, p.nc_m1, l1w);
+    seg(ML.b1_b, E, pl1b + b1row, p.nc_m1, p.ld1);
+    seg(ML.v0_w, (int64_t)E * S, pl1w + (int64_t)(b1row + E) * S, p.nc_m1, l1w);
+    seg(ML.v0_b, E, pl1b + b1row + E, p.nc_m1, p.ld1);
+    seg(ML.v2_w, E, parts + p.v2, p.nblk, E + 1);
+    seg(ML.v2_b, 1, parts + p.v2 + E, p.nblk, E + 1);
+    g.n = n; g.total = ML.total; g.grad = d_params; g.norm_part = parts + p.norm; g.scalars = nullptr; g.unnormalized = 1;
+    { ProfScope _ps("k_grad_reduce", st); launch_k(k_grad_reduce, dim3((unsigned)ceil_div64(ML.total, GRED_EPB)), dim3(256), 0, st, false, g); }
+    MAL_LAUNCH_CHECK("k_grad_reduce");
     return 0;
 }
 

@@ -40,7 +40,7 @@ class QLearner(Learner):
         self.mixer = None
         if args.mixer is not None:
             if args.mixer == "vdn":
-                self.mixer = VDNMixer()
+                self.mixer = VDNMixer(args)
             elif args.mixer == "qmix":
                 self.mixer = QMixer(args)
             else:

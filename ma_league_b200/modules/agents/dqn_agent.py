@@ -9,6 +9,7 @@ import torch.nn as nn
 
 from ... import _native as nat
 from ...flat import ensure_flat
+from .. import autograd as ag
 from .agent_network import AgentNetwork
 
 
@@ -33,8 +34,16 @@ class DQNAgentNetwork(AgentNetwork):
         return th.zeros(self.args.batch_size, 1, 1, device=self.args.device)
 
     def forward(self, inputs, hidden_states):
-        """inputs [rows, input_shape] -> (q [rows, A], hidden_states unchanged).  Inference only."""
+        """inputs [rows, input_shape] -> (q [rows, A], hidden_states unchanged).  Records an autograd node under
+        `args.autograd_forward` (modules/autograd.py)."""
         x = nat.require_cuda(inputs, "inputs")
+        if ag.recording(self, x, *self.parameters()):
+            ag._reject_input_grad(x, "agent input")
+            x = x.detach().float().contiguous()
+            cfg = dict(rows=x.shape[0], N=1, OBS=self.input_shape, A=self.args.n_actions, dense_input=nat.STEP_DENSE,
+                       obs_ptr=x.data_ptr(), obs_sb=x.stride(0), last_ptr=None, last_sb=0)
+            with th.cuda.device(x.device):
+                return ag.agent_step(self, cfg, x, None, None), hidden_states
         if x.dtype != th.float32 or x.stride(-1) != 1:
             x = x.float().contiguous()
         rows = x.shape[0]

@@ -8,6 +8,7 @@ import torch.nn as nn
 
 from ... import _native as nat
 from ...flat import ensure_flat
+from .. import autograd as ag
 from .agent_network import AgentNetwork
 
 
@@ -33,8 +34,20 @@ class DRQNAgentNetwork(AgentNetwork):
 
     def forward(self, inputs, hidden_state):
         """inputs [rows, input_shape] (already assembled), hidden_state [..., 64] -> (q [rows, A], h' [rows, 64]).
-        Inference only: the learner differentiates through its own fused path, not through this call."""
+        Records an autograd node under `args.autograd_forward` (modules/autograd.py); the learner differentiates through
+        its own fused path, not through this call."""
         x = nat.require_cuda(inputs, "inputs")
+        if ag.recording(self, x, hidden_state, *self.parameters()):
+            ag._reject_input_grad(x, "agent input")
+            x = x.detach().float().contiguous()
+            h = hidden_state.reshape(-1, nat.HID)
+            if h.shape[0] != x.shape[0]:
+                h = h.expand(x.shape[0], nat.HID)
+            h = h.float().contiguous()
+            cfg = dict(rows=x.shape[0], N=1, OBS=self.input_shape, A=self.args.n_actions, dense_input=nat.STEP_DENSE,
+                       obs_ptr=x.data_ptr(), obs_sb=x.stride(0), last_ptr=None, last_sb=0)
+            with th.cuda.device(x.device):
+                return ag.agent_step(self, cfg, x, None, h)
         if x.dtype != th.float32 or x.stride(-1) != 1:
             x = x.float().contiguous()
         rows = x.shape[0]

@@ -9,6 +9,7 @@ import torch.nn as nn
 
 from ... import _native as nat
 from ...flat import ensure_flat
+from .. import autograd as ag
 
 
 class QMixer(nn.Module):
@@ -50,7 +51,13 @@ class QMixer(nn.Module):
         return ensure_flat(self)
 
     def forward(self, agent_qs, states):
-        """agent_qs [B,T,N], states [B,T,S] -> q_tot [B,T,1] (inference; the learner uses its fused path)."""
+        """agent_qs [B,T,N], states [B,T,S] -> q_tot [B,T,1].  Records an autograd node under `args.autograd_forward`
+        (modules/autograd.py); the learner uses its fused path."""
+        if ag.recording(self, agent_qs, states, *self.parameters()):
+            ag._reject_input_grad(states, "states")
+            q = nat.require_cuda(agent_qs, "agent_qs").float().contiguous()
+            s = states if (states.dtype == th.float32 and states.stride(-1) == 1) else states.float().contiguous()
+            return ag.QMix.apply(self, q, s, *self.parameters())
         q = nat.require_cuda(agent_qs, "agent_qs").float().contiguous()
         B, T, N = q.shape
         s = states

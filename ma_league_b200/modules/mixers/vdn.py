@@ -3,10 +3,17 @@ import torch as th
 import torch.nn as nn
 
 from ... import _native as nat
+from .. import autograd as ag
 
 
 class VDNMixer(nn.Module):
+    def __init__(self, args=None):
+        super().__init__()
+        self.args = args          # only `autograd_forward` is read (the reference's VDNMixer takes no arguments)
+
     def forward(self, agent_qs, batch):
+        if ag.recording(self, agent_qs):
+            return ag.VDN.apply(nat.require_cuda(agent_qs, "agent_qs").float().contiguous())
         q = nat.require_cuda(agent_qs, "agent_qs")
         B, T, N = q.shape
         q = q.float().contiguous()
