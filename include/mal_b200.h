@@ -32,6 +32,7 @@ extern "C" {
 #define MAL_HID 64
 #define MAL_MAX_ACTIONS 32
 #define MAL_MAX_EMBED 32
+#define MAL_MAX_POLICIES 1024   /* n_policies cap of the per-match policy entries (the schedule kernel's shared memory) */
 
 /* A scheme field of an EpisodeBatch (marl/components/episode_batch.py:89-143):
  * tensor [B, TT, *inner] whose inner dims are contiguous; sb/st are the batch / time strides
@@ -254,6 +255,35 @@ typedef struct mal_rollout_io {
 int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
                      const mal_rollout_io_t *io, const float *h_in, float *h_out, float *q, const mal_select_t *sel,
                      void *stream);
+
+/* Per-match policies: one rollout / act-select launch over `bs` matches in which match b plays its own entry of a table of
+ * agents (a league opponent per match, or every pairing of a population in cross-play).  `table` is [n_policies, table_ld]
+ * fp32, row k = the flat parameters of agent k in state_dict order (DeviceAgentPool.pool, agent.flat_params()); table_ld
+ * >= the agent's parameter count and may be odd (4-byte alignment is enough).  The table is read at every step, never
+ * copied.  Recurrent agent (MAL_AGENT_RNN) only; 1 <= n_policies <= MAL_MAX_POLICIES.
+ *
+ * mal_policy_schedule_bytes: host-only (no device needed): size of the schedule buffer for (bs, n_agents, n_policies),
+ *   -1 with mal_last_error set for arguments the entries reject.
+ * mal_policy_schedule: ONE launch, once per assignment: match_policy [bs] (int32, device) -> `schedule` (a caller-owned,
+ *   16-byte aligned device buffer of mal_policy_schedule_bytes; its content is internal to the library).  An id outside
+ *   [0, n_policies) sets *status (device int, may be NULL) to 1 and its match is left out: no step reads its rows or
+ *   anything outside the table.
+ * mal_agent_step_pool / mal_rollout_step_pool: mal_agent_step / mal_rollout_step (every argument means what it means
+ *   there; rows = bs * n_agents) with match b's rows computed from table row match_policy[b].  Row indices of inputs,
+ *   hidden states, outputs, avail rows and Philox draws are unchanged, so each match gets bit for bit what the plain entry
+ *   computes over the whole batch with its policy.  The schedule must have been built for the same bs, n_agents and
+ *   n_policies (a CTA that finds another shape in it computes nothing). */
+int64_t mal_policy_schedule_bytes(int32_t bs, int32_t n_agents, int32_t n_policies);
+int mal_policy_schedule(const int32_t *match_policy, int32_t bs, int32_t n_agents, int32_t n_policies,
+                        void *schedule, int32_t *status, void *stream);
+int mal_agent_step_pool(const float *table, int64_t table_ld, int32_t n_policies, const void *schedule,
+                        int32_t rows, int32_t n_agents, int32_t obs_dim, int32_t n_actions, int32_t dense_input,
+                        const float *obs, int64_t obs_sb, const float *last_onehot, int64_t onehot_sb,
+                        const float *h_in, float *h_out, float *q, const mal_select_t *sel, void *stream);
+int mal_rollout_step_pool(const float *table, int64_t table_ld, int32_t n_policies, const void *schedule,
+                          int32_t bs, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
+                          const mal_rollout_io_t *io, const float *h_in, float *h_out, float *q,
+                          const mal_select_t *sel, void *stream);
 
 /* Launch counters per kernel flavour since process start, for tests that assert which variant the launch heuristics
  * picked: "linear_tc2" (pipelined tcgen05 GEMM), "linear_tc", "reduce_tc", "reduce_tc_swap", "reduce_ffma",

@@ -25,6 +25,7 @@ SC_RAW0 = 8     # raw sums: sum mtd^2, sum |mtd|, sum q_tot*m, sum targets*m, su
 HID = 64
 MAX_ACTIONS = 32
 MAX_EMBED = 32
+MAX_POLICIES = 1024                          # n_policies cap of the per-match policy entries (MAL_MAX_POLICIES)
 
 
 class MalError(RuntimeError):
@@ -118,6 +119,14 @@ _PROTOS = {
                                  C.POINTER(Select), C.c_void_p]),
     "mal_rollout_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(RolloutIO), C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.POINTER(Select), C.c_void_p]),
+    "mal_policy_schedule_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
+    "mal_policy_schedule": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mal_agent_step_pool": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                      C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.POINTER(Select), C.c_void_p]),
+    "mal_rollout_step_pool": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                        C.c_int32, C.POINTER(RolloutIO), C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.POINTER(Select), C.c_void_p]),
     "mal_mixer_forward": (C.c_int, [C.c_int32] * 7 + [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                                                       C.c_void_p, C.c_void_p, C.c_void_p]),
     "mal_agent_step_backward_workspace": (C.c_int64, [C.c_int32] * 6),

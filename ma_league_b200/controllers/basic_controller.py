@@ -4,6 +4,9 @@
 Philox), `forward` the same kernel without the selection tail.  The reference's hooks (`_build_inputs`,
 `_compute_agent_outputs`, `_build_agent`, `_get_input_shape`) are kept: a subclass that overrides the first two is
 served through them (dense-input kernel) instead of the fused path.
+
+`set_match_policies(table, ids)` makes match b of the batch play row ids[b] of a [K, P] table of flat agent buffers
+(league opponents, cross-play pairings) instead of the controller's own agent: still one launch per step.
 """
 from __future__ import annotations
 
@@ -15,6 +18,7 @@ import torch as th
 from .. import _native as nat
 from ..components.action_selectors import make_select_struct
 from ..exceptions import HiddenStateNotInitialized
+from ..flat import ensure_flat
 from ..modules import autograd as ag
 from ..modules.agents import REGISTRY as agent_REGISTRY
 from ..modules.agents.drqn_agent import DRQNAgentNetwork
@@ -26,6 +30,70 @@ class BasicMAC(MultiAgentController):
     def __init__(self, scheme, groups, args):
         super().__init__(scheme, groups, args)
         self._obs_dim = scheme["obs"]["vshape"] if isinstance(scheme["obs"]["vshape"], int) else scheme["obs"]["vshape"][0]
+        self._pool = None           # set_match_policies: (table, ids on the device, schedule buffer)
+
+    # ------------------------------------------------------------------ per-match policies
+    def set_match_policies(self, table, ids=None):
+        """Make match b play with the agent in row `ids[b]` of `table` instead of `self.agent`; `set_match_policies(None)`
+        goes back to the controller's own agent.
+
+        `table` is a [K, P] float32 CUDA tensor whose rows are flat agent buffers in state_dict order (e.g.
+        `DeviceAgentPool.pool`, rows of `agent.flat_params()`), P = this agent's parameter count; `ids` holds one policy
+        per match (a sequence, CPU or CUDA tensor).  The ids are checked and bucketed by policy here, once per assignment
+        (one launch); the table itself is read at every step and never copied, so a `pool.sync()` (or any in-place write
+        to the table) between steps takes effect at the next step.  While policies are set, `select_actions`,
+        `rollout_step` and `forward` run the pooled kernels (still one launch per step), `init_hidden` must be called with
+        `len(ids)` matches, and nothing records an autograd node: the pooled path reads no parameter of `self.agent`.
+        Recurrent agent only."""
+        if table is None:
+            self._pool = None
+            return
+        if not isinstance(table, th.Tensor) or not table.is_cuda:
+            raise nat.MalError("the policy table must be a CUDA tensor: the B200 path has no CPU fallback")
+        if not self._rollout_fusable():
+            raise nat.MalError("per-match policies need the fused recurrent agent path (not the dqn agent or a subclass "
+                               "that overrides the input hooks)")
+        if getattr(self, "ensemble", None):
+            raise nat.MalError("per-match policies do not run ensemble agents")
+        if table.dim() != 2 or table.dtype != th.float32 or table.stride(1) != 1:
+            raise nat.MalError("the policy table must be a [K, P] float32 tensor with contiguous rows")
+        n_params = ensure_flat(self.agent).numel()
+        if table.shape[1] != n_params:
+            raise ValueError("agent architectures differ: %d vs %d parameters" % (table.shape[1], n_params))
+        K = table.shape[0]
+        if not 1 <= K <= nat.MAX_POLICIES:
+            raise ValueError("the policy table must have between 1 and %d rows, got %d" % (nat.MAX_POLICIES, K))
+        ids = th.as_tensor(ids).reshape(-1)
+        if ids.numel() == 0 or ids.is_floating_point() or ids.dtype == th.bool:
+            raise ValueError("ids must hold one integer policy per match")
+        if int(ids.min()) < 0 or int(ids.max()) >= K:
+            raise ValueError("policy ids must be in [0, %d)" % K)
+        dev = table.device
+        bs = ids.numel()
+        ids_dev = ids.to(device=dev, dtype=th.int32)
+        lib = nat.lib()
+        nbytes = lib.mal_policy_schedule_bytes(bs, self.n_agents, K)
+        if nbytes < 0:
+            raise nat.MalError(lib.mal_last_error().decode())
+        sched = th.empty((nbytes + 3) // 4, dtype=th.int32, device=dev)
+        with nat.on_device(dev):
+            nat.check(lib.mal_policy_schedule(ids_dev.data_ptr(), bs, self.n_agents, K, sched.data_ptr(), None,
+                                              nat.current_stream(dev)), "mal_policy_schedule")
+        self._pool = (table, ids_dev, sched)
+
+    @property
+    def match_policies(self):
+        """The per-match policy ids set by `set_match_policies` (int32 device tensor), or None."""
+        return None if self._pool is None else self._pool[1]
+
+    def _pool_args(self, dev, B):
+        """(table ptr, table_ld, K, schedule ptr) of the pooled launches for a batch of B matches on `dev`."""
+        table, ids, sched = self._pool
+        if table.device != dev:
+            raise nat.MalError("the policy table lives on %s, the batch on %s" % (table.device, dev))
+        if B != ids.numel():
+            raise nat.MalError("per-match policies were set for %d matches, the batch has %d" % (ids.numel(), B))
+        return table.data_ptr(), table.stride(0), table.shape[0], sched.data_ptr()
 
     # ------------------------------------------------------------------ public API
     def select_actions(self, ep_batch, t_ep, t_env, bs=slice(None), test_mode=False, u=None, e=None):
@@ -121,10 +189,15 @@ class BasicMAC(MultiAgentController):
         buf = th.empty(rows * (A + nat.HID), dtype=th.float32, device=dev)       # q | h_out, one allocation
         q = buf[:rows * A].view(B, N, A)
         h_out = buf[rows * A:].view(rows, nat.HID)
-        flat = self.agent.flat_params()
         with nat.on_device(dev):
-            nat.check(nat.lib().mal_rollout_step(flat.data_ptr(), B, N, OBS, A, C.byref(io), h_ptr, h_out.data_ptr(),
-                                                 q.data_ptr(), C.byref(s), nat.current_stream(dev)), "mal_rollout_step")
+            if self._pool is not None:
+                nat.check(nat.lib().mal_rollout_step_pool(*self._pool_args(dev, B), B, N, OBS, A, C.byref(io), h_ptr,
+                                                          h_out.data_ptr(), q.data_ptr(), C.byref(s), nat.current_stream(dev)),
+                          "mal_rollout_step_pool")
+            else:
+                flat = self.agent.flat_params()
+                nat.check(nat.lib().mal_rollout_step(flat.data_ptr(), B, N, OBS, A, C.byref(io), h_ptr, h_out.data_ptr(),
+                                                     q.data_ptr(), C.byref(s), nat.current_stream(dev)), "mal_rollout_step")
         self.hidden_states = h_out
         if status is not None and int(status.item()) != 0:
             raise ValueError("Expected at least one available action per agent (Categorical probs are all zero)")
@@ -134,6 +207,11 @@ class BasicMAC(MultiAgentController):
         """Q-values [bs, N, A] of timestep t.  Under `args.autograd_forward` (grad mode on, agent parameters or the hidden
         state requiring grad) the step records an autograd node (modules/autograd.py), so that a loss over the outputs can
         be back-propagated into the agent's parameters through time."""
+        if self._pool is not None:
+            if getattr(self.args, "autograd_forward", False) and th.is_grad_enabled():
+                raise nat.MalError("forward with per-match policies records no autograd node (it reads no parameter of "
+                                   "the agent); call it under torch.no_grad() or clear the policies")
+            return self._step(ep_batch, t, None)
         if self._fusable():
             if self.hidden_states is not None and ag.recording(self, self.hidden_states, *self.agent.parameters()):
                 return self._step_recorded(ep_batch, t)
@@ -145,6 +223,7 @@ class BasicMAC(MultiAgentController):
         return agent_outs.view(ep_batch.batch_size, self.n_agents, -1)
 
     def init_hidden(self, batch_size):
+        self._check_pool_batch(batch_size)
         if isinstance(self.agent, DQNAgentNetwork):
             # The reference's expand() of the 3-D placeholder (basic_controller.py:59-60 on dqn_agent.py:27-32) raises a
             # RuntimeError, i.e. the "dqn" agent cannot be rolled out or trained there; here the placeholder is a
@@ -152,6 +231,10 @@ class BasicMAC(MultiAgentController):
             self.hidden_states = th.zeros(batch_size, self.n_agents, 1, device=self.args.device)
             return
         self.hidden_states = self.agent.init_hidden().unsqueeze(0).expand(batch_size, self.n_agents, -1)
+
+    def _check_pool_batch(self, batch_size):
+        if self._pool is not None and batch_size != self._pool[1].numel():
+            raise nat.MalError("per-match policies were set for %d matches, init_hidden(%d)" % (self._pool[1].numel(), batch_size))
 
     def update_trained_steps(self, update):
         if isinstance(update, th.Tensor):   # device-side count: accumulate without a host sync
@@ -288,11 +371,16 @@ class BasicMAC(MultiAgentController):
         buf = th.empty(rows * (A + nat.HID), dtype=th.float32, device=dev)      # q | h_out, one allocation
         q = buf[:rows * A].view(B, N, A)
         h_out = buf[rows * A:].view(rows, nat.HID)
-        flat = self.agent.flat_params()
+        sel = C.byref(select_struct) if select_struct is not None else None
         with nat.on_device(dev):
-            nat.check(nat.lib().mal_agent_step(
-                flat.data_ptr(), rows, N, OBS, A, flags << 1, obs_ptr, obs_all.stride(0), last_ptr, last_sb, h_ptr,
-                h_out.data_ptr(), q.data_ptr(), C.byref(select_struct) if select_struct is not None else None,
-                nat.current_stream(dev)), "mal_agent_step")
+            if self._pool is not None:
+                nat.check(nat.lib().mal_agent_step_pool(
+                    *self._pool_args(dev, B), rows, N, OBS, A, flags << 1, obs_ptr, obs_all.stride(0), last_ptr, last_sb,
+                    h_ptr, h_out.data_ptr(), q.data_ptr(), sel, nat.current_stream(dev)), "mal_agent_step_pool")
+            else:
+                flat = self.agent.flat_params()
+                nat.check(nat.lib().mal_agent_step(
+                    flat.data_ptr(), rows, N, OBS, A, flags << 1, obs_ptr, obs_all.stride(0), last_ptr, last_sb, h_ptr,
+                    h_out.data_ptr(), q.data_ptr(), sel, nat.current_stream(dev)), "mal_agent_step")
         self.hidden_states = h_out
         return q

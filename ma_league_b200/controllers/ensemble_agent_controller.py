@@ -41,6 +41,8 @@ class EnsembleMAC(BasicMAC):
     def forward(self, ep_batch, t, test_mode=False):
         if self.native_hidden_states is None:
             raise HiddenStateNotInitialized()
+        if self.ensemble and self._pool is not None:
+            raise MalError("per-match policies do not run ensemble agents")
         if self.ensemble and getattr(self.args, "autograd_forward", False) and th.is_grad_enabled():
             raise MalError("EnsembleMAC.forward does not record autograd nodes for ensemble agents (a fixed-policy opponent); "
                            "call it under torch.no_grad() or switch args.autograd_forward off")
@@ -57,6 +59,7 @@ class EnsembleMAC(BasicMAC):
         return agent_outs
 
     def init_hidden(self, batch_size):
+        self._check_pool_batch(batch_size)
         self.native_hidden_states = self.agent.init_hidden().unsqueeze(0).expand(batch_size, self.n_agents, -1)
         self.hidden_states = self.native_hidden_states
         self.ensemble_hidden_states = {aid: agent.init_hidden().unsqueeze(0).expand(batch_size, 1, -1)

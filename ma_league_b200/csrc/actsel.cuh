@@ -136,12 +136,137 @@ __device__ __forceinline__ void select_row(const SelectArgs &s, int row, int A, 
     select_core(s, row, A, lane, qv, select_avail(s, row, A, lane), ev, uu, io);
 }
 
-// Per-match part of the fused rollout step (rows r0 .. r0+AS_ROWS-1 of this CTA; the row with n == 0 acts for its match):
+// ---------------------------------------------------------------------------------------------
+// Per-match policies (league rollouts / cross-play): one launch steps B matches that each play their own entry of a
+// [K, table_ld] table of flat agent buffers.  k_policy_schedule buckets the matches by policy once per assignment and
+// writes a work list; CTA c of a pooled step kernel (template parameter POOL) then runs entry c: the policy whose
+// parameters it reads and up to AS_ROWS agent rows of matches that play it.  Every row keeps its ORIGINAL index for
+// inputs, hidden state, outputs, avail rows and Philox draws, so a pooled step computes for each match exactly what the
+// plain step computes over the whole batch with that match's parameters.
+//
+// Schedule buffer (int32, internal to the library; mal_policy_schedule_bytes sizes it):
+//   header [PS_HDR]:      used CTAs, rows (bs * N), n_agents, n_policies, 0...
+//   entries [PS_ENT] each: row[0..7] (-1: padding, always at the end), policy, 0...
+// ---------------------------------------------------------------------------------------------
+#define PS_HDR 16
+#define PS_ENT 16
+#define PS_THREADS 1024
+static_assert(MAL_MAX_POLICIES <= PS_THREADS, "k_policy_schedule scans one policy per thread");
+
+// the row of local slot r of this CTA: r0 + r, or the work list's entry (padding and anything outside [0, rows) -> rows,
+// which every `row < rows` test of the step kernels skips)
+template <bool POOL>
+__device__ __forceinline__ int cta_row(int r0, const int32_t *rl, int r, int rows) {
+    if constexpr (POOL) {
+        const int v = __ldg(rl + r);
+        return (v >= 0 && v < rows) ? v : rows;
+    } else {
+        return r0 + r;
+    }
+}
+// two consecutive parameters: one 8-byte load in the plain kernels (flat_params() is 16-byte aligned); a pooled table row
+// starts at policy * table_ld floats, which need not be even
+template <bool POOL>
+__device__ __forceinline__ float2 ldg_f2(const float2 *p) {
+    if constexpr (POOL) {
+        const float *f = reinterpret_cast<const float *>(p);
+        return make_float2(__ldg(f), __ldg(f + 1));
+    } else {
+        return __ldg(p);
+    }
+}
+// Pooled CTA set-up: false when the CTA has nothing to do (past the used count, a schedule built for another shape, or a
+// policy outside the table), else P = this CTA's table row and rl = its row list.  Called before any barrier.
+__device__ __forceinline__ bool pool_cta(const float *&P, const int32_t *&rl, const float *table, int64_t table_ld,
+                                         int n_policies, const int32_t *sched, int rows, int N) {
+    const int4 h = __ldg(reinterpret_cast<const int4 *>(sched));
+    if ((int)blockIdx.x >= h.x || h.y != rows || h.z != N || h.w != n_policies) return false;
+    rl = sched + PS_HDR + (int64_t)blockIdx.x * PS_ENT;
+    const int p = __ldg(rl + AS_ROWS);
+    if (p < 0 || p >= n_policies) return false;
+    P = table + (int64_t)p * table_ld;
+    return true;
+}
+
+// One CTA: match_policy[bs] -> work list.  A stable counting sort by policy: bucket p's rows are those of its matches in
+// match order (each match's N rows consecutive), cut into CTAs of AS_ROWS.  sum over p of ceil(rows_p / 8) is at most
+// ceil(rows / 8) + min(K, bs) - 1, the grid the pooled launch uses.  An id outside [0, K) sets *status and its match's
+// rows are left out of the list.
+__global__ void __launch_bounds__(PS_THREADS) k_policy_schedule(const int32_t *mp, int bs, int N, int K, int32_t *sched,
+                                                                 int32_t *status) {
+    __shared__ int cnt[MAL_MAX_POLICIES], end[MAL_MAX_POLICIES], run[MAL_MAX_POLICIES];
+    __shared__ int wsum[PS_THREADS / 32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int p = tid; p < K; p += PS_THREADS) { cnt[p] = 0; run[p] = 0; }
+    __syncthreads();
+    for (int b = tid; b < bs; b += PS_THREADS) {
+        const int p = mp[b];
+        if (p >= 0 && p < K) atomicAdd(&cnt[p], 1);
+        else if (status) atomicExch(status, 1);
+    }
+    __syncthreads();
+    // inclusive scan of the CTAs per policy (K <= PS_THREADS: one bucket per thread)
+    int c = tid < K ? (cnt[tid] * N + AS_ROWS - 1) / AS_ROWS : 0;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, c, o); if (lane >= o) c += v; }
+    if (lane == 31) wsum[warp] = c;
+    __syncthreads();
+    if (warp == 0) {
+        int s = wsum[lane];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, s, o); if (lane >= o) s += v; }
+        wsum[lane] = s;
+    }
+    __syncthreads();
+    if (warp > 0) c += wsum[warp - 1];
+    if (tid < K) end[tid] = c;
+    const int used = wsum[PS_THREADS / 32 - 1];
+    if (tid == 0) {
+        sched[0] = used; sched[1] = bs * N; sched[2] = N; sched[3] = K;
+        for (int i = 4; i < PS_HDR; ++i) sched[i] = 0;
+    }
+    __syncthreads();
+    // every used entry: its policy (the first bucket whose CTA range ends after it) and padding rows
+    for (int e = tid; e < used; e += PS_THREADS) {
+        int lo = 0, hi = K - 1;
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (end[mid] > e) hi = mid; else lo = mid + 1; }
+        int32_t *ent = sched + PS_HDR + (int64_t)e * PS_ENT;
+        for (int r = 0; r < AS_ROWS; ++r) ent[r] = -1;
+        ent[AS_ROWS] = lo;
+        for (int r = AS_ROWS + 1; r < PS_ENT; ++r) ent[r] = 0;
+    }
+    __syncthreads();
+    // one warp places the matches in order: the rank of a match in its bucket = matches of that policy before it
+    if (warp == 0) {
+        for (int b0 = 0; b0 < bs; b0 += 32) {
+            const int b = b0 + lane;
+            const int p = b < bs ? mp[b] : -1;
+            const bool ok = p >= 0 && p < K;
+            const unsigned same = __match_any_sync(0xffffffffu, ok ? p : -1);
+            const int base = ok ? run[p] : 0;
+            __syncwarp();
+            if (ok) {
+                const int rank = base + __popc(same & ((1u << lane) - 1));
+                if ((same & ((1u << lane) - 1)) == 0) run[p] = base + __popc(same);
+                const int e0 = p > 0 ? end[p - 1] : 0;                  // bucket p's first entry
+                for (int n = 0; n < N; ++n) {
+                    const int pos = rank * N + n;                        // row slot within the bucket
+                    sched[PS_HDR + (int64_t)(e0 + pos / AS_ROWS) * PS_ENT + pos % AS_ROWS] = b * N + n;
+                }
+            }
+            __syncwarp();
+        }
+    }
+}
+
+// Per-match part of the fused rollout step (rows of this CTA; the row with n == 0 acts for its match):
 // state / filled at t, reward / terminated at t-1.
-__device__ __forceinline__ void rollout_match_fields(const RolloutIO &io, int r0, int rows, int N, int tid, int nthreads) {
+template <bool POOL = false>
+__device__ __forceinline__ void rollout_match_fields(const RolloutIO &io, int r0, int rows, int N, int tid, int nthreads,
+                                                     const int32_t *rl = nullptr) {
     for (int r = 0; r < AS_ROWS; ++r) {
-        const int row = r0 + r;
-        if (row >= rows) break;
+        const int row = cta_row<POOL>(r0, rl, r, rows);
+        if (row >= rows) { if (POOL) continue; break; }
         const int b = row / N;
         if (row - b * N != 0) continue;
         for (int k = tid; k < io.S; k += nthreads) io.state_t[(int64_t)b * io.state_sb + k] = io.env_state[(int64_t)b * io.env_state_sb + k];
@@ -200,12 +325,15 @@ struct AgentStepArgs {
     int do_select;
     SelectArgs sel;
     RolloutIO io;
+    // pooled instances only (POOL = true): params is the [n_policies, table_ld] table, sched the work list
+    const int32_t *sched; int64_t table_ld; int n_policies;
 };
 
 // Latency plan: a CTA needs every weight exactly once, and nothing but the inputs depends on anything, so ALL
 // global loads (inputs, 48 GRU weight rows per warp, fc1 / fc2 rows, biases) are issued back to back at kernel entry
 // into registers; the phases below then only touch registers and shared memory.
 #define AS_FC1_MAXK 7    // ceil(224 / 32): obs+action columns handled per lane
+template <bool POOL>
 __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
     extern __shared__ float as_smem[];
     const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.in.last + a.in.id, a.A);
@@ -220,6 +348,8 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int r0 = blockIdx.x * AS_ROWS;
     const float *P = a.params;
+    const int32_t *rl = nullptr;
+    if constexpr (POOL) { if (!pool_cta(P, rl, a.params, a.table_ld, a.n_policies, a.sched, a.rows, a.N)) return; }
 
     // ---- issue every global load up front ---------------------------------------------------------------------
     float2 wg[2 * G3 / AS_WARPS];                // GRU rows warp, warp+8, ... of [W_ih ; W_hh]   (48 x float2)
@@ -228,7 +358,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
         const int jj = warp + AS_WARPS * i;
         const bool hh = jj >= G3;
         const int j = hh ? jj - G3 : jj;
-        wg[i] = __ldg(reinterpret_cast<const float2 *>(P + (hh ? L.w_hh : L.w_ih) + (int64_t)j * HID) + lane);
+        wg[i] = ldg_f2<POOL>(reinterpret_cast<const float2 *>(P + (hh ? L.w_hh : L.w_ih) + (int64_t)j * HID) + lane);
     }
     float w1[HID / AS_WARPS][AS_FC1_MAXK];       // fc1 rows warp, warp+8, ...; columns lane, lane+32, ...
     float b1x[HID / AS_WARPS];                   // fc1 bias + agent-id column, for the row this lane finalises
@@ -238,7 +368,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
         const float *w = P + L.fc1_w + (int64_t)j * L.d_in;
 #pragma unroll
         for (int c = 0; c < AS_FC1_MAXK; ++c) w1[i][c] = (lane + 32 * c < Kin) ? __ldg(w + lane + 32 * c) : 0.0f;
-        const int row = r0 + (lane >> 2);
+        const int row = cta_row<POOL>(r0, rl, lane >> 2, a.rows);
         const int n = row < a.rows ? row % a.N : 0;
         b1x[i] = __ldg(P + L.fc1_b + j) + (a.in.id ? __ldg(w + Kin + n) : 0.0f);
     }
@@ -250,7 +380,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
         w2[i] = make_float2(0.f, 0.f);
         b2[i] = 0.0f;
         if (j < a.A) {
-            w2[i] = __ldg(reinterpret_cast<const float2 *>(P + L.fc2_w + (int64_t)j * HID) + lane);
+            w2[i] = ldg_f2<POOL>(reinterpret_cast<const float2 *>(P + L.fc2_w + (int64_t)j * HID) + lane);
             b2[i] = __ldg(P + L.fc2_b + j);
         }
     }
@@ -262,7 +392,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
 
     // ---- stage inputs (obs | last action one-hot) and previous hidden state
     for (int idx = tid; idx < AS_ROWS * Kin; idx += AS_THREADS) {
-        int r = idx / Kin, k = idx - r * Kin, row = r0 + r;
+        int r = idx / Kin, k = idx - r * Kin, row = cta_row<POOL>(r0, rl, r, a.rows);
         float v = 0.0f;
         if (row < a.rows) {
             const int b = row / a.N, n = row - b * a.N;
@@ -275,9 +405,9 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
         }
         in_s[r * ldin + k] = v;
     }
-    if (a.io.enabled) rollout_match_fields(a.io, r0, a.rows, a.N, tid, AS_THREADS);
+    if (a.io.enabled) rollout_match_fields<POOL>(a.io, r0, a.rows, a.N, tid, AS_THREADS, rl);
     for (int idx = tid; idx < AS_ROWS * HID; idx += AS_THREADS) {
-        int r = idx >> 6, row = r0 + r;
+        int r = idx >> 6, row = cta_row<POOL>(r0, rl, r, a.rows);
         h_s[idx] = (a.h_in && row < a.rows) ? a.h_in[(int64_t)row * HID + (idx & 63)] : 0.0f;
     }
     __syncthreads();
@@ -324,7 +454,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
 
     // ---- gate math: r,z,n ; h' = n + z (h - n)
     for (int idx = tid; idx < AS_ROWS * HID; idx += AS_THREADS) {
-        int r = idx >> 6, i = idx & 63, row = r0 + r;
+        int r = idx >> 6, i = idx & 63, row = cta_row<POOL>(r0, rl, r, a.rows);
         const float *g = g_s + r * 2 * G3;
         float rr = sigmoidf_acc(g[i] + g[G3 + i] + bir);
         float zz = sigmoidf_acc(g[HID + i] + g[G3 + HID + i] + biz);
@@ -350,7 +480,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
                 for (int r = 0; r < 8; ++r) acc[r] = fmaf(w2[i].y, hv[r][1], w2[i].x * hv[r][0]);
                 float s = warp_fold8(acc, lane);
                 if ((lane & 3) == 0) {
-                    int r = lane >> 2, row = r0 + r;
+                    int r = lane >> 2, row = cta_row<POOL>(r0, rl, r, a.rows);
                     s += b2[i];
                     q_s[r * 32 + j] = s;
                     if (row < a.rows) a.q[(int64_t)row * a.A + j] = s;
@@ -362,7 +492,7 @@ __global__ void __launch_bounds__(AS_THREADS, 1) k_agent_step(AgentStepArgs a) {
     __syncthreads();
     // ---- epsilon-greedy selection: one warp per row
     {
-        int row = r0 + warp;
+        int row = cta_row<POOL>(r0, rl, warp, a.rows);
         if (row < a.rows) select_row(a.sel, row, a.A, lane, lane < a.A ? q_s[warp * 32 + lane] : 0.0f, a.io.enabled ? &a.io : nullptr);
     }
 }
@@ -406,6 +536,7 @@ __device__ __forceinline__ void load_a_frag(float (&av)[4], const float *W, int6
     av[3] = (r1 < M && c1 < K) ? __ldg(W + (int64_t)r1 * ldw + c1) : 0.0f;
 }
 
+template <bool POOL>
 __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs a) {
     extern __shared__ float as_smem[];
     const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.in.last + a.in.id, a.A);
@@ -421,6 +552,8 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
     const int g = lane >> 2, tig = lane & 3;
     const int r0 = blockIdx.x * AS_ROWS;
     const float *P = a.params;
+    const int32_t *rl = nullptr;
+    if constexpr (POOL) { if (!pool_cta(P, rl, a.params, a.table_ld, a.n_policies, a.sched, a.rows, a.N)) return; }
 
     // ---- EVERY global operand of the step is requested here, before the first barrier, so that the kernel pays one
     //      memory round trip: weights of this warp's tiles, biases, the selector's avail flags and draws
@@ -440,7 +573,7 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
             if (q < nks1) load_a_frag(wih[q], P + L.fc1_w, L.d_in, HID, Kin, 16 * warp, q, g, tig);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            const int j = 16 * warp + g + 8 * (i >> 1), row = r0 + 2 * tig + (i & 1);
+            const int j = 16 * warp + g + 8 * (i >> 1), row = cta_row<POOL>(r0, rl, 2 * tig + (i & 1), a.rows);
             const int n = row < a.rows ? row % a.N : 0;
             fb[i] = __ldg(P + L.fc1_b + j) + (a.in.id ? __ldg(P + L.fc1_w + (int64_t)j * L.d_in + Kin + n) : 0.0f);
         }
@@ -458,15 +591,15 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
         biz = __ldg(P + L.b_ih + HID + i) + __ldg(P + L.b_hh + HID + i);
         bin = __ldg(P + L.b_ih + 2 * HID + i); bhn = __ldg(P + L.b_hh + 2 * HID + i);
     }
-    int sel_av = 0;                              // selector operands of row r0 + warp (warps 0-7)
+    int sel_av = 0;                              // selector operands of this CTA's row `warp` (warps 0-7)
     float sel_ev = 1.0f, sel_uu = 1.0f;
-    if (a.do_select && warp < AS_ROWS && r0 + warp < a.rows) {
-        sel_av = select_avail(a.sel, r0 + warp, a.A, lane);
-        select_draws(a.sel, r0 + warp, a.A, lane, sel_ev, sel_uu);     // Philox rounds run under the load latency
+    if (a.do_select && warp < AS_ROWS && cta_row<POOL>(r0, rl, warp, a.rows) < a.rows) {
+        sel_av = select_avail(a.sel, cta_row<POOL>(r0, rl, warp, a.rows), a.A, lane);
+        select_draws(a.sel, cta_row<POOL>(r0, rl, warp, a.rows), a.A, lane, sel_ev, sel_uu);     // Philox rounds run under the load latency
     }
     // ---- stage inputs (obs | last action one-hot, zero padded) and the previous hidden state
     for (int idx = tid; idx < AS_ROWS * ldin; idx += AL_THREADS) {
-        const int r = idx / ldin, k = idx - r * ldin, row = r0 + r;
+        const int r = idx / ldin, k = idx - r * ldin, row = cta_row<POOL>(r0, rl, r, a.rows);
         float v = 0.0f;
         if (row < a.rows && k < Kin) {
             const int b = row / a.N, n = row - b * a.N;
@@ -479,9 +612,9 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
         }
         in_s[idx] = v;
     }
-    if (a.io.enabled) rollout_match_fields(a.io, r0, a.rows, a.N, tid, AL_THREADS);
+    if (a.io.enabled) rollout_match_fields<POOL>(a.io, r0, a.rows, a.N, tid, AL_THREADS, rl);
     for (int idx = tid; idx < AS_ROWS * HID; idx += AL_THREADS) {
-        const int r = idx >> 6, row = r0 + r;
+        const int r = idx >> 6, row = cta_row<POOL>(r0, rl, r, a.rows);
         h_s[r * 68 + (idx & 63)] = (a.h_in && row < a.rows) ? a.h_in[(int64_t)row * HID + (idx & 63)] : 0.0f;
     }
     __syncthreads();
@@ -531,7 +664,7 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
 
     // ---- gate math: r,z,n ; h' = n + z (h - n): one (row, unit) pair per thread
     {
-        const int r = tid >> 6, i = tid & 63, row = r0 + r;
+        const int r = tid >> 6, i = tid & 63, row = cta_row<POOL>(r0, rl, r, a.rows);
         const float *gg = g_s + r * 2 * G3;
         const float rr = sigmoidf_acc(gg[i] + gg[G3 + i] + bir);
         const float zz = sigmoidf_acc(gg[HID + i] + gg[G3 + HID + i] + biz);
@@ -550,7 +683,7 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
         for (int ks = 0; ks < 8; ++ks) mma3(d, whh[ks], hn_s[g * 68 + 8 * ks + tig], hn_s[g * 68 + 8 * ks + tig + 4]);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            const int j = 16 * warp + g + 8 * (i >> 1), r = 2 * tig + (i & 1), row = r0 + r;
+            const int j = 16 * warp + g + 8 * (i >> 1), r = 2 * tig + (i & 1), row = cta_row<POOL>(r0, rl, r, a.rows);
             if (j < a.A) {
                 const float s = d[i] + f2b[i >> 1];
                 q_s[r * 32 + j] = s;
@@ -562,7 +695,7 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
     __syncthreads();
     // ---- epsilon-greedy selection: one warp per row
     if (warp < AS_ROWS) {
-        const int row = r0 + warp;
+        const int row = cta_row<POOL>(r0, rl, warp, a.rows);
         if (row < a.rows) select_core(a.sel, row, a.A, lane, lane < a.A ? q_s[warp * 32 + lane] : 0.0f, sel_av, sel_ev, sel_uu,
                                       a.io.enabled ? &a.io : nullptr);
     }
@@ -570,6 +703,7 @@ __global__ void __launch_bounds__(AL_THREADS, 1) k_agent_step_lat(AgentStepArgs 
 
 // Throughput variant for large row counts (many CTAs per SM): weight rows are streamed from L2 as they are used
 // instead of being parked in 255 registers per thread.
+template <bool POOL>
 __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs a) {
     extern __shared__ float as_smem[];
     const AgentLayout L = agent_layout(a.dense ? a.OBS : a.OBS + a.in.last + a.in.id, a.A, a.kind);
@@ -585,10 +719,12 @@ __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int r0 = blockIdx.x * AS_ROWS;
     const float *P = a.params;
+    const int32_t *rl = nullptr;
+    if constexpr (POOL) { if (!pool_cta(P, rl, a.params, a.table_ld, a.n_policies, a.sched, a.rows, a.N)) return; }
 
     // ---- stage inputs (obs | last action one-hot) and previous hidden state
     for (int idx = tid; idx < AS_ROWS * Kin; idx += AS_THREADS) {
-        int r = idx / Kin, k = idx - r * Kin, row = r0 + r;
+        int r = idx / Kin, k = idx - r * Kin, row = cta_row<POOL>(r0, rl, r, a.rows);
         float v = 0.0f;
         if (row < a.rows) {
             const int b = row / a.N, n = row - b * a.N;
@@ -601,9 +737,9 @@ __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs 
         }
         in_s[r * ldin + k] = v;
     }
-    if (a.io.enabled) rollout_match_fields(a.io, r0, a.rows, a.N, tid, AS_THREADS);
+    if (a.io.enabled) rollout_match_fields<POOL>(a.io, r0, a.rows, a.N, tid, AS_THREADS, rl);
     for (int idx = tid; idx < AS_ROWS * HID; idx += AS_THREADS) {
-        int r = idx >> 6, row = r0 + r;
+        int r = idx >> 6, row = cta_row<POOL>(r0, rl, r, a.rows);
         h_s[idx] = (rnn && a.h_in && row < a.rows) ? a.h_in[(int64_t)row * HID + (idx & 63)] : 0.0f;
     }
     __syncthreads();
@@ -619,7 +755,7 @@ __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs 
         }
         float s = warp_fold8(acc, lane);
         if ((lane & 3) == 0) {
-            int r = lane >> 2, row = r0 + r;
+            int r = lane >> 2, row = cta_row<POOL>(r0, rl, r, a.rows);
             int n = row < a.rows ? row % a.N : 0;
             s += __ldg(P + L.fc1_b + j) + (a.in.id ? __ldg(w + Kin + n) : 0.0f);
             x_s[r * HID + j] = fmaxf(s, 0.0f);
@@ -639,7 +775,7 @@ __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs 
         for (int jj = warp; jj < 2 * G3; jj += AS_WARPS) {
             const bool hh = jj >= G3;
             const int j = hh ? jj - G3 : jj;
-            const float2 wv = __ldg(reinterpret_cast<const float2 *>(P + (hh ? L.w_hh : L.w_ih) + (int64_t)j * HID) + lane);
+            const float2 wv = ldg_f2<POOL>(reinterpret_cast<const float2 *>(P + (hh ? L.w_hh : L.w_ih) + (int64_t)j * HID) + lane);
             float acc[8];
 #pragma unroll
             for (int r = 0; r < 8; ++r)
@@ -655,7 +791,7 @@ __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs 
         for (int idx = tid; idx < AS_ROWS * HID; idx += AS_THREADS) hn_s[idx] = x_s[idx];
     } else
     for (int idx = tid; idx < AS_ROWS * HID; idx += AS_THREADS) {
-        int r = idx >> 6, i = idx & 63, row = r0 + r;
+        int r = idx >> 6, i = idx & 63, row = cta_row<POOL>(r0, rl, r, a.rows);
         const float *g = g_s + r * 2 * G3;
         float rr = sigmoidf_acc(g[i] + g[G3 + i]);
         float zz = sigmoidf_acc(g[HID + i] + g[G3 + HID + i]);
@@ -673,13 +809,13 @@ __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs 
 #pragma unroll
         for (int r = 0; r < 8; ++r) { hv[r][0] = hn_s[r * HID + 2 * lane]; hv[r][1] = hn_s[r * HID + 2 * lane + 1]; }
         for (int j = warp; j < a.A; j += AS_WARPS) {
-            const float2 wv = __ldg(reinterpret_cast<const float2 *>(P + L.fc2_w + (int64_t)j * HID) + lane);
+            const float2 wv = ldg_f2<POOL>(reinterpret_cast<const float2 *>(P + L.fc2_w + (int64_t)j * HID) + lane);
             float acc[8];
 #pragma unroll
             for (int r = 0; r < 8; ++r) acc[r] = fmaf(wv.y, hv[r][1], wv.x * hv[r][0]);
             float s = warp_fold8(acc, lane);
             if ((lane & 3) == 0) {
-                int r = lane >> 2, row = r0 + r;
+                int r = lane >> 2, row = cta_row<POOL>(r0, rl, r, a.rows);
                 s += __ldg(P + L.fc2_b + j);
                 q_s[r * 32 + j] = s;
                 if (row < a.rows) a.q[(int64_t)row * a.A + j] = s;
@@ -690,7 +826,7 @@ __global__ void __launch_bounds__(AS_THREADS) k_agent_step_stream(AgentStepArgs 
     __syncthreads();
     // ---- epsilon-greedy selection: one warp per row
     {
-        int row = r0 + warp;
+        int row = cta_row<POOL>(r0, rl, warp, a.rows);
         if (row < a.rows) select_row(a.sel, row, a.A, lane, lane < a.A ? q_s[warp * 32 + lane] : 0.0f, a.io.enabled ? &a.io : nullptr);
     }
 }

@@ -383,33 +383,39 @@ extern "C" int mal_eps_greedy_select(const float *q, int64_t q_ld, int32_t rows,
 }
 
 static thread_local int g_actsel_lat = 1;    // 1: mma.sync latency kernel for rollout-sized launches; 0: lanes-along-k register kernel
-static int launch_agent_step(AgentStepArgs &a, cudaStream_t stream) {
+// POOL: the per-match-policy instances; `ctas` is then the schedule's upper bound (CTAs past its used count exit at once)
+// and the variant is chosen on that grid by the same rule
+template <bool POOL>
+static int launch_agent_step(AgentStepArgs &a, cudaStream_t stream, int ctas) {
     const int Kin = a.in.last_end();
     const size_t smem = sizeof(float) * (size_t)(AS_ROWS * (Kin + 1) + AS_ROWS * HID * 3 + AS_ROWS * 2 * G3 + AS_ROWS * 32);
     MAL_REQUIRE(smem <= 200 * 1024 && Kin <= 32 * AS_FC1_MAXK, "mal_agent_step: input width %d too large (max %d)", Kin,
                 32 * AS_FC1_MAXK);
     int sms, tps;
     if (device_sm_count(&sms, &tps)) return 2;
-    const int ctas = (a.rows + AS_ROWS - 1) / AS_ROWS;
+    const char *name = POOL ? "k_agent_step_pool" : "k_agent_step";
     if (ctas <= sms && a.kind == MAL_AGENT_RNN && g_actsel_lat) {   // rollouts: latency is what counts
         const size_t smem_l = sizeof(float) * (size_t)(AS_ROWS * (((Kin + 7) & ~7) + 4) + AS_ROWS * 68 * 3 + AS_ROWS * 2 * G3 + AS_ROWS * 32);
         static size_t attr[MAL_MAX_DEV];
-        if (smem_l > 48 * 1024) if (int rc = ensure_dyn_smem(k_agent_step_lat, smem_l, attr)) return rc;
-        ProfScope _ps("k_agent_step", stream);
-        k_agent_step_lat<<<ctas, AL_THREADS, smem_l, stream>>>(a);
+        if (smem_l > 48 * 1024) if (int rc = ensure_dyn_smem(k_agent_step_lat<POOL>, smem_l, attr)) return rc;
+        ProfScope _ps(name, stream);
+        k_agent_step_lat<POOL><<<ctas, AL_THREADS, smem_l, stream>>>(a);
     } else if (ctas <= 2 * sms && a.kind == MAL_AGENT_RNN) {   // all weights prefetched into registers
         static size_t attr[MAL_MAX_DEV];
-        if (smem > 48 * 1024) if (int rc = ensure_dyn_smem(k_agent_step, smem, attr)) return rc;
-        ProfScope _ps("k_agent_step", stream);
-        k_agent_step<<<ctas, AS_THREADS, smem, stream>>>(a);
+        if (smem > 48 * 1024) if (int rc = ensure_dyn_smem(k_agent_step<POOL>, smem, attr)) return rc;
+        ProfScope _ps(name, stream);
+        k_agent_step<POOL><<<ctas, AS_THREADS, smem, stream>>>(a);
     } else {
         static size_t attr[MAL_MAX_DEV];
-        if (smem > 48 * 1024) if (int rc = ensure_dyn_smem(k_agent_step_stream, smem, attr)) return rc;
-        ProfScope _ps("k_agent_step", stream);
-        k_agent_step_stream<<<ctas, AS_THREADS, smem, stream>>>(a);
+        if (smem > 48 * 1024) if (int rc = ensure_dyn_smem(k_agent_step_stream<POOL>, smem, attr)) return rc;
+        ProfScope _ps(name, stream);
+        k_agent_step_stream<POOL><<<ctas, AS_THREADS, smem, stream>>>(a);
     }
-    MAL_LAUNCH_CHECK("k_agent_step");
+    MAL_LAUNCH_CHECK(name);
     return 0;
+}
+static int launch_agent_step(AgentStepArgs &a, cudaStream_t stream) {
+    return launch_agent_step<false>(a, stream, (a.rows + AS_ROWS - 1) / AS_ROWS);
 }
 
 // dense_input of mal_agent_step / mal_dqn_step: bit 0 = the caller assembled the input (obs_dim columns, nothing to
@@ -423,19 +429,29 @@ static int step_input(int32_t dense_input, AgentStepArgs *a) {
     return 0;
 }
 
-extern "C" int mal_agent_step(const float *agent, int32_t rows, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
-                              int32_t dense_input, const float *obs, int64_t obs_sb, const float *last_onehot,
-                              int64_t onehot_sb, const float *h_in, float *h_out, float *q, const mal_select_t *sel,
-                              void *stream) {
-    MAL_REQUIRE(agent && obs && h_out && q && rows > 0, "mal_agent_step: bad arguments");
+static int agent_step_args(const char *what, const float *agent, int32_t rows, int32_t n_agents, int32_t obs_dim,
+                           int32_t n_actions, int32_t dense_input, const float *obs, int64_t obs_sb, const float *last_onehot,
+                           int64_t onehot_sb, const float *h_in, float *h_out, float *q, AgentStepArgs *ap) {
+    MAL_REQUIRE(agent && obs && h_out && q && rows > 0, "%s: bad arguments", what);
     MAL_REQUIRE(n_actions >= 1 && n_actions <= MAL_MAX_ACTIONS, "n_actions must be in [1, %d]", MAL_MAX_ACTIONS);
-    MAL_REQUIRE(n_agents >= 1 && obs_dim >= 1, "mal_agent_step: bad dims");
-    AgentStepArgs a;
+    MAL_REQUIRE(n_agents >= 1 && obs_dim >= 1, "%s: bad dims", what);
+    AgentStepArgs &a = *ap;
     memset(&a, 0, sizeof(a));
     a.params = agent; a.rows = rows; a.N = n_agents; a.OBS = obs_dim; a.A = n_actions;
     if (int rc = step_input(dense_input, &a)) return rc;
     a.obs = obs; a.obs_sb = obs_sb; a.onehot = a.in.last > 0 ? last_onehot : nullptr; a.onehot_sb = onehot_sb;
-    a.h_in = h_in; a.h_out = h_out; a.q = q; a.do_select = sel ? 1 : 0;
+    a.h_in = h_in; a.h_out = h_out; a.q = q;
+    return 0;
+}
+
+extern "C" int mal_agent_step(const float *agent, int32_t rows, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
+                              int32_t dense_input, const float *obs, int64_t obs_sb, const float *last_onehot,
+                              int64_t onehot_sb, const float *h_in, float *h_out, float *q, const mal_select_t *sel,
+                              void *stream) {
+    AgentStepArgs a;
+    if (int rc = agent_step_args("mal_agent_step", agent, rows, n_agents, obs_dim, n_actions, dense_input, obs, obs_sb,
+                                 last_onehot, onehot_sb, h_in, h_out, q, &a)) return rc;
+    a.do_select = sel ? 1 : 0;
     if (sel) if (int rc = fill_select(sel, rows, n_agents, n_actions, &a.sel)) return rc;
     return launch_agent_step(a, (cudaStream_t)stream);
 }
@@ -458,26 +474,23 @@ extern "C" int mal_dqn_step(const float *agent, int32_t rows, int32_t n_agents, 
     return launch_agent_step(a, (cudaStream_t)stream);
 }
 
-extern "C" int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
-                                const mal_rollout_io_t *io, const float *h_in, float *h_out, float *q, const mal_select_t *sel,
-                                void *stream) {
-    MAL_REQUIRE(agent && io && sel && h_out && q && bs > 0, "mal_rollout_step: bad arguments");
+static int rollout_args(const char *what, const float *agent, int32_t bs, int32_t n_agents, int32_t obs_dim,
+                        int32_t n_actions, const mal_rollout_io_t *io, const float *h_in, float *h_out, float *q,
+                        const mal_select_t *sel, AgentStepArgs *ap) {
+    MAL_REQUIRE(agent && io && sel && h_out && q && bs > 0, "%s: bad arguments", what);
     MAL_REQUIRE(n_actions >= 1 && n_actions <= MAL_MAX_ACTIONS, "n_actions must be in [1, %d]", MAL_MAX_ACTIONS);
-    MAL_REQUIRE(n_agents >= 1 && obs_dim >= 1 && io->state_dim >= 1, "mal_rollout_step: bad dims");
+    MAL_REQUIRE(n_agents >= 1 && obs_dim >= 1 && io->state_dim >= 1, "%s: bad dims", what);
     MAL_REQUIRE(io->env_state && io->env_avail && io->env_obs && io->state_t && io->avail_t && io->obs_t && io->filled_t &&
-                    io->actions_t && io->onehot_t, "mal_rollout_step: environment / batch pointers missing");
-    MAL_REQUIRE(!io->prev_reward || (io->prev_done && io->reward_tm1 && io->term_tm1), "mal_rollout_step: previous-step fields missing");
-    MAL_REQUIRE((io->agent_input & ~3) == 0, "mal_rollout_step: unknown agent_input bits %d", io->agent_input);
-    AgentStepArgs a;
+                    io->actions_t && io->onehot_t, "%s: environment / batch pointers missing", what);
+    MAL_REQUIRE(!io->prev_reward || (io->prev_done && io->reward_tm1 && io->term_tm1), "%s: previous-step fields missing", what);
+    MAL_REQUIRE((io->agent_input & ~3) == 0, "%s: unknown agent_input bits %d", what, io->agent_input);
+    AgentStepArgs &a = *ap;
     memset(&a, 0, sizeof(a));
     const int rows = bs * n_agents;
     a.params = agent; a.rows = rows; a.N = n_agents; a.OBS = obs_dim; a.A = n_actions; a.dense = 0;
     a.in = agent_input(obs_dim, n_actions, n_agents, io->agent_input);
     a.obs = io->env_obs; a.obs_sb = io->env_obs_sb; a.onehot = io->onehot_tm1; a.onehot_sb = io->onehot_tm1_sb;
     a.h_in = h_in; a.h_out = h_out; a.q = q; a.do_select = 1;
-    mal_select_t s2 = *sel;
-    s2.avail = io->env_avail; s2.avail_sb = io->env_avail_sb;
-    if (int rc = fill_select(&s2, rows, n_agents, n_actions, &a.sel)) return rc;
     RolloutIO &r = a.io;
     r.enabled = 1; r.S = io->state_dim;
     r.env_state = io->env_state; r.env_state_sb = io->env_state_sb; r.alive = io->alive;
@@ -486,7 +499,91 @@ extern "C" int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents
     r.obs_t = io->obs_t; r.obs_sb = io->obs_sb; r.filled_t = (long long *)io->filled_t; r.filled_sb = io->filled_sb;
     r.actions_t = (long long *)io->actions_t; r.actions_sb = io->actions_sb; r.onehot_t = io->onehot_t; r.onehot_sb = io->onehot_sb;
     r.reward_tm1 = io->reward_tm1; r.reward_sb = io->reward_sb; r.term_tm1 = io->term_tm1; r.term_sb = io->term_sb;
+    return 0;
+}
+// the selector of a rollout step reads the environment's avail rows of `io`
+static int rollout_select(const mal_select_t *sel, const mal_rollout_io_t *io, AgentStepArgs *a) {
+    mal_select_t s2 = *sel;
+    s2.avail = io->env_avail; s2.avail_sb = io->env_avail_sb;
+    return fill_select(&s2, a->rows, a->N, a->A, &a->sel);
+}
+
+extern "C" int mal_rollout_step(const float *agent, int32_t bs, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
+                                const mal_rollout_io_t *io, const float *h_in, float *h_out, float *q, const mal_select_t *sel,
+                                void *stream) {
+    AgentStepArgs a;
+    if (int rc = rollout_args("mal_rollout_step", agent, bs, n_agents, obs_dim, n_actions, io, h_in, h_out, q, sel, &a)) return rc;
+    if (int rc = rollout_select(sel, io, &a)) return rc;
     return launch_agent_step(a, (cudaStream_t)stream);
+}
+
+// ---------------------------------------------------------------------------------------------
+// per-match policies (actsel.cuh: k_policy_schedule and the POOL instances of the step kernels)
+// ---------------------------------------------------------------------------------------------
+static int check_pool_shape(const char *what, int32_t bs, int32_t n_agents, int32_t n_policies) {
+    MAL_REQUIRE(bs >= 1 && n_agents >= 1, "%s: bs and n_agents must be >= 1", what);
+    MAL_REQUIRE((int64_t)bs * n_agents <= (1 << 30), "%s: bs * n_agents = %lld rows is too many", what, (long long)bs * n_agents);
+    MAL_REQUIRE(n_policies >= 1 && n_policies <= MAL_MAX_POLICIES, "%s: n_policies must be in [1, %d], got %d", what,
+                MAL_MAX_POLICIES, n_policies);
+    return 0;
+}
+// upper bound of the used CTAs: sum over policies of ceil(rows_p / 8) <= ceil(rows / 8) + (non-empty policies - 1)
+static int64_t pool_grid(int32_t rows, int32_t bs, int32_t n_policies) {
+    return ceil_div64(rows, AS_ROWS) + (n_policies < bs ? n_policies : bs) - 1;
+}
+
+extern "C" int64_t mal_policy_schedule_bytes(int32_t bs, int32_t n_agents, int32_t n_policies) {
+    if (check_pool_shape("mal_policy_schedule_bytes", bs, n_agents, n_policies)) return -1;
+    return (int64_t)sizeof(int32_t) * (PS_HDR + pool_grid(bs * n_agents, bs, n_policies) * PS_ENT);
+}
+
+extern "C" int mal_policy_schedule(const int32_t *match_policy, int32_t bs, int32_t n_agents, int32_t n_policies,
+                                   void *schedule, int32_t *status, void *stream) {
+    if (int rc = check_pool_shape("mal_policy_schedule", bs, n_agents, n_policies)) return rc;
+    MAL_REQUIRE(match_policy && schedule, "mal_policy_schedule: null argument");
+    MAL_REQUIRE(((uintptr_t)schedule & 15) == 0, "mal_policy_schedule: the schedule buffer must be 16-byte aligned");
+    { ProfScope _ps("k_policy_schedule", (cudaStream_t)stream);
+      k_policy_schedule<<<1, PS_THREADS, 0, (cudaStream_t)stream>>>(match_policy, bs, n_agents, n_policies, (int32_t *)schedule, status); }
+    MAL_LAUNCH_CHECK("k_policy_schedule");
+    return 0;
+}
+
+static int pool_args(const char *what, const float *table, int64_t table_ld, int32_t n_policies, const void *schedule,
+                     AgentStepArgs *a) {
+    if (int rc = check_pool_shape(what, a->rows / a->N, a->N, n_policies)) return rc;
+    MAL_REQUIRE(table && schedule, "%s: null table or schedule", what);
+    MAL_REQUIRE(a->rows % a->N == 0, "%s: rows %d is not a multiple of n_agents %d", what, a->rows, a->N);
+    MAL_REQUIRE(((uintptr_t)schedule & 15) == 0, "%s: the schedule buffer must be 16-byte aligned", what);
+    const int64_t P = agent_layout(a->in.d_in, a->A).total;
+    MAL_REQUIRE(table_ld >= P, "%s: table_ld %lld is smaller than the agent's %lld parameters", what, (long long)table_ld,
+                (long long)P);
+    a->sched = (const int32_t *)schedule; a->table_ld = table_ld; a->n_policies = n_policies;
+    return 0;
+}
+
+extern "C" int mal_agent_step_pool(const float *table, int64_t table_ld, int32_t n_policies, const void *schedule,
+                                   int32_t rows, int32_t n_agents, int32_t obs_dim, int32_t n_actions, int32_t dense_input,
+                                   const float *obs, int64_t obs_sb, const float *last_onehot, int64_t onehot_sb,
+                                   const float *h_in, float *h_out, float *q, const mal_select_t *sel, void *stream) {
+    AgentStepArgs a;
+    if (int rc = agent_step_args("mal_agent_step_pool", table, rows, n_agents, obs_dim, n_actions, dense_input, obs, obs_sb,
+                                 last_onehot, onehot_sb, h_in, h_out, q, &a)) return rc;
+    if (int rc = pool_args("mal_agent_step_pool", table, table_ld, n_policies, schedule, &a)) return rc;
+    a.do_select = sel ? 1 : 0;
+    if (sel) if (int rc = fill_select(sel, rows, n_agents, n_actions, &a.sel)) return rc;
+    return launch_agent_step<true>(a, (cudaStream_t)stream, (int)pool_grid(rows, rows / n_agents, n_policies));
+}
+
+extern "C" int mal_rollout_step_pool(const float *table, int64_t table_ld, int32_t n_policies, const void *schedule,
+                                     int32_t bs, int32_t n_agents, int32_t obs_dim, int32_t n_actions,
+                                     const mal_rollout_io_t *io, const float *h_in, float *h_out, float *q,
+                                     const mal_select_t *sel, void *stream) {
+    AgentStepArgs a;
+    if (int rc = rollout_args("mal_rollout_step_pool", table, bs, n_agents, obs_dim, n_actions, io, h_in, h_out, q, sel, &a))
+        return rc;
+    if (int rc = pool_args("mal_rollout_step_pool", table, table_ld, n_policies, schedule, &a)) return rc;
+    if (int rc = rollout_select(sel, io, &a)) return rc;
+    return launch_agent_step<true>(a, (cudaStream_t)stream, (int)pool_grid(a.rows, bs, n_policies));
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -1,3 +1,4 @@
 from .agent_pool import DeviceAgentPool
+from .cross_play import cross_play_returns
 
-__all__ = ["DeviceAgentPool"]
+__all__ = ["DeviceAgentPool", "cross_play_returns"]
