@@ -54,6 +54,9 @@ typedef struct mal_batch {
     mal_field_t reward;               /* f32 [B,TT,1] */
     mal_field_t terminated;           /* u8  [B,TT,1] */
     mal_field_t filled;               /* i64 [B,TT,1] */
+    mal_field_t weight;               /* f32 [B] importance weights of prioritized replay (sb = batch stride, st unused), or
+                                         ptr = NULL: unweighted.  Weighted: loss = sum_b w_b sum_t (td*m)^2 / sum m, seed
+                                         2 w_b td m^2; the other statistics are unweighted.  Rejected with cfg.unnormalized */
 } mal_batch_t;
 
 /* MAL_MIXER_NONE: independent Q-learners (IQL, `mixer: None`): no mixing network, every agent has its own TD error
@@ -384,6 +387,28 @@ typedef struct mal_wire_layout {
 int mal_wire_layout(int32_t TT, int32_t N, int32_t OBS, int32_t S, mal_wire_layout_t *out);
 int mal_wire_pack(const mal_batch_t *batch, void *wire, const mal_wire_layout_t *layout, int32_t *status, void *stream);
 int mal_wire_unpack(const mal_batch_t *batch, const void *wire, const mal_wire_layout_t *layout, void *stream);
+
+/* Proportional prioritized episode replay (Schaul et al., 2016) over the live slots [0, n) of a replay buffer.
+ *
+ * mal_per_sample: ONE launch.  total = sum p_i, p_min = min p_i over the n slots (fixed reduction / scan order, fp64 prefix
+ *   sums: identical inputs give bit-identical ids).  Draw j of B takes x_j = (j + u_j) * total / B and returns the first slot
+ *   whose inclusive prefix sum exceeds x_j (sampling with replacement, stratified); ids [B] int64 can go straight into
+ *   mal_record_copy as src_ids.  weights [B] f32: w_j = (p_min / p_{id_j})^beta (1 where p_{id_j} = 0).  Uniforms: u [B]
+ *   (device) when non-NULL; otherwise Philox4x32-10 at (seed, offset) in exactly the layout th.rand(B) uses on this device,
+ *   and *advance (may be NULL) receives what the caller adds to the generator's offset (0 for injected uniforms).
+ *   priorities must be 16-byte aligned, >= 0 and finite.
+ * mal_per_update: ONE launch after a learner step over the workspace's td ([B*T*n_q], row m = b*T + t; n_q = 1 with a mixer,
+ *   N without) and mask ([B*T]): priorities[ids[b]] = (sum_{t,n} |td*m| / sum_{t,n} m + eps)^alpha (0 for the ratio when the
+ *   episode has no live transition).  When a batch samples a slot twice the occurrence with the highest batch index wins;
+ *   ids outside [0, capacity) are skipped.  *max_priority (device float) is raised to the largest new priority.
+ * The _check queries are host-only (no device needed): 0, or non-zero with mal_last_error set for arguments the entries
+ *   reject (n == 0, B < 1, a negative or non-finite alpha / beta / eps). */
+int mal_per_sample_check(int64_t n, int32_t B, float beta);
+int mal_per_sample(const float *priorities, int64_t n, int32_t B, float beta, const float *u, uint64_t seed,
+                   uint64_t offset, int64_t *ids, float *weights, uint64_t *advance, void *stream);
+int mal_per_update_check(int32_t B, int32_t T, int32_t n_q, float alpha, float eps);
+int mal_per_update(const float *td, const float *mask, int32_t B, int32_t T, int32_t n_q, const int64_t *ids,
+                   float alpha, float eps, float *priorities, int64_t capacity, float *max_priority, void *stream);
 
 /* EpisodeBatch.max_t_filled, episode_batch.py:240-242: out[0] = max_b sum_t filled[b,t]. */
 int mal_max_t_filled(const int64_t *filled, int64_t sb, int64_t st, int32_t B, int32_t TT, int32_t *out,

@@ -6,7 +6,7 @@ Python API.  Sub-packages mirror the reference's `marl.*` layout:
 """
 from . import _native
 from .components.episode_batch import EpisodeBatch
-from .components.replay_buffers import ReplayBuffer
+from .components.replay_buffers import ReplayBuffer, PrioritizedReplayBuffer
 from .components.transforms import OneHot
 from .components.action_selectors import EpsilonGreedyActionSelector, REGISTRY as action_REGISTRY
 from .controllers import BasicMAC, EnsembleMAC, REGISTRY as mac_REGISTRY
@@ -14,6 +14,6 @@ from .learners import QLearner, REGISTRY as learner_REGISTRY
 from .modules.agents import DRQNAgentNetwork, DQNAgentNetwork, REGISTRY as agent_REGISTRY
 from .modules.mixers import QMixer, VDNMixer
 
-__all__ = ["EpisodeBatch", "ReplayBuffer", "OneHot", "EpsilonGreedyActionSelector", "BasicMAC", "QLearner",
+__all__ = ["EpisodeBatch", "ReplayBuffer", "PrioritizedReplayBuffer", "OneHot", "EpsilonGreedyActionSelector", "BasicMAC", "QLearner",
            "EnsembleMAC", "DRQNAgentNetwork", "DQNAgentNetwork", "QMixer", "VDNMixer", "mac_REGISTRY", "learner_REGISTRY", "agent_REGISTRY",
            "action_REGISTRY"]

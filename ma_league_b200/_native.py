@@ -39,7 +39,7 @@ class Field(C.Structure):
 class Batch(C.Structure):
     _fields_ = [("B", C.c_int32), ("TT", C.c_int32), ("N", C.c_int32), ("A", C.c_int32), ("OBS", C.c_int32),
                 ("S", C.c_int32), ("obs", Field), ("onehot", Field), ("actions", Field), ("avail", Field),
-                ("state", Field), ("reward", Field), ("terminated", Field), ("filled", Field)]
+                ("state", Field), ("reward", Field), ("terminated", Field), ("filled", Field), ("weight", Field)]
 
 
 class LearnerCfg(C.Structure):
@@ -144,6 +144,12 @@ _PROTOS = {
     "mal_wire_layout": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(WireLayout)]),
     "mal_wire_pack": (C.c_int, [C.POINTER(Batch), C.c_void_p, C.POINTER(WireLayout), C.c_void_p, C.c_void_p]),
     "mal_wire_unpack": (C.c_int, [C.POINTER(Batch), C.c_void_p, C.POINTER(WireLayout), C.c_void_p]),
+    "mal_per_sample_check": (C.c_int, [C.c_int64, C.c_int32, C.c_float]),
+    "mal_per_sample": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_float, C.c_void_p, C.c_uint64, C.c_uint64,
+                                 C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p]),
+    "mal_per_update_check": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_float]),
+    "mal_per_update": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_float, C.c_float,
+                                 C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "mal_max_t_filled": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
 }
 EXPORTS = tuple(_PROTOS)

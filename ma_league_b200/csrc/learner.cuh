@@ -613,6 +613,7 @@ struct MixArgs {
     float *dh_head;                    // [TT*R,64]: rows of t < T: d_chosen * fc2.weight[a_t, :] (gather + fc2 backward)
     float *part_stats;                 // [gridDim.x][MIX_NSTAT]
     float *part_v2;                    // [gridDim.x][E+1] d V.2.weight | d V.2.bias
+    mal_field_t weight;                // k_mix_td<true>: f32 [B] importance weights (batch stride sb)
 };
 
 __device__ __forceinline__ float qmix_row(const MixArgs &a, int net, int64_t m, const float *q, int lane,
@@ -638,6 +639,9 @@ __device__ __forceinline__ float qmix_row(const MixArgs &a, int net, int64_t m, 
     return y;
 }
 
+// WEIGHTED: prioritized replay's importance weights w_b scale episode b's loss term and seed (the <false> instance is the
+// unweighted step, unchanged); multiplying by w_b = 1.0f is exact, so weights of one reproduce it bit for bit.
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
     __shared__ float s_stats[8][MIX_NSTAT];
     __shared__ float s_v2[8][MAL_MAX_EMBED + 1];
@@ -703,19 +707,24 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
         const float target = rew + a.gamma * (1.0f - term) * ty;
         const float tdv = y - target;
         const float mtd = tdv * mk;
-        const float gseed = 2.0f * mtd * mk;   // (d loss / d q_tot) * mask.sum()
+        float gseed = 2.0f * mtd * mk;         // (d loss / d q_tot) * mask.sum()
+        float lterm = mtd * mtd;
+        if (WEIGHTED) {
+            const float wb = *(reinterpret_cast<const float *>(a.weight.ptr) + (int64_t)b * a.weight.sb);
+            gseed *= wb; lterm *= wb;
+        }
         if (iql) {
             if (lane == 0) a.mask[m] = mk;
             if (lane < a.N) {
                 const int64_t e = m * a.N + lane;
                 a.q_tot[e] = y; a.target_q_tot[e] = ty; a.targets[e] = target; a.td[e] = tdv;
-                st[0] += mtd * mtd; st[1] += fabsf(mtd); st[2] += y * mk; st[3] += target * mk;
+                st[0] += lterm; st[1] += fabsf(mtd); st[2] += y * mk; st[3] += target * mk;
                 st[4] += mk; st[5] += (mk != 0.0f) ? 1.0f : 0.0f;
             }
         } else if (lane == 0) {
             a.mask[m] = mk;
             a.q_tot[m] = y; a.target_q_tot[m] = ty; a.targets[m] = target; a.td[m] = tdv;
-            st[0] += mtd * mtd; st[1] += fabsf(mtd); st[2] += y * mk; st[3] += target * mk;
+            st[0] += lterm; st[1] += fabsf(mtd); st[2] += y * mk; st[3] += target * mk;
             st[4] += mk; st[5] += (mk != 0.0f) ? 1.0f : 0.0f;
         }
         int act_mine = lane < a.N ? (int)(field_ptr<long long>(a.actions, b, t)[lane]) : 0;

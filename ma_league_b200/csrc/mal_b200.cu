@@ -13,6 +13,7 @@
 #include "agent_in_gemm.cuh"
 #include "tc_reduce.cuh"
 #include "autograd.cuh"
+#include "per.cuh"
 
 // ---------------------------------------------------------------------------------------------
 static thread_local char g_err[512] = "";
@@ -603,6 +604,8 @@ static int get_dims(const mal_batch_t *b, const mal_learner_cfg_t *c, Dims *d) {
     MAL_REQUIRE(b->N <= MAL_MAX_ACTIONS, "n_agents must be <= %d", MAL_MAX_ACTIONS);
     MAL_REQUIRE(c->mixer == MAL_MIXER_VDN || c->mixer == MAL_MIXER_QMIX2 || c->mixer == MAL_MIXER_QMIX1 ||
                 c->mixer == MAL_MIXER_NONE, "Mixer %d not recognised.", c->mixer);
+    MAL_REQUIRE(!b->weight.ptr || !c->unnormalized,
+                "importance weights (prioritized replay) are not supported in unnormalized (data-parallel) mode");
     d->B = b->B; d->TT = b->TT; d->T = b->TT - 1; d->N = b->N; d->A = b->A; d->OBS = b->OBS; d->S = b->S;
     MAL_REQUIRE(c->agent_kind == MAL_AGENT_RNN || c->agent_kind == MAL_AGENT_DQN, "agent kind %d not recognised", c->agent_kind);
     d->kind = c->agent_kind;
@@ -1213,8 +1216,14 @@ extern "C" int mal_learner_forward(const mal_batch_t *batch, const mal_learner_c
         a.q_tot = F(plan->q_tot); a.target_q_tot = F(plan->target_q_tot); a.targets = F(plan->targets); a.td = F(plan->td);
         a.d_a2 = F(plan->d_a2); a.d_y1 = F(plan->d_y1); a.d_chosen = F(plan->d_chosen);
         a.part_stats = parts + pl.mix_stats; a.part_v2 = parts + pl.mix_v2;
-        if (g_rec_carveout & 4) { static bool cv[MAL_MAX_DEV]; if (int rc = ensure_max_carveout(k_mix_td, cv)) return rc; }
-        { ProfScope _ps("k_mix_td", st); launch_k(k_mix_td, dim3(pl.nblk_mix), dim3(256), 0, st, true, a); }   // stream predecessor: k_q_head
+        a.weight = batch->weight;
+        if (batch->weight.ptr) {                     // prioritized replay: importance-weighted loss and seeds
+            if (g_rec_carveout & 4) { static bool cv[MAL_MAX_DEV]; if (int rc = ensure_max_carveout(k_mix_td<true>, cv)) return rc; }
+            { ProfScope _ps("k_mix_td_w", st); launch_k(k_mix_td<true>, dim3(pl.nblk_mix), dim3(256), 0, st, true, a); }
+        } else {
+            if (g_rec_carveout & 4) { static bool cv[MAL_MAX_DEV]; if (int rc = ensure_max_carveout(k_mix_td<false>, cv)) return rc; }
+            { ProfScope _ps("k_mix_td", st); launch_k(k_mix_td<false>, dim3(pl.nblk_mix), dim3(256), 0, st, true, a); }   // stream predecessor: k_q_head
+        }
         MAL_LAUNCH_CHECK("k_mix_td");
         // nothing before the gradient gather reads the scalars: inside mal_learner_step the finalize runs on the side
         // stream (the backward joins that stream before k_grad_reduce) and leaves the critical path
@@ -1936,5 +1945,61 @@ extern "C" int mal_copy_f32(float *dst, const float *src, int64_t n, void *strea
     int64_t grid = ceil_div64(n, 1024); if (grid > 1184) grid = 1184; if (grid < 1) grid = 1;
     { ProfScope _ps("k_copy_f32", (cudaStream_t)stream); k_copy_f32<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(dst, src, n); }
     MAL_LAUNCH_CHECK("k_copy_f32");
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// prioritized episode replay
+// ---------------------------------------------------------------------------------------------
+static bool finite_nonneg(float v) { return v >= 0.0f && v <= 3.402823466e38f; }   // false for NaN and +inf too
+
+extern "C" int mal_per_sample_check(int64_t n, int32_t B, float beta) {
+    MAL_REQUIRE(n >= 1, "mal_per_sample: the buffer holds no episode (n = %lld)", (long long)n);
+    MAL_REQUIRE(B >= 1, "mal_per_sample: batch size %d must be >= 1", B);
+    MAL_REQUIRE(finite_nonneg(beta), "mal_per_sample: beta must be finite and >= 0");
+    return 0;
+}
+
+extern "C" int mal_per_sample(const float *priorities, int64_t n, int32_t B, float beta, const float *u, uint64_t seed,
+                              uint64_t offset, int64_t *ids, float *weights, uint64_t *advance, void *stream) {
+    if (int rc = mal_per_sample_check(n, B, beta)) return rc;
+    MAL_REQUIRE(priorities && ids && weights, "mal_per_sample: null argument");
+    MAL_REQUIRE((reinterpret_cast<uintptr_t>(priorities) & 15) == 0, "mal_per_sample: priorities must be 16-byte aligned");
+    PerSampleArgs a;
+    a.p = priorities; a.n = n; a.per = align_up64(ceil_div64(n, PER_THREADS), 4); a.B = B; a.beta = beta;
+    a.u = u; a.seed = seed; a.offset = offset; a.ids = ids; a.w = weights; a.grid = 1;
+    if (!u) {                                    // th.rand(B)'s grid and generator advance on this device
+        int sms, tps;
+        if (device_sm_count(&sms, &tps)) return 2;
+        const uint64_t cap = (uint64_t)sms * (uint64_t)(tps / 256);
+        uint64_t g = ((uint64_t)B + 255) / 256; if (g > cap) g = cap;
+        a.grid = (uint32_t)g;
+        if (advance) *advance = (((uint64_t)B - 1) / (256 * g * 4) + 1) * 4;
+    } else if (advance) {
+        *advance = 0;
+    }
+    { ProfScope _ps("k_per_sample", (cudaStream_t)stream); k_per_sample<<<1, PER_THREADS, 0, (cudaStream_t)stream>>>(a); }
+    MAL_LAUNCH_CHECK("k_per_sample");
+    return 0;
+}
+
+extern "C" int mal_per_update_check(int32_t B, int32_t T, int32_t n_q, float alpha, float eps) {
+    MAL_REQUIRE(B >= 1, "mal_per_update: batch size %d must be >= 1", B);
+    MAL_REQUIRE(T >= 1 && n_q >= 1 && n_q <= MAL_MAX_ACTIONS, "mal_per_update: bad shape (T = %d, n_q = %d)", T, n_q);
+    MAL_REQUIRE(finite_nonneg(alpha), "mal_per_update: alpha must be finite and >= 0");
+    MAL_REQUIRE(finite_nonneg(eps), "mal_per_update: eps must be finite and >= 0");
+    return 0;
+}
+
+extern "C" int mal_per_update(const float *td, const float *mask, int32_t B, int32_t T, int32_t n_q, const int64_t *ids,
+                              float alpha, float eps, float *priorities, int64_t capacity, float *max_priority,
+                              void *stream) {
+    if (int rc = mal_per_update_check(B, T, n_q, alpha, eps)) return rc;
+    MAL_REQUIRE(td && mask && ids && priorities && max_priority && capacity >= 1, "mal_per_update: null argument");
+    PerUpdateArgs a;
+    a.td = td; a.mask = mask; a.B = B; a.T = T; a.nq = n_q; a.ids = ids; a.capacity = capacity;
+    a.alpha = alpha; a.eps = eps; a.priorities = priorities; a.max_priority = max_priority;
+    { ProfScope _ps("k_per_update", (cudaStream_t)stream); k_per_update<<<(unsigned)ceil_div64(B, 8), 256, 0, (cudaStream_t)stream>>>(a); }
+    MAL_LAUNCH_CHECK("k_per_update");
     return 0;
 }

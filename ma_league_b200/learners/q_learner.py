@@ -160,6 +160,8 @@ class QLearner(Learner):
         """Flat buffers, plan and workspace for this batch shape."""
         dev = batch["obs"].device
         bs = self._batch_struct(batch)
+        if bs.weight.ptr:                # the cached struct may carry the weights of an earlier train() call
+            bs.weight = nat.Field()
         cfg = self._cfg()
         key = (bs.B, bs.TT, bs.N, bs.A, bs.OBS, bs.S, cfg.mixer, cfg.save_q, str(dev))
         if key != self._ws_key:
@@ -192,12 +194,15 @@ class QLearner(Learner):
         return self._ws_f32(self._plan.scalars, 64)
 
     # ------------------------------------------------------------------ training
-    def train(self, batch, t_env: int, episode_num: int):
+    def train(self, batch, t_env: int, episode_num: int, weights=None):
+        """`weights`: optional importance weights [B] (f32, on the batch's device) of prioritized replay: the loss becomes
+        sum_b w_b sum_t (td*m)^2 / sum m.  None is the unweighted step, bit for bit."""
         bs, cfg, f = self._prepare(batch)
         if self.optimiser is None:
             raise nat.MalError("call build_optimizer() before train() (ma_experiment.py:61)")
         dev = batch["obs"].device
         dp = cfg.unnormalized != 0
+        self._set_weights(bs, weights, dev, dp)
         counted = False                          # True: the trained-steps counter was advanced inside the replayed graph
         if dp:
             self._train_data_parallel(bs, cfg, f, dev)
@@ -238,6 +243,17 @@ class QLearner(Learner):
             self.logger.log_stat(self.name + "target_mean", float(h[nat.SC_TARGET]), t_env)
             self.log_stats_t = t_env
 
+    def _set_weights(self, bs, weights, dev, dp):
+        if weights is None:
+            return
+        if dp or getattr(self.args, "data_parallel", False):
+            raise nat.MalError("importance weights (prioritized replay) are not supported with data_parallel: "
+                               "sharded sampling would need a sampler per rank and a global normaliser")
+        if not isinstance(weights, th.Tensor) or weights.device != dev or weights.dtype != th.float32 or \
+                weights.dim() != 1 or weights.numel() != bs.B:
+            raise nat.MalError("weights must be a float32 [B] tensor on the batch's device")
+        bs.weight = nat.Field(weights.data_ptr(), weights.stride(0), 0)
+
     def _step_eager(self, bs, cfg, f, dev):
         with nat.on_device(dev):
             nat.check(nat.lib().mal_learner_step(C.byref(bs), C.byref(cfg), C.byref(self._plan),
@@ -250,7 +266,7 @@ class QLearner(Learner):
         """Replay the captured step when this exact set of device addresses / shapes / hyper-parameters was seen
         before; first sighting runs eagerly (it also warms the library's streams and kernel attributes), the second
         one captures."""
-        fields = (bs.obs, bs.onehot, bs.actions, bs.avail, bs.state, bs.reward, bs.terminated, bs.filled)
+        fields = (bs.obs, bs.onehot, bs.actions, bs.avail, bs.state, bs.reward, bs.terminated, bs.filled, bs.weight)
         key = (tuple((x.ptr, x.sb, x.st) for x in fields), bs.B, bs.TT, bs.N, bs.A, bs.OBS, bs.S,
                tuple(getattr(cfg, n) for n, _ in cfg._fields_),
                tuple(0 if v is None else v.data_ptr() for v in f.values()), self._ws.data_ptr(), self._grad.data_ptr(),
@@ -400,17 +416,33 @@ class QLearner(Learner):
         unfilled) without the host sync that `max_t_filled` as a Python slice bound costs.  `truncate=True` keeps the
         reference's exact sequence (one device->host sync per step, less arithmetic when episodes are short).
         Precondition of the masked form, as in the reference's steppers: an episode shorter than the sequence length
-        ends with `terminated = 1` on its last transition."""
+        ends with `terminated = 1` on its last transition.
+
+        A `PrioritizedReplayBuffer` runs sample (by priority, beta = `buffer.beta_at(t_env)`) -> record copy -> the
+        importance-weighted step -> priority update of the sampled episodes from the step's TD errors: two launches more
+        than the uniform step, and still no host sync in the masked form."""
+        from ..components.replay_buffers.prioritized_replay_buffer import PrioritizedReplayBuffer
+        per = isinstance(buffer, PrioritizedReplayBuffer)
+        if per and getattr(self.args, "data_parallel", False):
+            raise nat.MalError("prioritized replay is not supported with data_parallel")
         st = getattr(self, "_stage", None)
         if st is None or st.batch_size != batch_size or st.max_seq_length != buffer.max_seq_length or \
                 st._storage.device != buffer._storage.device or not st._layout.same_as(buffer._layout):
             st = buffer._gather_records(th.zeros(batch_size, dtype=th.long))   # a packed batch with the buffer's layout
             self._stage = st
-        buffer.sample_into(st)
+        if per:
+            buffer.sample_into(st, buffer.beta_at(t_env))
+        else:
+            buffer.sample_into(st)
         batch = st
         if truncate:
             batch = st[:, :int(st.max_t_filled())]
-        self.train(batch, t_env, episode_num)
+        self.train(batch, t_env, episode_num, weights=st.weights if per else None)
+        if per:
+            B, T = batch.batch_size, batch.max_seq_length - 1
+            Q = self.args.n_agents if self.mixer is None else 1
+            buffer.update_priorities(st.ids, self._ws_f32(self._plan.td, B * T * Q).view(B, T, Q),
+                                     self._ws_f32(self._plan.mask, B * T))
         return batch
 
     def forward_only(self, batch):
