@@ -82,8 +82,17 @@ typedef struct mal_learner_cfg {
                                          and clip + RMSprop skip its parameters and square_avg (only the mixer trains) */
     int32_t agent_kind;               /* MAL_AGENT_RNN (drqn_agent.py) or MAL_AGENT_DQN (dqn_agent.py: fc1 -> ReLU -> fc2) */
     int32_t agent_input;              /* MAL_IN_* bits (0: obs | last action | agent id); sets d_in and n_agent_params */
+    int32_t returns;                  /* MAL_RETURNS_*: the TD targets (0, a zeroed tail: the 1-step target) */
+    float td_lambda;                  /* MAL_RETURNS_TD_LAMBDA: lambda in [0, 1] (build_td_lambda_targets, coma_learner.py:10-21) */
 } mal_learner_cfg_t;
 enum { MAL_AGENT_RNN = 0, MAL_AGENT_DQN = 1 };
+/* MAL_RETURNS_ONE_STEP: targets = r_t + gamma (1 - term_t) tq[t] (q_learner.py:86).
+ * MAL_RETURNS_TD_LAMBDA: with tq[b,t] = target_q_tot of row (b,t) and the learner mask m,
+ *     R[b,T] = tq[b,T-1] (1 - sum_{t<T} term[b,t])
+ *     R[b,t] = lambda gamma R[b,t+1] + m[b,t] (r[b,t] + (1 - lambda) gamma (1 - term[b,t]) tq[b,t])   t = T-1 .. 0
+ *     targets = R[:, 0:T]   (per (b, agent) for MAL_MIXER_NONE, with r, term and m broadcast over agents).
+ * Everything downstream of the targets (td, loss, seeds, importance weights, statistics) is unchanged. */
+enum { MAL_RETURNS_ONE_STEP = 0, MAL_RETURNS_TD_LAMBDA = 1 };
 
 /* Byte offsets of every intermediate inside the caller-owned workspace (filled by mal_learner_plan).
  * Row index of the [TT*R, .] arrays is m = t*R + b*N + n; of the [B*T, .] arrays m = b*T + t.

@@ -19,6 +19,7 @@ ABI_VERSION = 6
 MIXER_VDN, MIXER_QMIX2, MIXER_QMIX1, MIXER_NONE = 0, 1, 2, 3    # MIXER_NONE: independent Q-learners (IQL)
 AGENT_RNN, AGENT_DQN = 0, 1
 IN_NO_LAST_ACTION, IN_NO_AGENT_ID = 1, 2     # agent-input switches (mal_learner_cfg_t.agent_input, mal_rollout_io_t.agent_input)
+RETURNS_ONE_STEP, RETURNS_TD_LAMBDA = 0, 1   # mal_learner_cfg_t.returns: 1-step or TD(lambda) targets
 STEP_DENSE = 1                               # dense_input of mal_agent_step / mal_dqn_step: bit 0; bits 1..2 = IN_* << 1
 SC_MASK_SUM, SC_LOSS, SC_TD_ABS, SC_Q_TAKEN, SC_TARGET, SC_GRAD_NORM, SC_MASK_COUNT, SC_STATUS = range(8)
 SC_RAW0 = 8     # raw sums: sum mtd^2, sum |mtd|, sum q_tot*m, sum targets*m, sum m, count
@@ -46,7 +47,7 @@ class LearnerCfg(C.Structure):
     _fields_ = [("mixer", C.c_int32), ("double_q", C.c_int32), ("embed", C.c_int32), ("hyper_embed", C.c_int32),
                 ("gamma", C.c_float), ("lr", C.c_float), ("alpha", C.c_float), ("eps", C.c_float),
                 ("clip", C.c_float), ("save_q", C.c_int32), ("unnormalized", C.c_int32), ("freeze_agent", C.c_int32),
-                ("agent_kind", C.c_int32), ("agent_input", C.c_int32)]
+                ("agent_kind", C.c_int32), ("agent_input", C.c_int32), ("returns", C.c_int32), ("td_lambda", C.c_float)]
 
 
 _PLAN_FIELDS = ["total_bytes", "n_agent_params", "n_mixer_params", "x_on", "x_tg", "gi_on", "gi_tg", "h_on", "h_tg",

@@ -616,7 +616,9 @@ struct MixArgs {
     mal_field_t weight;                // k_mix_td<true>: f32 [B] importance weights (batch stride sb)
 };
 
-__device__ __forceinline__ float qmix_row(const MixArgs &a, int net, int64_t m, const float *q, int lane,
+// q(n): agent n's Q-value of row m (an array read, or a shuffle from the lane that holds it)
+template <class QOf>
+__device__ __forceinline__ float qmix_row(const MixArgs &a, int net, int64_t m, QOf q, int lane,
                                           float *pre_out, float *hidden_out, float *wf_out, float *v1_out) {
     const MixerLayout ML = mixer_layout(a.mixer, a.S, a.N, a.E, a.HE);
     const int two = (ML.layers == 2);
@@ -628,7 +630,7 @@ __device__ __forceinline__ float qmix_row(const MixArgs &a, int net, int64_t m, 
     float pre = act ? y1[lane] : 0.0f;
     for (int n = 0; n < a.N; ++n) {
         float w1 = act ? fabsf(a2[n * a.E + lane]) : 0.0f;
-        pre = fmaf(q[n], w1, pre);
+        pre = fmaf(q(n), w1, pre);
     }
     float hidden = pre > 0.0f ? pre : expm1f(pre);
     float wf = act ? fabsf(a2[a.N * a.E + lane]) : 0.0f;
@@ -641,8 +643,10 @@ __device__ __forceinline__ float qmix_row(const MixArgs &a, int net, int64_t m, 
 
 // WEIGHTED: prioritized replay's importance weights w_b scale episode b's loss term and seed (the <false> instance is the
 // unweighted step, unchanged); multiplying by w_b = 1.0f is exact, so weights of one reproduce it bit for bit.
-template <bool WEIGHTED>
-__global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
+// GIVEN_TARGETS (TD(lambda), k_mix_td_lambda): the targets were formed by k_td_lambda and are read, not computed; the
+// target mixer row is then not evaluated here (k_mix_tq wrote target_q_tot).
+template <bool WEIGHTED, bool GIVEN_TARGETS>
+__device__ __forceinline__ void mix_td_body(MixArgs a) {
     __shared__ float s_stats[8][MIX_NSTAT];
     __shared__ float s_v2[8][MAL_MAX_EMBED + 1];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -669,19 +673,22 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
         const int b = (int)((unsigned)m / (unsigned)a.T), t = (int)m - b * a.T;
         // lane n holds agent n's chosen / target Q (N <= 32): one coalesced load each, broadcast by shuffle
         const float qc = lane < a.N ? a.chosen[m * a.N + lane] : 0.0f;
-        const float qt = lane < a.N ? a.target_max[m * a.N + lane] : 0.0f;
+        const float qt = !GIVEN_TARGETS && lane < a.N ? a.target_max[m * a.N + lane] : 0.0f;
         // per-transition scalars (issued early: independent of the mixing arithmetic)
         float mk = (float)(*field_ptr<long long>(a.filled, b, t));
         if (t > 0) mk = mk * (1.0f - (float)(*field_ptr<unsigned char>(a.terminated, b, t - 1)));   // mask[:, 1:] *= 1 - terminated[:, :-1]
         const float rew = *field_ptr<float>(a.reward, b, t);
         const float term = (float)(*field_ptr<unsigned char>(a.terminated, b, t));
-        float y, ty, pre = 0, hidden = 0, wf = 0, v1 = 0;
+        float y, ty = 0.0f, pre = 0, hidden = 0, wf = 0, v1 = 0;
         const float *a2o = a.a2[0] + m * ld2;
         const bool iql = a.mixer == MAL_MIXER_NONE;       // warp-uniform
         if (a.mixer == MAL_MIXER_VDN) {
-            y = warp_sum(qc); ty = warp_sum(qt);
+            y = warp_sum(qc);
+            if (!GIVEN_TARGETS) ty = warp_sum(qt);
         } else if (iql) {
             y = qc; ty = qt;                             // lane n: agent n's chosen / target Q (lanes >= N carry zeros)
+        } else if (GIVEN_TARGETS) {
+            y = qmix_row(a, 0, m, [&](int n) { return __shfl_sync(0xffffffffu, qc, n); }, lane, &pre, &hidden, &wf, &v1);
         } else {
             // online and target mixer rows side by side (lane = embed unit): hidden = elu(q . |w1| + b1), y = hidden . |w_f| + V(s)
             const float *a2t = a.a2[1] + m * ld2;
@@ -704,7 +711,9 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
             y = warp_sum(act ? fmaf(hidden, wf, v1 * v2w_o) : 0.0f) + v2b_o;
             ty = warp_sum(act ? fmaf(hidden_t, wf_t, v1_t * v2w_t) : 0.0f) + v2b_t;
         }
-        const float target = rew + a.gamma * (1.0f - term) * ty;
+        float target;
+        if (GIVEN_TARGETS) target = iql ? (lane < a.N ? a.targets[m * a.N + lane] : 0.0f) : a.targets[m];
+        else target = rew + a.gamma * (1.0f - term) * ty;
         const float tdv = y - target;
         const float mtd = tdv * mk;
         float gseed = 2.0f * mtd * mk;         // (d loss / d q_tot) * mask.sum()
@@ -717,13 +726,17 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
             if (lane == 0) a.mask[m] = mk;
             if (lane < a.N) {
                 const int64_t e = m * a.N + lane;
-                a.q_tot[e] = y; a.target_q_tot[e] = ty; a.targets[e] = target; a.td[e] = tdv;
+                a.q_tot[e] = y;
+                if (!GIVEN_TARGETS) { a.target_q_tot[e] = ty; a.targets[e] = target; }
+                a.td[e] = tdv;
                 st[0] += lterm; st[1] += fabsf(mtd); st[2] += y * mk; st[3] += target * mk;
                 st[4] += mk; st[5] += (mk != 0.0f) ? 1.0f : 0.0f;
             }
         } else if (lane == 0) {
             a.mask[m] = mk;
-            a.q_tot[m] = y; a.target_q_tot[m] = ty; a.targets[m] = target; a.td[m] = tdv;
+            a.q_tot[m] = y;
+            if (!GIVEN_TARGETS) { a.target_q_tot[m] = ty; a.targets[m] = target; }
+            a.td[m] = tdv;
             st[0] += lterm; st[1] += fabsf(mtd); st[2] += y * mk; st[3] += target * mk;
             st[4] += mk; st[5] += (mk != 0.0f) ? 1.0f : 0.0f;
         }
@@ -799,6 +812,13 @@ __global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) {
     }
 }
 
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(256, 4) k_mix_td(MixArgs a) { mix_td_body<WEIGHTED, false>(a); }
+
+// TD(lambda): the mixing / TD / seed step over the targets k_td_lambda left in a.targets
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(256, 4) k_mix_td_lambda(MixArgs a) { mix_td_body<WEIGHTED, true>(a); }
+
 // stand-alone mixer forward (QMixer.forward / VDNMixer.forward called outside the learner)
 __global__ void __launch_bounds__(256) k_mix_fwd(MixArgs a) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -812,7 +832,7 @@ __global__ void __launch_bounds__(256) k_mix_fwd(MixArgs a) {
         } else {
             float d0, d1, d2, d3;
             for (int n = 0; n < a.N; ++n) q[n] = a.chosen[m * a.N + n];
-            y = qmix_row(a, 0, m, q, lane, &d0, &d1, &d2, &d3);
+            y = qmix_row(a, 0, m, [&](int n) { return q[n]; }, lane, &d0, &d1, &d2, &d3);
         }
         if (lane == 0) a.q_tot[m] = y;
     }

@@ -14,6 +14,7 @@
 #include "tc_reduce.cuh"
 #include "autograd.cuh"
 #include "per.cuh"
+#include "td_lambda.cuh"
 
 // ---------------------------------------------------------------------------------------------
 static thread_local char g_err[512] = "";
@@ -606,6 +607,9 @@ static int get_dims(const mal_batch_t *b, const mal_learner_cfg_t *c, Dims *d) {
                 c->mixer == MAL_MIXER_NONE, "Mixer %d not recognised.", c->mixer);
     MAL_REQUIRE(!b->weight.ptr || !c->unnormalized,
                 "importance weights (prioritized replay) are not supported in unnormalized (data-parallel) mode");
+    MAL_REQUIRE(c->returns == MAL_RETURNS_ONE_STEP || c->returns == MAL_RETURNS_TD_LAMBDA, "returns %d not recognised",
+                c->returns);
+    MAL_REQUIRE(c->td_lambda >= 0.0f && c->td_lambda <= 1.0f, "td_lambda must be a number in [0, 1]");   // false for NaN
     d->B = b->B; d->TT = b->TT; d->T = b->TT - 1; d->N = b->N; d->A = b->A; d->OBS = b->OBS; d->S = b->S;
     MAL_REQUIRE(c->agent_kind == MAL_AGENT_RNN || c->agent_kind == MAL_AGENT_DQN, "agent kind %d not recognised", c->agent_kind);
     d->kind = c->agent_kind;
@@ -1217,7 +1221,28 @@ extern "C" int mal_learner_forward(const mal_batch_t *batch, const mal_learner_c
         a.d_a2 = F(plan->d_a2); a.d_y1 = F(plan->d_y1); a.d_chosen = F(plan->d_chosen);
         a.part_stats = parts + pl.mix_stats; a.part_v2 = parts + pl.mix_v2;
         a.weight = batch->weight;
-        if (batch->weight.ptr) {                     // prioritized replay: importance-weighted loss and seeds
+        if (cfg->returns == MAL_RETURNS_TD_LAMBDA) {
+            // TD(lambda): target rows, then the per-episode reverse recursion, then the step over the given targets
+            if (g_rec_carveout & 4) { static bool cv[MAL_MAX_DEV]; if (int rc = ensure_max_carveout(k_mix_tq, cv)) return rc; }
+            { ProfScope _ps("k_mix_tq", st); launch_k(k_mix_tq, dim3(pl.nblk_mix), dim3(256), 0, st, true, a); }
+            MAL_LAUNCH_CHECK("k_mix_tq");
+            TdLambdaArgs tl;
+            tl.tq = a.target_q_tot; tl.targets = a.targets;
+            tl.reward = batch->reward; tl.terminated = batch->terminated; tl.filled = batch->filled;
+            tl.B = d.B; tl.T = d.T; tl.Q = d.mixer == MAL_MIXER_NONE ? d.N : 1;
+            tl.lg = (double)cfg->td_lambda * (double)cfg->gamma;
+            tl.xg = (1.0 - (double)cfg->td_lambda) * (double)cfg->gamma;
+            const int64_t n_ep = (int64_t)tl.B * tl.Q;
+            { ProfScope _ps("k_td_lambda", st); launch_k(k_td_lambda, dim3((unsigned)ceil_div64(n_ep, TDL_WARPS)), dim3(32 * TDL_WARPS), 0, st, true, tl); }
+            MAL_LAUNCH_CHECK("k_td_lambda");
+            if (batch->weight.ptr) {
+                if (g_rec_carveout & 4) { static bool cv[MAL_MAX_DEV]; if (int rc = ensure_max_carveout(k_mix_td_lambda<true>, cv)) return rc; }
+                { ProfScope _ps("k_mix_td_lambda_w", st); launch_k(k_mix_td_lambda<true>, dim3(pl.nblk_mix), dim3(256), 0, st, true, a); }
+            } else {
+                if (g_rec_carveout & 4) { static bool cv[MAL_MAX_DEV]; if (int rc = ensure_max_carveout(k_mix_td_lambda<false>, cv)) return rc; }
+                { ProfScope _ps("k_mix_td_lambda", st); launch_k(k_mix_td_lambda<false>, dim3(pl.nblk_mix), dim3(256), 0, st, true, a); }
+            }
+        } else if (batch->weight.ptr) {              // prioritized replay: importance-weighted loss and seeds
             if (g_rec_carveout & 4) { static bool cv[MAL_MAX_DEV]; if (int rc = ensure_max_carveout(k_mix_td<true>, cv)) return rc; }
             { ProfScope _ps("k_mix_td_w", st); launch_k(k_mix_td<true>, dim3(pl.nblk_mix), dim3(256), 0, st, true, a); }
         } else {

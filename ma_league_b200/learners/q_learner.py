@@ -2,11 +2,13 @@
 (marl/learners/q_learner.py:11-147).
 
 `train()` is one call into libmal_b200 (`mal_learner_step`): online + target RNN unroll, chosen-Q gather, masked
-double-Q target max, mixers, TD loss, full backward (mixer + BPTT), clip_grad_norm_ and RMSprop.  Nothing is read
+double-Q target max, mixers, TD loss, full backward (mixer + BPTT), clip_grad_norm_ and RMSprop.  The TD targets are
+the 1-step targets of q_learner.py:86, or lambda-returns when `args.td_lambda` is a number in [0, 1] (INTEGRATION.md).  Nothing is read
 back to the host except on log steps (the reference syncs every step through `.item()`, q_learner.py:113).
 """
 import copy
 import ctypes as C
+import numbers
 
 import torch as th
 
@@ -91,7 +93,18 @@ class QLearner(Learner):
                               self.mixer.hypernet_embed if qm else 0, a.gamma, a.lr, a.optim_alpha, a.optim_eps,
                               a.grad_norm_clip, int(self.save_q), int(self._dp_world() > 1), int(self._agent_frozen()),
                               getattr(self.mac.agent, "mal_kind", nat.AGENT_RNN),
-                              nat.agent_input_flags(getattr(a, "obs_last_action", True), getattr(a, "obs_agent_id", True)))
+                              nat.agent_input_flags(getattr(a, "obs_last_action", True), getattr(a, "obs_agent_id", True)),
+                              *self._returns())
+
+    def _returns(self):
+        """(mal_learner_cfg_t.returns, td_lambda) from `args.td_lambda`: absent or None is the 1-step target of
+        q_learner.py:86; a number in [0, 1] selects TD(lambda) targets (build_td_lambda_targets, coma_learner.py:10-21)."""
+        lam = getattr(self.args, "td_lambda", None)
+        if lam is None:
+            return nat.RETURNS_ONE_STEP, 0.0
+        if isinstance(lam, bool) or not isinstance(lam, numbers.Real) or not 0.0 <= float(lam) <= 1.0:
+            raise nat.MalError("args.td_lambda must be None or a number in [0, 1], got %r" % (lam,))
+        return nat.RETURNS_TD_LAMBDA, float(lam)
 
     def _agent_frozen(self):
         """`freeze_agent_weights()` (multi_agent_controller.py:74-76, `args.freeze_native`): in the reference a frozen
