@@ -197,6 +197,35 @@ int mal_learner_step(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, con
                      float *agent, const float *target_agent, float *mixer, const float *target_mixer,
                      void *workspace, float *grad, float *square_avg, void *stream);
 
+/* Adam (torch.optim.Adam with amsgrad = False, maximize = False and L2 weight decay that is not decoupled) in place of
+ * RMSprop.  For the trained parameters (a frozen prefix is skipped), after clip_grad_norm_ scaled grad in place:
+ *     g' = g + weight_decay * p  (not written back) ; t = step + 1
+ *     m = beta1 m + (1 - beta1) g' ; v = beta2 v + (1 - beta2) g'^2
+ *     p -= (lr / (1 - beta1^t)) * m / (sqrt(v) / sqrt(1 - beta2^t) + eps) ; step = t
+ * with the bias corrections computed in double.  The caller owns the optimiser state, MAL_ADAM_STATE_FLOATS(P) floats
+ * for P = n_agent + n_mixer parameters, zeroed before the first step:
+ *     exp_avg [P] | exp_avg_sq [P] | step (f32) | ticket (u32 bits, must stay 0 between calls)
+ * The step counter lives in this buffer on the device, so a captured CUDA graph advances it on every replay.  As
+ * torch's float32 `step` state, it counts exactly up to 2^24 steps. */
+#define MAL_ADAM_STATE_FLOATS(P) (2 * (P) + 2)
+typedef struct mal_adam {
+    double lr, beta1, beta2, eps, weight_decay;   /* lr, betas, eps, weight_decay of the optimiser's param group */
+    float clip;                                   /* grad_norm_clip (q_learner.py:104) */
+} mal_adam_t;
+
+/* mal_learner_step with Adam: cfg->lr / alpha / eps / clip are not read, `adam` holds the hyper-parameters. */
+int mal_learner_step_adam(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
+                          float *agent, const float *target_agent, float *mixer, const float *target_mixer,
+                          void *workspace, float *grad, const mal_adam_t *adam, float *adam_state, void *stream);
+/* mal_clip_rmsprop with Adam (same grad, scalars, scratch, denominator and n_frozen contract). */
+int mal_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad, float *adam_state,
+                  const mal_adam_t *adam, float *scalars, float *scratch, const float *denominator, int64_t n_frozen,
+                  void *stream);
+/* mal_peer_allreduce_clip_rmsprop with Adam. */
+int mal_peer_allreduce_clip_adam(const void *const *peer_bufs, int32_t world, float *agent, int64_t n_agent, float *mixer,
+                                 int64_t n_mixer, float *grad_out, float *tail_out, int32_t tail, float *adam_state,
+                                 const mal_adam_t *adam, float *scalars, float *scratch, int64_t n_frozen, void *stream);
+
 /* update_targets, q_learner.py:127-131 (load_state_dict of the flat buffers). */
 int mal_copy_f32(float *dst, const float *src, int64_t n, void *stream);
 

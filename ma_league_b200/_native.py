@@ -56,6 +56,17 @@ _PLAN_FIELDS = ["total_bytes", "n_agent_params", "n_mixer_params", "x_on", "x_tg
                 "dh_head", "partials", "partials_bytes", "scalars", "w_t"]
 
 
+class AdamHyper(C.Structure):
+    """mal_adam_t: the hyper-parameters of the Adam step (mal_learner_step_adam, mal_clip_adam)."""
+    _fields_ = [("lr", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double),
+                ("weight_decay", C.c_double), ("clip", C.c_float)]
+
+
+def adam_state_floats(n_params: int) -> int:
+    """MAL_ADAM_STATE_FLOATS: exp_avg [P] | exp_avg_sq [P] | step (f32) | ticket (u32)."""
+    return 2 * n_params + 2
+
+
 class Plan(C.Structure):
     _fields_ = [(n, C.c_int64) for n in _PLAN_FIELDS]
 
@@ -114,6 +125,14 @@ _PROTOS = {
                                                   C.c_void_p]),
     "mal_learner_step": (C.c_int, [C.POINTER(Batch), C.POINTER(LearnerCfg), C.POINTER(Plan), C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mal_learner_step_adam": (C.c_int, [C.POINTER(Batch), C.POINTER(LearnerCfg), C.POINTER(Plan), C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(AdamHyper), C.c_void_p,
+                                        C.c_void_p]),
+    "mal_clip_adam": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                C.POINTER(AdamHyper), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "mal_peer_allreduce_clip_adam": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
+                                               C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                               C.POINTER(AdamHyper), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "mal_copy_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "mal_agent_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                  C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,

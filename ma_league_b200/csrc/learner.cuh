@@ -1042,14 +1042,10 @@ __global__ void __launch_bounds__(256) k_sumsq(float *g, int64_t n, float *norm_
 // =============================================================================================
 // clip_grad_norm_ (q_learner.py:104) + RMSprop.step (learner.py:25-31), one pass over the flat buffers
 // =============================================================================================
-__global__ void __launch_bounds__(256) k_clip_rmsprop(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer,
-                                                      float *grad, float *sq, const float *norm_part, int n_part,
-                                                      float lr, float alpha, float eps, float clip, float *scalars,
-                                                      const float *denominator, int64_t n_frozen) {
-    __shared__ float s_red[8];
-    __shared__ float s_coef;
-    pdl_wait();
-    // every block recomputes the global norm from the per-block partials in the same fixed order
+// The clip prologue of k_clip_rmsprop and k_clip_adam: every block recomputes the global norm from the per-block
+// partials in the same fixed order; thread 0 leaves min(clip / (norm + 1e-6), 1) in s_coef (read after a barrier).
+__device__ __forceinline__ void clip_coef_prologue(const float *norm_part, int n_part, float clip, float *scalars,
+                                                   float *s_red, float &s_coef) {
     float s = 0.0f;
     for (int i = threadIdx.x; i < n_part; i += 256) s += norm_part[i];
     s = warp_sum(s);
@@ -1063,6 +1059,16 @@ __global__ void __launch_bounds__(256) k_clip_rmsprop(float *agent, int64_t n_ag
         s_coef = coef < 1.0f ? coef : 1.0f;
         if (blockIdx.x == 0) scalars[MAL_SC_GRAD_NORM] = norm;
     }
+}
+
+__global__ void __launch_bounds__(256) k_clip_rmsprop(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer,
+                                                      float *grad, float *sq, const float *norm_part, int n_part,
+                                                      float lr, float alpha, float eps, float clip, float *scalars,
+                                                      const float *denominator, int64_t n_frozen) {
+    __shared__ float s_red[8];
+    __shared__ float s_coef;
+    pdl_wait();
+    clip_coef_prologue(norm_part, n_part, clip, scalars, s_red, s_coef);
     __syncthreads();
     const float coef = s_coef;
     const int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x;
@@ -1073,6 +1079,49 @@ __global__ void __launch_bounds__(256) k_clip_rmsprop(float *agent, int64_t n_ag
     const float v = alpha * sq[p] + (1.0f - alpha) * gv * gv;
     sq[p] = v;
     *param = *param - lr * gv / (sqrtf(v) + eps);
+}
+
+// clip_grad_norm_ + torch.optim.Adam.step (amsgrad = False, maximize = False, L2 weight decay added to the gradient),
+// one pass over the flat buffers.  state = exp_avg[P] | exp_avg_sq[P] | step (f32) | ticket (u32).  The step counter
+// lives on the device so that a replayed CUDA graph advances it: every block reads the old step, then takes a ticket;
+// the last block to arrive (all others have read by then) re-arms the ticket and writes step + 1.
+__global__ void __launch_bounds__(256) k_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer,
+                                                   float *grad, float *state, const float *norm_part, int n_part,
+                                                   mal_adam_t h, float *scalars, const float *denominator, int64_t n_frozen) {
+    __shared__ float s_red[8];
+    __shared__ float s_coef, s_step_size, s_bc2_sqrt;
+    pdl_wait();
+    const int64_t P = n_agent + n_mixer;
+    clip_coef_prologue(norm_part, n_part, h.clip, scalars, s_red, s_coef);
+    if (threadIdx.x == 0) {
+        const float step = state[2 * P];
+        const double t = (double)step + 1.0;
+        // bias corrections in double, as torch's non-capturable Adam computes them on the host
+        s_step_size = (float)(-h.lr / (1.0 - pow(h.beta1, t)));
+        s_bc2_sqrt = (float)sqrt(1.0 - pow(h.beta2, t));
+        unsigned *ticket = reinterpret_cast<unsigned *>(state + 2 * P + 1);
+        __threadfence();                                          // this block's read of step precedes its ticket
+        if (atomicAdd(ticket, 1u) == gridDim.x - 1) {
+            __threadfence();
+            *ticket = 0u;
+            state[2 * P] = step + 1.0f;
+        }
+    }
+    __syncthreads();
+    const float coef = s_coef, step_size = s_step_size, bc2_sqrt = s_bc2_sqrt;
+    const int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (p >= P || p < n_frozen) return;                           // frozen parameters: Adam skips them (p.grad is None)
+    float *param = p < n_agent ? agent + p : mixer + (p - n_agent);
+    float g = grad[p] * (denominator ? 1.0f / denominator[0] : 1.0f) * coef;
+    grad[p] = g;                                                  // clip_grad_norm_ scales .grad in place
+    const float pv = *param;
+    if (h.weight_decay != 0.0) g += (float)h.weight_decay * pv;  // grad.add(param, alpha=weight_decay): not written back
+    const float m = state[p], v = state[P + p];
+    const float mn = m + (float)(1.0 - h.beta1) * (g - m);                 // exp_avg.lerp_(grad, 1 - beta1)
+    const float vn = v * (float)h.beta2 + (float)(1.0 - h.beta2) * g * g;  // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1 - beta2)
+    state[p] = mn;
+    state[P + p] = vn;
+    *param = pv + step_size * (mn / (sqrtf(vn) / bc2_sqrt + (float)h.eps));   // addcdiv_(exp_avg, denom, -step_size)
 }
 
 __global__ void __launch_bounds__(256) k_copy_f32(float *dst, const float *src, int64_t n) {

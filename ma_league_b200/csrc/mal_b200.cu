@@ -1914,6 +1914,22 @@ extern "C" int mal_clip_rmsprop(float *agent, int64_t n_agent, float *mixer, int
                                scalars, denominator, n_frozen, (cudaStream_t)stream);
 }
 
+// k_peer_allreduce_grad: rank-order sum of the peers' un-normalised halves into grad_out / tail_out, and the norm partials
+static int peer_allreduce(const char *who, const void *const *peer_bufs, int32_t world, int64_t P, float *grad_out,
+                          float *tail_out, int32_t tail, float *scratch, int64_t n_frozen, cudaStream_t st) {
+    MAL_REQUIRE(peer_bufs && world >= 1 && world <= PEER_MAX, "%s: world size must be in [1, %d]", who, PEER_MAX);
+    PeerBufs pb;
+    memset(&pb, 0, sizeof(pb));
+    pb.world = world;
+    for (int r = 0; r < world; ++r) {
+        MAL_REQUIRE(peer_bufs[r], "%s: null peer buffer", who);
+        pb.p[r] = reinterpret_cast<const float *>(peer_bufs[r]);
+    }
+    { ProfScope _ps("k_peer_allreduce_grad", st); k_peer_allreduce_grad<<<(unsigned)ceil_div64(P, 256), 256, 0, st>>>(pb, P, tail, grad_out, tail_out, scratch, n_frozen); }
+    MAL_LAUNCH_CHECK("k_peer_allreduce_grad");
+    return 0;
+}
+
 extern "C" int mal_peer_allreduce_clip_rmsprop(const void *const *peer_bufs, int32_t world, float *agent, int64_t n_agent,
                                                float *mixer, int64_t n_mixer, float *grad_out, float *tail_out, int32_t tail,
                                                float *square_avg, float lr, float alpha, float eps, float clip,
@@ -1922,26 +1938,19 @@ extern "C" int mal_peer_allreduce_clip_rmsprop(const void *const *peer_bufs, int
     MAL_REQUIRE(peer_bufs && world >= 1 && world <= PEER_MAX, "mal_peer_allreduce_clip_rmsprop: world size must be in [1, %d]", PEER_MAX);
     MAL_REQUIRE(agent && grad_out && tail_out && square_avg && scalars && scratch && n_agent > 0 && n_mixer >= 0 && tail >= 5 && tail <= 32,
                 "mal_peer_allreduce_clip_rmsprop: bad arguments (scratch needs ceil(P/256) floats, tail >= 5)");
-    PeerBufs pb;
-    memset(&pb, 0, sizeof(pb));
-    pb.world = world;
-    for (int r = 0; r < world; ++r) {
-        MAL_REQUIRE(peer_bufs[r], "mal_peer_allreduce_clip_rmsprop: null peer buffer");
-        pb.p[r] = reinterpret_cast<const float *>(peer_bufs[r]);
-    }
     const int64_t P = n_agent + n_mixer;
-    const int nb = (int)ceil_div64(P, 256);
     cudaStream_t st = (cudaStream_t)stream;
-    { ProfScope _ps("k_peer_allreduce_grad", st); k_peer_allreduce_grad<<<nb, 256, 0, st>>>(pb, P, tail, grad_out, tail_out, scratch, n_frozen); }
-    MAL_LAUNCH_CHECK("k_peer_allreduce_grad");
-    return launch_clip_rmsprop(agent, n_agent, mixer, n_mixer, grad_out, square_avg, scratch, nb, lr, alpha, eps, clip,
+    if (int rc = peer_allreduce("mal_peer_allreduce_clip_rmsprop", peer_bufs, world, P, grad_out, tail_out, tail, scratch, n_frozen, st)) return rc;
+    return launch_clip_rmsprop(agent, n_agent, mixer, n_mixer, grad_out, square_avg, scratch, (int)ceil_div64(P, 256), lr, alpha, eps, clip,
                                scalars, nullptr, n_frozen, st);
 }
 
-extern "C" int mal_learner_step(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
+// forward + backward of the fused step (mal_learner_step, mal_learner_step_adam); *norm_part / *n_part / *scalars are
+// the inputs of the optimiser kernel's clip prologue
+static int learner_step_fwd_bwd(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
                                 float *agent, const float *target_agent, float *mixer, const float *target_mixer,
-                                void *workspace, float *grad, float *square_avg, void *stream) {
-    MAL_REQUIRE(square_avg, "mal_learner_step: square_avg missing");
+                                void *workspace, float *grad, void *stream, const float **norm_part, int *n_part,
+                                float **scalars) {
     MAL_REQUIRE(!cfg || !cfg->unnormalized, "mal_learner_step: unnormalized (data-parallel) mode needs the split calls");
     g_defer_stats = true;
     const int rc_f = mal_learner_forward(batch, cfg, plan, agent, target_agent, mixer, target_mixer, workspace, stream);
@@ -1957,11 +1966,92 @@ extern "C" int mal_learner_step(const mal_batch_t *batch, const mal_learner_cfg_
     if (device_sm_count(&sms, &tps)) return 2;
     const PartLayout pl = part_layout(d, sms);
     uint8_t *ws = (uint8_t *)workspace;
-    float *parts = reinterpret_cast<float *>(ws + plan->partials);
-    float *scalars = reinterpret_cast<float *>(ws + plan->scalars);
+    *norm_part = reinterpret_cast<const float *>(ws + plan->partials) + pl.norm;
+    *n_part = pl.nblk_norm;
+    *scalars = reinterpret_cast<float *>(ws + plan->scalars);
+    return 0;
+}
+
+extern "C" int mal_learner_step(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
+                                float *agent, const float *target_agent, float *mixer, const float *target_mixer,
+                                void *workspace, float *grad, float *square_avg, void *stream) {
+    MAL_REQUIRE(square_avg, "mal_learner_step: square_avg missing");
+    const float *norm_part;
+    int n_part;
+    float *scalars;
+    if (int rc = learner_step_fwd_bwd(batch, cfg, plan, agent, target_agent, mixer, target_mixer, workspace, grad, stream,
+                                      &norm_part, &n_part, &scalars)) return rc;
     return launch_clip_rmsprop(agent, plan->n_agent_params, mixer, plan->n_mixer_params, grad, square_avg,
-                               parts + pl.norm, pl.nblk_norm, cfg->lr, cfg->alpha, cfg->eps, cfg->clip, scalars,
+                               norm_part, n_part, cfg->lr, cfg->alpha, cfg->eps, cfg->clip, scalars,
                                nullptr, cfg->freeze_agent ? plan->n_agent_params : 0, (cudaStream_t)stream, true);   // stream predecessor: k_grad_reduce
+}
+
+// ---------------------------------------------------------------------------------------------
+// Adam
+// ---------------------------------------------------------------------------------------------
+static int check_adam(const char *who, const mal_adam_t *h, const float *state) {
+    MAL_REQUIRE(h && state, "%s: adam hyper-parameters or state missing", who);
+    MAL_REQUIRE((reinterpret_cast<uintptr_t>(state) & 3) == 0, "%s: adam_state must be 4-byte aligned", who);
+    MAL_REQUIRE(h->lr >= 0.0 && h->eps >= 0.0 && h->weight_decay >= 0.0 && h->beta1 >= 0.0 && h->beta1 < 1.0 &&
+                h->beta2 >= 0.0 && h->beta2 < 1.0,
+                "%s: need lr, eps, weight_decay >= 0 and betas in [0, 1) (torch.optim.Adam's checks)", who);
+    return 0;
+}
+
+static int launch_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad, float *state,
+                            const float *norm_part, int n_part, const mal_adam_t &h, float *scalars,
+                            const float *denominator, int64_t n_frozen, cudaStream_t st, bool pdl = false) {
+    const int64_t P = n_agent + n_mixer;
+    { ProfScope _ps("k_clip_adam", st); launch_k(k_clip_adam, dim3((unsigned)ceil_div64(P, 256)), dim3(256), 0, st, pdl, agent, n_agent, mixer, n_mixer, grad, state,
+                                                             norm_part, n_part, h, scalars, denominator, n_frozen); }
+    MAL_LAUNCH_CHECK("k_clip_adam");
+    return 0;
+}
+
+extern "C" int mal_learner_step_adam(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
+                                     float *agent, const float *target_agent, float *mixer, const float *target_mixer,
+                                     void *workspace, float *grad, const mal_adam_t *adam, float *adam_state, void *stream) {
+    if (int rc = check_adam("mal_learner_step_adam", adam, adam_state)) return rc;
+    const float *norm_part;
+    int n_part;
+    float *scalars;
+    if (int rc = learner_step_fwd_bwd(batch, cfg, plan, agent, target_agent, mixer, target_mixer, workspace, grad, stream,
+                                      &norm_part, &n_part, &scalars)) return rc;
+    return launch_clip_adam(agent, plan->n_agent_params, mixer, plan->n_mixer_params, grad, adam_state, norm_part, n_part,
+                            *adam, scalars, nullptr, cfg->freeze_agent ? plan->n_agent_params : 0, (cudaStream_t)stream,
+                            true);   // stream predecessor: k_grad_reduce
+}
+
+extern "C" int mal_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad, float *adam_state,
+                             const mal_adam_t *adam, float *scalars, float *scratch, const float *denominator,
+                             int64_t n_frozen, void *stream) {
+    if (int rc = check_adam("mal_clip_adam", adam, adam_state)) return rc;
+    MAL_REQUIRE(agent && grad && scalars && scratch && n_agent > 0 && n_mixer >= 0,
+                "mal_clip_adam: bad arguments (scratch needs ceil(P/256) floats)");
+    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "mal_clip_adam: n_frozen out of range");
+    MAL_REQUIRE(n_mixer == 0 || mixer, "mal_clip_adam: mixer buffer missing");
+    const int64_t P = n_agent + n_mixer;
+    const int nb = (int)ceil_div64(P, 256);
+    { ProfScope _ps("k_sumsq", (cudaStream_t)stream); k_sumsq<<<nb, 256, 0, (cudaStream_t)stream>>>(grad, P, scratch, denominator, n_frozen); }
+    MAL_LAUNCH_CHECK("k_sumsq");
+    return launch_clip_adam(agent, n_agent, mixer, n_mixer, grad, adam_state, scratch, nb, *adam, scalars, denominator,
+                            n_frozen, (cudaStream_t)stream);
+}
+
+extern "C" int mal_peer_allreduce_clip_adam(const void *const *peer_bufs, int32_t world, float *agent, int64_t n_agent,
+                                            float *mixer, int64_t n_mixer, float *grad_out, float *tail_out, int32_t tail,
+                                            float *adam_state, const mal_adam_t *adam, float *scalars, float *scratch,
+                                            int64_t n_frozen, void *stream) {
+    if (int rc = check_adam("mal_peer_allreduce_clip_adam", adam, adam_state)) return rc;
+    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "mal_peer_allreduce_clip_adam: n_frozen out of range");
+    MAL_REQUIRE(agent && grad_out && tail_out && scalars && scratch && n_agent > 0 && n_mixer >= 0 && tail >= 5 && tail <= 32,
+                "mal_peer_allreduce_clip_adam: bad arguments (scratch needs ceil(P/256) floats, tail >= 5)");
+    MAL_REQUIRE(n_mixer == 0 || mixer, "mal_peer_allreduce_clip_adam: mixer buffer missing");
+    const int64_t P = n_agent + n_mixer;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = peer_allreduce("mal_peer_allreduce_clip_adam", peer_bufs, world, P, grad_out, tail_out, tail, scratch, n_frozen, st)) return rc;
+    return launch_clip_adam(agent, n_agent, mixer, n_mixer, grad_out, adam_state, scratch, (int)ceil_div64(P, 256), *adam,
+                            scalars, nullptr, n_frozen, st);
 }
 
 extern "C" int mal_copy_f32(float *dst, const float *src, int64_t n, void *stream) {

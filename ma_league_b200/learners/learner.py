@@ -1,6 +1,7 @@
-"""Learner base (reference: marl/learners/learner.py:6-78): name prefix + RMSprop construction."""
+"""Learner base (reference: marl/learners/learner.py:6-78): name prefix + optimiser construction (RMSprop, or Adam
+with `args.optimizer: "adam"` as pymarl2's configs select it)."""
 import torch as th
-from torch.optim import RMSprop
+from torch.optim import Adam, RMSprop
 
 from .. import _native as nat
 from ..flat import flat_views
@@ -38,11 +39,69 @@ class FusedRMSprop(RMSprop):
         return super().state_dict()
 
     def load_state_dict(self, state_dict):
+        if any("alpha" not in g or "betas" in g for g in state_dict["param_groups"]):
+            raise nat.MalError("not a torch.optim.RMSprop state dict (an Adam checkpoint needs args.optimizer: adam)")
         super().load_state_dict(state_dict)
         self._bind(True)
 
     def step(self, closure=None):
         raise nat.MalError("FusedRMSprop is stepped by QLearner.train (clip + RMSprop run inside mal_learner_step)")
+
+
+class FusedAdam(Adam):
+    """torch.optim.Adam (amsgrad=False, maximize=False, L2 weight decay that is not decoupled; betas and eps at torch's
+    defaults unless a loaded state dict brings its own) whose state lives in ONE flat device buffer
+    `exp_avg[P] | exp_avg_sq[P] | step | ticket` (MAL_ADAM_STATE_FLOATS) and whose step is the fused clip+Adam kernel.
+    `exp_avg`, `exp_avg_sq` and `step` of every parameter are views of that buffer; the step counter lives on the device
+    so that a replayed CUDA graph advances it.  state_dict()/load_state_dict() keep torch's format (a CPU float32
+    `step` per parameter), so checkpoints interoperate with a stock torch.optim.Adam."""
+
+    def __init__(self, params, lr, weight_decay=0.0):
+        params = list(params)
+        super().__init__(params, lr=lr, weight_decay=weight_decay)
+        self._plist = params
+        self._steps = 0
+        self.flat_state = None
+        self._bind(None)
+
+    def _bind(self, loaded):
+        P = sum(p.numel() for p in self._plist)
+        dev = self._plist[0].device
+        self.flat_state = th.zeros(nat.adam_state_floats(P), dtype=th.float32, device=dev)
+        steps = 0
+        for p, m, v in zip(self._plist, flat_views(self.flat_state, self._plist), flat_views(self.flat_state, self._plist, P)):
+            st = self.state[p]
+            if loaded and "exp_avg" in st:
+                m.copy_(st["exp_avg"].to(dev))
+                v.copy_(st["exp_avg_sq"].to(dev))
+                steps = max(steps, int(st["step"].item()))
+            st["exp_avg"], st["exp_avg_sq"], st["step"] = m, v, self.flat_state[2 * P]
+        self._steps = steps
+        self.flat_state[2 * P] = float(steps)
+
+    def hyper(self, lr, clip):
+        """mal_adam_t of this optimiser: betas, eps and weight_decay from param_groups[0], lr and clip from the args."""
+        g = self.param_groups[0]
+        return nat.AdamHyper(lr, g["betas"][0], g["betas"][1], g["eps"], g["weight_decay"], clip)
+
+    def state_dict(self):
+        sd = super().state_dict()
+        step = th.tensor(float(self._steps))           # the host count equals the device counter; no sync needed
+        sd["state"] = {k: dict(v, step=step.clone()) for k, v in sd["state"].items()}
+        return sd
+
+    def load_state_dict(self, state_dict):
+        for g in state_dict["param_groups"]:
+            if "betas" not in g or "alpha" in g:
+                raise nat.MalError("not a torch.optim.Adam state dict (a RMSprop checkpoint needs args.optimizer: rmsprop)")
+            for k in ("amsgrad", "maximize", "decoupled_weight_decay"):
+                if g.get(k, False):
+                    raise nat.MalError("the fused Adam step does not support %s=True" % k)
+        super().load_state_dict(state_dict)
+        self._bind(True)
+
+    def step(self, closure=None):
+        raise nat.MalError("FusedAdam is stepped by QLearner.train (clip + Adam run inside mal_learner_step_adam)")
 
 
 class Learner:
@@ -56,8 +115,16 @@ class Learner:
         self.optimiser = None
 
     def build_optimizer(self):
-        self.optimiser = FusedRMSprop(params=self.parameters(), lr=self.args.lr, alpha=self.args.optim_alpha,
-                                      eps=self.args.optim_eps)
+        """`args.optimizer`: absent or "rmsprop" (learner.py:25-31), or "adam" (pymarl2's qmix configs)."""
+        kind = getattr(self.args, "optimizer", None)
+        if kind is None or kind == "rmsprop":
+            self.optimiser = FusedRMSprop(params=self.parameters(), lr=self.args.lr, alpha=self.args.optim_alpha,
+                                          eps=self.args.optim_eps)
+        elif kind == "adam":
+            self.optimiser = FusedAdam(params=self.parameters(), lr=self.args.lr,
+                                       weight_decay=getattr(self.args, "weight_decay", 0.0))
+        else:
+            raise nat.MalError('args.optimizer must be "rmsprop" or "adam", got %r' % (kind,))
 
     def parameters(self):
         raise NotImplementedError()

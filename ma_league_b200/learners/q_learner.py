@@ -2,7 +2,8 @@
 (marl/learners/q_learner.py:11-147).
 
 `train()` is one call into libmal_b200 (`mal_learner_step`): online + target RNN unroll, chosen-Q gather, masked
-double-Q target max, mixers, TD loss, full backward (mixer + BPTT), clip_grad_norm_ and RMSprop.  The TD targets are
+double-Q target max, mixers, TD loss, full backward (mixer + BPTT), clip_grad_norm_ and RMSprop, or Adam with
+`args.optimizer: "adam"` (`mal_learner_step_adam`).  The TD targets are
 the 1-step targets of q_learner.py:86, or lambda-returns when `args.td_lambda` is a number in [0, 1] (INTEGRATION.md).  Nothing is read
 back to the host except on log steps (the reference syncs every step through `.item()`, q_learner.py:113).
 """
@@ -16,7 +17,7 @@ from .. import _native as nat
 from ..flat import ensure_flat, flat_views
 from ..modules.mixers.qmix import QMixer
 from ..modules.mixers.vdn import VDNMixer
-from .learner import Learner
+from .learner import FusedAdam, Learner
 
 
 DP_RAW = 6     # raw sums written by k_stats_finalize at scalars[SC_RAW0:]: sum mtd^2, sum|mtd|, sum q_tot*m,
@@ -216,13 +217,14 @@ class QLearner(Learner):
         dev = batch["obs"].device
         dp = cfg.unnormalized != 0
         self._set_weights(bs, weights, dev, dp)
+        adam = self._adam()
         counted = False                          # True: the trained-steps counter was advanced inside the replayed graph
         if dp:
-            self._train_data_parallel(bs, cfg, f, dev)
+            self._train_data_parallel(bs, cfg, f, dev, adam)
         elif self.use_graphs and not self.save_q:
-            counted = self._step_graphed(bs, cfg, f, dev)
+            counted = self._step_graphed(bs, cfg, f, dev, adam)
         else:
-            self._step_eager(bs, cfg, f, dev)
+            self._step_eager(bs, cfg, f, dev, adam)
         self.optimiser._steps += 1
         if getattr(self, "_grad_views", None) is None:   # p.grad = views of the flat (clipped) gradient, bound once
             params = self.parameters()
@@ -267,7 +269,20 @@ class QLearner(Learner):
             raise nat.MalError("weights must be a float32 [B] tensor on the batch's device")
         bs.weight = nat.Field(weights.data_ptr(), weights.stride(0), 0)
 
-    def _step_eager(self, bs, cfg, f, dev):
+    def _adam(self):
+        """The optimiser kernel of every training path: None selects clip + RMSprop (FusedRMSprop), a mal_adam_t
+        clip + Adam (FusedAdam, lr and clip read from the args like the RMSprop path reads them)."""
+        opt = self.optimiser
+        return opt.hyper(self.args.lr, self.args.grad_norm_clip) if isinstance(opt, FusedAdam) else None
+
+    def _step_eager(self, bs, cfg, f, dev, adam):
+        if adam is not None:
+            with nat.on_device(dev):
+                nat.check(nat.lib().mal_learner_step_adam(
+                    C.byref(bs), C.byref(cfg), C.byref(self._plan), nat.ptr(f["agent"]), nat.ptr(f["tagent"]),
+                    nat.ptr(f["mixer"]), nat.ptr(f["tmixer"]), nat.ptr(self._ws), nat.ptr(self._grad), C.byref(adam),
+                    nat.ptr(self.optimiser.flat_state), nat.current_stream(dev)), "mal_learner_step_adam")
+            return
         with nat.on_device(dev):
             nat.check(nat.lib().mal_learner_step(C.byref(bs), C.byref(cfg), C.byref(self._plan),
                                                  nat.ptr(f["agent"]), nat.ptr(f["tagent"]), nat.ptr(f["mixer"]),
@@ -275,7 +290,7 @@ class QLearner(Learner):
                                                  nat.ptr(self.optimiser.flat_sq), nat.current_stream(dev)),
                       "mal_learner_step")
 
-    def _step_graphed(self, bs, cfg, f, dev):
+    def _step_graphed(self, bs, cfg, f, dev, adam):
         """Replay the captured step when this exact set of device addresses / shapes / hyper-parameters was seen
         before; first sighting runs eagerly (it also warms the library's streams and kernel attributes), the second
         one captures."""
@@ -283,7 +298,8 @@ class QLearner(Learner):
         key = (tuple((x.ptr, x.sb, x.st) for x in fields), bs.B, bs.TT, bs.N, bs.A, bs.OBS, bs.S,
                tuple(getattr(cfg, n) for n, _ in cfg._fields_),
                tuple(0 if v is None else v.data_ptr() for v in f.values()), self._ws.data_ptr(), self._grad.data_ptr(),
-               self.optimiser.flat_sq.data_ptr(), str(dev))
+               self.optimiser.flat_sq.data_ptr() if adam is None else
+               (self.optimiser.flat_state.data_ptr(),) + tuple(getattr(adam, n) for n, _ in adam._fields_), str(dev))
         entry = self._graphs.get(key, False)
         if entry:
             graph, n_kernels = entry
@@ -295,11 +311,11 @@ class QLearner(Learner):
             if len(self._graphs) >= self._graph_cap:
                 self._graphs.pop(next(iter(self._graphs)))
             self._graphs[key] = None
-            self._step_eager(bs, cfg, f, dev)
+            self._step_eager(bs, cfg, f, dev, adam)
             self.n_eager_steps += 1
             return False
         if self._graph_captures_left <= 0:
-            self._step_eager(bs, cfg, f, dev)
+            self._step_eager(bs, cfg, f, dev, adam)
             self.n_eager_steps += 1
             return False
         self._graph_captures_left -= 1
@@ -312,22 +328,22 @@ class QLearner(Learner):
         sc = self.scalars()
         self.mac.update_trained_steps(th.zeros(1, dtype=th.int32, device=dev))      # the device counter exists before capture
         with th.cuda.graph(graph, capture_error_mode="thread_local"):   # other threads may keep using CUDA meanwhile
-            self._step_eager(bs, cfg, f, dev)
+            self._step_eager(bs, cfg, f, dev, adam)
             self.mac.update_trained_steps(sc[nat.SC_MASK_COUNT:nat.SC_MASK_COUNT + 1].view(th.int32))
         n_kernels = lib.mal_launch_count() - n0
         self._graphs[key] = (graph, n_kernels)
         graph.replay()                          # capture only records: this performs the step
         return True
 
-    def _train_data_parallel(self, bs, cfg, f, dev):
+    def _train_data_parallel(self, bs, cfg, f, dev, adam):
         """Config 5 (SURVEY.md 8e): every rank back-propagates the UN-normalised sum over its batch shard, one
         all-reduce(sum) carries the flat gradient plus the raw statistic sums (incl. mask.sum()), then every rank
-        divides by the global mask sum and applies the identical clip + RMSprop, which reproduces
+        divides by the global mask sum and applies the identical clip + RMSprop (or Adam), which reproduces
         `loss = sum(masked_td^2) / mask.sum()` of q_learner.py:98 over the global batch."""
         import torch.distributed as dist
         sym = self._dp_symmetric(self._grad.numel(), dev)
         if sym is not None:
-            return self._train_data_parallel_fused(bs, cfg, f, dev, sym)
+            return self._train_data_parallel_fused(bs, cfg, f, dev, sym, adam)
         lib, st = nat.lib(), nat.current_stream(dev)
         n_total = self._grad.numel()
         with nat.on_device(dev):
@@ -344,13 +360,19 @@ class QLearner(Learner):
         dist.all_reduce(self._grad_store, op=dist.ReduceOp.SUM)
         denom = self._grad_store[n_total + 4:]            # global mask.sum()
         a = self.args
+        n_frozen = self._plan.n_agent_params if cfg.freeze_agent else 0
         with nat.on_device(dev):
-            nat.check(lib.mal_clip_rmsprop(nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
-                                           self._plan.n_mixer_params, nat.ptr(self._grad),
-                                           nat.ptr(self.optimiser.flat_sq), a.lr, a.optim_alpha, a.optim_eps,
-                                           a.grad_norm_clip, nat.ptr(self.scalars()), nat.ptr(self._dp_scratch),
-                                           nat.ptr(denom), self._plan.n_agent_params if cfg.freeze_agent else 0, st),
-                      "mal_clip_rmsprop")
+            if adam is not None:
+                nat.check(lib.mal_clip_adam(nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
+                                            self._plan.n_mixer_params, nat.ptr(self._grad),
+                                            nat.ptr(self.optimiser.flat_state), C.byref(adam), nat.ptr(self.scalars()),
+                                            nat.ptr(self._dp_scratch), nat.ptr(denom), n_frozen, st), "mal_clip_adam")
+            else:
+                nat.check(lib.mal_clip_rmsprop(nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
+                                               self._plan.n_mixer_params, nat.ptr(self._grad),
+                                               nat.ptr(self.optimiser.flat_sq), a.lr, a.optim_alpha, a.optim_eps,
+                                               a.grad_norm_clip, nat.ptr(self.scalars()), nat.ptr(self._dp_scratch),
+                                               nat.ptr(denom), n_frozen, st), "mal_clip_rmsprop")
         if self.dp_profile is not None:
             ev1 = th.cuda.Event(enable_timing=True)
             ev1.record()
@@ -386,7 +408,7 @@ class QLearner(Learner):
             return None
         return self._dp_sym
 
-    def _train_data_parallel_fused(self, bs, cfg, f, dev, sym):
+    def _train_data_parallel_fused(self, bs, cfg, f, dev, sym, adam):
         buf, hdl, ptrs = sym
         lib, st = nat.lib(), nat.current_stream(dev)
         n_total = self._grad.numel()
@@ -405,13 +427,20 @@ class QLearner(Learner):
             ev0.record()
         hdl.barrier(channel=0)                           # every rank's half h is complete (and half h^1 is free again)
         a = self.args
+        n_frozen = self._plan.n_agent_params if cfg.freeze_agent else 0
         with nat.on_device(dev):
-            nat.check(lib.mal_peer_allreduce_clip_rmsprop(
-                ptrs[h], hdl.world_size, nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
-                self._plan.n_mixer_params, nat.ptr(self._grad), nat.ptr(self._grad_store[n_total:]), DP_TAIL,
-                nat.ptr(self.optimiser.flat_sq), a.lr, a.optim_alpha, a.optim_eps, a.grad_norm_clip,
-                nat.ptr(self.scalars()), nat.ptr(self._dp_scratch),
-                self._plan.n_agent_params if cfg.freeze_agent else 0, st), "mal_peer_allreduce_clip_rmsprop")
+            if adam is not None:
+                nat.check(lib.mal_peer_allreduce_clip_adam(
+                    ptrs[h], hdl.world_size, nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
+                    self._plan.n_mixer_params, nat.ptr(self._grad), nat.ptr(self._grad_store[n_total:]), DP_TAIL,
+                    nat.ptr(self.optimiser.flat_state), C.byref(adam), nat.ptr(self.scalars()), nat.ptr(self._dp_scratch),
+                    n_frozen, st), "mal_peer_allreduce_clip_adam")
+            else:
+                nat.check(lib.mal_peer_allreduce_clip_rmsprop(
+                    ptrs[h], hdl.world_size, nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
+                    self._plan.n_mixer_params, nat.ptr(self._grad), nat.ptr(self._grad_store[n_total:]), DP_TAIL,
+                    nat.ptr(self.optimiser.flat_sq), a.lr, a.optim_alpha, a.optim_eps, a.grad_norm_clip,
+                    nat.ptr(self.scalars()), nat.ptr(self._dp_scratch), n_frozen, st), "mal_peer_allreduce_clip_rmsprop")
         if self.dp_profile is not None:
             ev1 = th.cuda.Event(enable_timing=True)
             ev1.record()
