@@ -356,6 +356,47 @@ int mal_debug_linear(int32_t M, int32_t K, int32_t Nout, const float *A, int64_t
                      int32_t w_trans, const float *bias, int32_t epi, const float *aux, int64_t ld_aux, float *Y,
                      int64_t ldy, int32_t use_tc, void *stream);
 
+/* Unit-test hooks for the split-M weight-gradient reductions of the learner's backward, dW[n,k] = sum_m dY[m,n] A[m,k].
+ * Each launches exactly the kernel instance the learner launches and writes the RAW per-chunk partials (no gather): chunk c
+ * covers rows [c * rows_per_chunk, min((c + 1) * rows_per_chunk, M)), n_chunks = ceil(M / rows_per_chunk).  rows_per_chunk
+ * must be a positive multiple of 64 and M < 2^31.  The mal_stat counters tick as in the learner.
+ *
+ * mal_debug_reduce: 1 to 3 problems as one grouped launch; part_w [n_chunks][Nout][K], part_b [n_chunks][Nout] (NULL: no
+ * bias).  All problems share the A loader a_kind:
+ *   MAL_RED_A_DENSE     row m reads A[(m - shift) * lda ..] (zero for m < shift);
+ *   MAL_RED_A_STATE     row m = b*T + t reads batch->state[b, t + shift] (T = TT - 1, shift <= 1, K <= S, M <= B*T);
+ *   MAL_RED_A_AGENT_IN  row m = t*R + b*N + n (R = B*N) reads [obs | one-hot(a_{t-1}) | agent id] as the MAL_IN_* bits of
+ *                       agent_input select them (K = d_in, shift 0, M <= TT*R).
+ *   batch is read by the last two only.  flavour: 0 fp32 FFMA (k_reduce_group); 1, 2, 3 tcgen05 k_reduce_tc with
+ *   "reduce_mn" = 0, 1, 2; 4 the 512-thread k_reduce_tc3 ("reduce_mn" = 3, the default).
+ * mal_debug_reduce_gru: the fused GRU weight gradients (k_reduce_gru) over M1 rows with h_{t-1}[m] = hout[m - R] (zero for
+ *   m < R).  x, hout [M1,64], d_g [M1,256] contiguous and 16-byte aligned.  Per chunk: wih_w [192][64] = d_g[:, :192]^T x,
+ *   whh_rz_w [128][64] = d_g[:, :128]^T h_{t-1}, whh_n_w [64][64] = d_g[:, 192:]^T h_{t-1}, the biases the column sums.
+ * mal_debug_reduce_fc1: the fc1 weight gradient over the full input width (k_reduce_fc1), d_x [M,64] contiguous and 16-byte
+ *   aligned, rows and input columns as MAL_RED_A_AGENT_IN; d_in <= 256.  part_w [n_chunks][64][d_in], part_b [n_chunks][64].
+ * mal_debug_fc2_grad: the fc2 gradients (k_fc2_grad) over the T*R rows of the batch's actions, d_chosen [B,T,N] and hout
+ *   [TT*R,64] (8-byte aligned) on `grid` CTAs: part_w [grid][A][64], part_b [grid][A]; CTA c sums the rows m whose
+ *   m mod (8 grid) lies in [8c, 8c + 8). */
+typedef struct mal_red_prob {
+    int64_t M, rows_per_chunk;
+    int32_t K, Nout, shift;
+    const float *dY;
+    int64_t ldy;
+    const float *A;                   /* MAL_RED_A_DENSE only */
+    int64_t lda;
+    float *part_w, *part_b;
+} mal_red_prob_t;
+enum { MAL_RED_A_DENSE = 0, MAL_RED_A_AGENT_IN = 1, MAL_RED_A_STATE = 2 };
+int mal_debug_reduce(int32_t flavour, int32_t a_kind, int32_t n_probs, const mal_red_prob_t *probs,
+                     const mal_batch_t *batch, int32_t agent_input, void *stream);
+int mal_debug_reduce_gru(const float *x, const float *hout, const float *d_g, int64_t M1, int32_t R, int64_t rows_per_chunk,
+                         float *wih_w, float *wih_b, float *whh_rz_w, float *whh_rz_b, float *whh_n_w, float *whh_n_b,
+                         void *stream);
+int mal_debug_reduce_fc1(const mal_batch_t *batch, int32_t agent_input, const float *d_x, int64_t M, int64_t rows_per_chunk,
+                         float *part_w, float *part_b, void *stream);
+int mal_debug_fc2_grad(const mal_batch_t *batch, const float *d_chosen, const float *hout, int32_t grid, float *part_w,
+                       float *part_b, void *stream);
+
 /* QMixer.forward / VDNMixer.forward outside the learner, qmix.py:41-59 / vdn.py:9-10 (MAL_MIXER_NONE is rejected:
  * there is no mixer module to run).
  * agent_qs [B*T,N] contiguous, states [B,T,S] with strides in elements, scratch >= B*T*(2*HE+2*E + E*N+E)

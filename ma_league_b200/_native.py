@@ -89,6 +89,17 @@ class RolloutIO(C.Structure):
                 ("agent_input", C.c_int32)]
 
 
+RED_A_DENSE, RED_A_AGENT_IN, RED_A_STATE = 0, 1, 2   # mal_red_prob_t loaders (mal_debug_reduce a_kind)
+RED_FFMA, RED_TC_MN0, RED_TC_MN1, RED_TC_MN2, RED_TC3 = range(5)   # mal_debug_reduce flavour
+
+
+class RedProb(C.Structure):
+    """mal_red_prob_t: one problem of mal_debug_reduce."""
+    _fields_ = [("M", C.c_int64), ("rows_per_chunk", C.c_int64), ("K", C.c_int32), ("Nout", C.c_int32),
+                ("shift", C.c_int32), ("dY", C.c_void_p), ("ldy", C.c_int64), ("A", C.c_void_p), ("lda", C.c_int64),
+                ("part_w", C.c_void_p), ("part_b", C.c_void_p)]
+
+
 class WireLayout(C.Structure):
     _fields_ = [(n, C.c_int64) for n in ("record_bytes", "off_state", "off_obs", "off_reward", "off_actions", "off_avail",
                                          "off_flags")]
@@ -107,7 +118,15 @@ _PROTOS = {
     "mal_debug_linear": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
                                    C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
                                    C.c_int32, C.c_void_p]),
-    "mal_agent_param_count": (C.c_int64, [C.c_int32, C.c_int32]),
+    "mal_debug_reduce": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(RedProb), C.POINTER(Batch), C.c_int32,
+                                   C.c_void_p]),
+    "mal_debug_reduce_gru": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int64] +
+                             [C.c_void_p] * 7),
+    "mal_debug_reduce_fc1": (C.c_int, [C.POINTER(Batch), C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                       C.c_void_p, C.c_void_p]),
+    "mal_debug_fc2_grad": (C.c_int, [C.POINTER(Batch), C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                     C.c_void_p]),
+    "mal_agent_param_count":(C.c_int64, [C.c_int32, C.c_int32]),
     "mal_agent_param_count_kind": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
     "mal_dqn_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int64,
                                C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(Select), C.c_void_p]),

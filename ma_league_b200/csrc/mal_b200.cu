@@ -1420,6 +1420,140 @@ static int launch_reduce(RedGroup &g, cudaStream_t st, const char *tag) {
     return 0;
 }
 
+// ---------------------------------------------------------------------------------------------
+// unit-test hooks of the weight-gradient reductions: the learner's own kernel instances, raw per-chunk partials
+// ---------------------------------------------------------------------------------------------
+static int debug_chunks(const char *who, int64_t M, int64_t rows_per_chunk, int *n_chunks) {
+    MAL_REQUIRE(M >= 1 && M < 2147483647LL, "%s: M = %lld must be in [1, 2^31 - 1)", who, (long long)M);
+    MAL_REQUIRE(rows_per_chunk > 0 && rows_per_chunk % RED_MR == 0, "%s: rows_per_chunk %lld must be a positive multiple of %d",
+                who, (long long)rows_per_chunk, RED_MR);
+    *n_chunks = (int)ceil_div64(M, rows_per_chunk);
+    return 0;
+}
+// Dims / BatchView of a batch for the loaders that read it (the mixer and hypernet fields of the config do not matter)
+static int debug_view(const char *who, const mal_batch_t *batch, int32_t agent_input, Dims *d, BatchView *bv) {
+    MAL_REQUIRE(batch, "%s: null batch", who);
+    mal_learner_cfg_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.mixer = MAL_MIXER_VDN; cfg.agent_kind = MAL_AGENT_RNN; cfg.agent_input = agent_input; cfg.returns = MAL_RETURNS_ONE_STEP;
+    if (int rc = get_dims(batch, &cfg, d)) return rc;
+    *bv = make_view(batch, *d);
+    return 0;
+}
+
+extern "C" int mal_debug_reduce(int32_t flavour, int32_t a_kind, int32_t n_probs, const mal_red_prob_t *probs,
+                                const mal_batch_t *batch, int32_t agent_input, void *stream) {
+    const char *who = "mal_debug_reduce";
+    MAL_REQUIRE(flavour >= 0 && flavour <= 4, "%s: flavour %d must be in [0, 4]", who, flavour);
+    MAL_REQUIRE(a_kind == A_DENSE || a_kind == A_STATE || a_kind == A_AGENT_IN, "%s: unknown a_kind %d", who, a_kind);
+    MAL_REQUIRE(probs && n_probs >= 1 && n_probs <= 3, "%s: need 1 to 3 problems", who);
+    RedGroup g;
+    memset(&g, 0, sizeof(g));
+    Dims d;
+    memset(&d, 0, sizeof(d));
+    if (a_kind != A_DENSE) {
+        if (int rc = debug_view(who, batch, agent_input, &d, &g.bv)) return rc;
+        if (a_kind == A_STATE) MAL_REQUIRE(batch->state.ptr, "%s: null state field", who);
+        else MAL_REQUIRE(batch->obs.ptr && (batch->onehot.ptr || d.in.last == 0), "%s: null obs / onehot field", who);
+    }
+    g.n = n_probs;
+    for (int i = 0; i < n_probs; ++i) {
+        const mal_red_prob_t &q = probs[i];
+        int nc;
+        if (int rc = debug_chunks(who, q.M, q.rows_per_chunk, &nc)) return rc;
+        MAL_REQUIRE(q.K >= 1 && q.Nout >= 1 && q.ldy >= q.Nout && q.shift >= 0, "%s: problem %d: bad K / Nout / ldy / shift", who, i);
+        MAL_REQUIRE(q.dY && q.part_w, "%s: problem %d: null dY or part_w", who, i);
+        if (a_kind == A_DENSE) {
+            MAL_REQUIRE(q.A && q.lda >= q.K, "%s: problem %d: null A or lda < K", who, i);
+        } else if (a_kind == A_STATE) {
+            MAL_REQUIRE(q.K <= d.S && q.shift <= d.TT - d.T && q.M <= d.BT, "%s: problem %d: state rows need K <= S, shift <= 1, M <= B*T",
+                        who, i);
+        } else {
+            MAL_REQUIRE(q.K == d.d_in && q.shift == 0 && q.M <= d.M1, "%s: problem %d: agent-input rows need K = d_in, shift 0, M <= TT*B*N",
+                        who, i);
+        }
+        g.p[i] = red(q.M, q.K, q.Nout, q.dY, q.ldy, a_kind, q.shift, q.A, q.lda, q.part_w, q.part_b, nc, q.rows_per_chunk);
+    }
+    // flavour 0: fp32 FFMA k_reduce_group; 1..4: tcgen05 with reduce_mn = flavour - 1 (4: the 512-thread k_reduce_tc3)
+    const int saved_tc = g_use_tc, saved_red = g_reduce_tc, saved_mn = g_reduce_mn;
+    const bool saved_pdl = g_next_pdl;
+    g_use_tc = flavour ? 1 : 0;
+    g_reduce_tc = flavour ? 2 : 0;
+    if (flavour) g_reduce_mn = flavour - 1;
+    g_next_pdl = false;
+    const int rc = launch_reduce(g, (cudaStream_t)stream, "k_reduce_group:debug");
+    g_use_tc = saved_tc; g_reduce_tc = saved_red; g_reduce_mn = saved_mn; g_next_pdl = saved_pdl;
+    return rc;
+}
+
+extern "C" int mal_debug_reduce_gru(const float *x, const float *hout, const float *d_g, int64_t M1, int32_t R,
+                                    int64_t rows_per_chunk, float *wih_w, float *wih_b, float *whh_rz_w, float *whh_rz_b,
+                                    float *whh_n_w, float *whh_n_b, void *stream) {
+    const char *who = "mal_debug_reduce_gru";
+    int nc;
+    if (int rc = debug_chunks(who, M1, rows_per_chunk, &nc)) return rc;
+    MAL_REQUIRE(R >= 1, "%s: R = %d must be >= 1", who, R);
+    MAL_REQUIRE(x && hout && d_g && wih_w && wih_b && whh_rz_w && whh_rz_b && whh_n_w && whh_n_b, "%s: null argument", who);
+    MAL_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(hout) | reinterpret_cast<uintptr_t>(d_g)) & 15) == 0,
+                "%s: x, hout and d_g must be 16-byte aligned", who);
+    ReduceGruArgs ra;
+    ra.x = x; ra.hout = hout; ra.d_g = d_g;
+    ra.wih_w = wih_w; ra.wih_b = wih_b; ra.whha_w = whh_rz_w; ra.whha_b = whh_rz_b; ra.whhb_w = whh_n_w; ra.whhb_b = whh_n_b;
+    ra.M1 = M1; ra.rows_per_chunk = rows_per_chunk; ra.n_chunks = nc; ra.R = R;
+    static size_t attr[MAL_MAX_DEV];
+    if (int rc = ensure_dyn_smem(k_reduce_gru, RG_SMEM_BYTES, attr)) return rc;
+    ++g_stat_reduce_tc;
+    cudaStream_t st = (cudaStream_t)stream;
+    { ProfScope _ps("k_reduce_gru:debug", st); launch_k(k_reduce_gru, dim3(nc), dim3(RT3_THREADS), RG_SMEM_BYTES, st, false, ra); }
+    MAL_LAUNCH_CHECK("k_reduce_gru");
+    return 0;
+}
+
+extern "C" int mal_debug_reduce_fc1(const mal_batch_t *batch, int32_t agent_input, const float *d_x, int64_t M,
+                                    int64_t rows_per_chunk, float *part_w, float *part_b, void *stream) {
+    const char *who = "mal_debug_reduce_fc1";
+    Dims d;
+    BatchView bv;
+    if (int rc = debug_view(who, batch, agent_input, &d, &bv)) return rc;
+    MAL_REQUIRE(d.d_in <= 256, "%s: input width %d > 256 (k_reduce_fc1 covers at most two 128-column halves)", who, d.d_in);
+    int nc;
+    if (int rc = debug_chunks(who, M, rows_per_chunk, &nc)) return rc;
+    MAL_REQUIRE(M <= d.M1, "%s: M = %lld rows > TT*B*N = %lld", who, (long long)M, (long long)d.M1);
+    MAL_REQUIRE(d_x && part_w && part_b && batch->obs.ptr && (batch->onehot.ptr || d.in.last == 0), "%s: null argument", who);
+    MAL_REQUIRE((reinterpret_cast<uintptr_t>(d_x) & 15) == 0, "%s: d_x must be 16-byte aligned", who);
+    ReduceFc1Args fa;
+    fa.d_x = d_x; fa.partW = part_w; fa.partB = part_b;
+    fa.M = M; fa.rows_per_chunk = rows_per_chunk; fa.n_chunks = nc; fa.d_in = d.d_in; fa.bv = bv;
+    static size_t attr[MAL_MAX_DEV];
+    if (int rc = ensure_dyn_smem(k_reduce_fc1, RF_SMEM_BYTES, attr)) return rc;
+    ++g_stat_reduce_fc1;
+    cudaStream_t st = (cudaStream_t)stream;
+    { ProfScope _ps("k_reduce_fc1:debug", st); launch_k(k_reduce_fc1, dim3(nc), dim3(RT3_THREADS), RF_SMEM_BYTES, st, false, fa); }
+    MAL_LAUNCH_CHECK("k_reduce_fc1");
+    return 0;
+}
+
+extern "C" int mal_debug_fc2_grad(const mal_batch_t *batch, const float *d_chosen, const float *hout, int32_t grid,
+                                  float *part_w, float *part_b, void *stream) {
+    const char *who = "mal_debug_fc2_grad";
+    Dims d;
+    BatchView bv;
+    if (int rc = debug_view(who, batch, 0, &d, &bv)) return rc;
+    MAL_REQUIRE(grid >= 1 && grid <= 65535, "%s: grid %d must be in [1, 65535]", who, grid);
+    MAL_REQUIRE(d_chosen && hout && part_w && part_b && batch->actions.ptr, "%s: null argument", who);
+    MAL_REQUIRE((reinterpret_cast<uintptr_t>(hout) & 7) == 0, "%s: hout must be 8-byte aligned", who);
+    Fc2GradArgs a;
+    a.d_chosen = d_chosen; a.actions = batch->actions; a.hout = hout; a.partW = part_w; a.partB = part_b;
+    a.T = d.T; a.N = d.N; a.A = d.A; a.R = d.R; a.rows = (int64_t)d.T * d.R;
+    const size_t smem = sizeof(float) * 8 * ((size_t)d.A * HID + 32);
+    static size_t attr[MAL_MAX_DEV];
+    if (int rc = ensure_dyn_smem(k_fc2_grad, smem, attr)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    { ProfScope _ps("k_fc2_grad:debug", st); k_fc2_grad<<<grid, 256, smem, st>>>(a); }
+    MAL_LAUNCH_CHECK("k_fc2_grad");
+    return 0;
+}
+
 // QMIX hypernet backward from the element-wise seeds d_a2 / d_y1: for two-layer hypernets the layer-2 input gradients
 //   d h1 = (d a1 . W_1.2) * (h1 > 0),  d hf = (d af . W_f.2) * (hf > 0)   (written into the h1 | hf columns of d_y1),
 // then the layer-2 and layer-1 weight-gradient split reductions into per-chunk partials.  Shared by the learner's backward and

@@ -39,8 +39,8 @@ def test_struct_sizes_match_c(nat):
     prog = r'''
     #include <stdio.h>
     #include "mal_b200.h"
-    int main(void) { printf("%zu %zu %zu %zu %zu\n", sizeof(mal_field_t), sizeof(mal_batch_t),
-        sizeof(mal_learner_cfg_t), sizeof(mal_plan_t), sizeof(mal_select_t)); return 0; }'''
+    int main(void) { printf("%zu %zu %zu %zu %zu %zu\n", sizeof(mal_field_t), sizeof(mal_batch_t),
+        sizeof(mal_learner_cfg_t), sizeof(mal_plan_t), sizeof(mal_select_t), sizeof(mal_red_prob_t)); return 0; }'''
     with tempfile.TemporaryDirectory() as d:
         src = os.path.join(d, "s.c")
         open(src, "w").write(prog)
@@ -48,7 +48,7 @@ def test_struct_sizes_match_c(nat):
         subprocess.check_call(["gcc", "-I", os.path.join(ROOT, "include"), src, "-o", exe])
         sizes = [int(x) for x in subprocess.check_output([exe]).split()]
     assert sizes == [C.sizeof(nat.Field), C.sizeof(nat.Batch), C.sizeof(nat.LearnerCfg), C.sizeof(nat.Plan),
-                     C.sizeof(nat.Select)]
+                     C.sizeof(nat.Select), C.sizeof(nat.RedProb)]
 
 
 def test_param_counts_match_survey_table(nat):
