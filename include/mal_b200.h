@@ -84,6 +84,9 @@ typedef struct mal_learner_cfg {
     int32_t agent_input;              /* MAL_IN_* bits (0: obs | last action | agent id); sets d_in and n_agent_params */
     int32_t returns;                  /* MAL_RETURNS_*: the TD targets (0, a zeroed tail: the 1-step target) */
     float td_lambda;                  /* MAL_RETURNS_TD_LAMBDA: lambda in [0, 1] (build_td_lambda_targets, coma_learner.py:10-21) */
+    double target_tau;                /* 0 (a zeroed tail): no soft target update.  tau in (0, 1]: mal_learner_step and
+                                         mal_learner_step_adam blend the target flats toward the updated parameters
+                                         after the optimiser step (see mal_soft_target_t) */
 } mal_learner_cfg_t;
 enum { MAL_AGENT_RNN = 0, MAL_AGENT_DQN = 1 };
 /* MAL_RETURNS_ONE_STEP: targets = r_t + gamma (1 - term_t) tq[t] (q_learner.py:86).
@@ -192,7 +195,8 @@ int mal_peer_allreduce_clip_rmsprop(const void *const *peer_bufs, int32_t world,
                                     float lr, float alpha, float eps, float clip, float *scalars, float *scratch,
                                     int64_t n_frozen, void *stream);
 
-/* forward + backward + clip + RMSprop in one call (the whole of q_learner.py:34-105). */
+/* forward + backward + clip + RMSprop in one call (the whole of q_learner.py:34-105).  With cfg->target_tau > 0 the
+ * step ends with the soft target update below and writes target_agent / target_mixer. */
 int mal_learner_step(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
                      float *agent, const float *target_agent, float *mixer, const float *target_mixer,
                      void *workspace, float *grad, float *square_avg, void *stream);
@@ -225,6 +229,35 @@ int mal_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, 
 int mal_peer_allreduce_clip_adam(const void *const *peer_bufs, int32_t world, float *agent, int64_t n_agent, float *mixer,
                                  int64_t n_mixer, float *grad_out, float *tail_out, int32_t tail, float *adam_state,
                                  const mal_adam_t *adam, float *scalars, float *scratch, int64_t n_frozen, void *stream);
+
+/* Soft target update (EPyMARL's `target_update_interval_or_tau` <= 1), in the optimiser kernel's pass over the
+ * parameters: after the clip + RMSprop / Adam update, for every parameter p of agent | mixer, the frozen prefix included,
+ *     c1 = (float)(1.0 - tau) (subtraction in double) ; c2 = (float)tau
+ *     target[p] = fp32(fp32(target[p] * c1) + fp32(p_new * c2))   (no FMA contraction)
+ * which is `target.data.copy_(target.data * (1.0 - tau) + param.data * tau)` on fp32 tensors; tau = 1 copies.  The target
+ * flats have the layout of the online flats.  The *_soft entries are their namesakes followed by this update; they
+ * reject a tau that is not a finite number in (0, 1] and a missing target buffer (target_mixer may be NULL when
+ * n_mixer = 0). */
+typedef struct mal_soft_target {
+    double tau;
+    float *target_agent;              /* [n_agent] */
+    float *target_mixer;              /* [n_mixer] */
+} mal_soft_target_t;
+int mal_clip_rmsprop_soft(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad,
+                          float *square_avg, float lr, float alpha, float eps, float clip, float *scalars,
+                          float *scratch, const float *denominator, int64_t n_frozen, const mal_soft_target_t *soft,
+                          void *stream);
+int mal_peer_allreduce_clip_rmsprop_soft(const void *const *peer_bufs, int32_t world, float *agent, int64_t n_agent,
+                                         float *mixer, int64_t n_mixer, float *grad_out, float *tail_out, int32_t tail,
+                                         float *square_avg, float lr, float alpha, float eps, float clip, float *scalars,
+                                         float *scratch, int64_t n_frozen, const mal_soft_target_t *soft, void *stream);
+int mal_clip_adam_soft(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad, float *adam_state,
+                       const mal_adam_t *adam, float *scalars, float *scratch, const float *denominator, int64_t n_frozen,
+                       const mal_soft_target_t *soft, void *stream);
+int mal_peer_allreduce_clip_adam_soft(const void *const *peer_bufs, int32_t world, float *agent, int64_t n_agent,
+                                      float *mixer, int64_t n_mixer, float *grad_out, float *tail_out, int32_t tail,
+                                      float *adam_state, const mal_adam_t *adam, float *scalars, float *scratch,
+                                      int64_t n_frozen, const mal_soft_target_t *soft, void *stream);
 
 /* update_targets, q_learner.py:127-131 (load_state_dict of the flat buffers). */
 int mal_copy_f32(float *dst, const float *src, int64_t n, void *stream);

@@ -47,7 +47,8 @@ class LearnerCfg(C.Structure):
     _fields_ = [("mixer", C.c_int32), ("double_q", C.c_int32), ("embed", C.c_int32), ("hyper_embed", C.c_int32),
                 ("gamma", C.c_float), ("lr", C.c_float), ("alpha", C.c_float), ("eps", C.c_float),
                 ("clip", C.c_float), ("save_q", C.c_int32), ("unnormalized", C.c_int32), ("freeze_agent", C.c_int32),
-                ("agent_kind", C.c_int32), ("agent_input", C.c_int32), ("returns", C.c_int32), ("td_lambda", C.c_float)]
+                ("agent_kind", C.c_int32), ("agent_input", C.c_int32), ("returns", C.c_int32), ("td_lambda", C.c_float),
+                ("target_tau", C.c_double)]
 
 
 _PLAN_FIELDS = ["total_bytes", "n_agent_params", "n_mixer_params", "x_on", "x_tg", "gi_on", "gi_tg", "h_on", "h_tg",
@@ -60,6 +61,11 @@ class AdamHyper(C.Structure):
     """mal_adam_t: the hyper-parameters of the Adam step (mal_learner_step_adam, mal_clip_adam)."""
     _fields_ = [("lr", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double),
                 ("weight_decay", C.c_double), ("clip", C.c_float)]
+
+
+class SoftTarget(C.Structure):
+    """mal_soft_target_t: tau and the target flats of the soft target update (the *_soft optimiser entries)."""
+    _fields_ = [("tau", C.c_double), ("target_agent", C.c_void_p), ("target_mixer", C.c_void_p)]
 
 
 def adam_state_floats(n_params: int) -> int:
@@ -152,6 +158,21 @@ _PROTOS = {
     "mal_peer_allreduce_clip_adam": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
                                                C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
                                                C.POINTER(AdamHyper), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "mal_clip_rmsprop_soft": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_float,
+                                        C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                        C.POINTER(SoftTarget), C.c_void_p]),
+    "mal_peer_allreduce_clip_rmsprop_soft": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_void_p, C.c_int64,
+                                                       C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32,
+                                                       C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_float,
+                                                       C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(SoftTarget),
+                                                       C.c_void_p]),
+    "mal_clip_adam_soft": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                     C.POINTER(AdamHyper), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                     C.POINTER(SoftTarget), C.c_void_p]),
+    "mal_peer_allreduce_clip_adam_soft": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
+                                                    C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                                    C.POINTER(AdamHyper), C.c_void_p, C.c_void_p, C.c_int64,
+                                                    C.POINTER(SoftTarget), C.c_void_p]),
     "mal_copy_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "mal_agent_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                  C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -1061,10 +1061,26 @@ __device__ __forceinline__ void clip_coef_prologue(const float *norm_part, int n
     }
 }
 
+// Soft target update of the SOFT optimiser instances: after the step, target = fp32(fp32(target * c1) + fp32(p_new * c2))
+// with c1 = fp32(1 - tau) (subtraction in double), c2 = fp32(tau): `target.data.copy_(target.data * (1.0 - tau) +
+// param.data * tau)` on fp32 tensors.  The target flats have the online flats' layout (agent | mixer).
+struct SoftBlend {
+    float *agent, *mixer;
+    float c1, c2;
+};
+
+__device__ __forceinline__ void soft_blend(const SoftBlend &s, int64_t p, int64_t n_agent, float p_new) {
+    float *t = p < n_agent ? s.agent + p : s.mixer + (p - n_agent);
+    *t = __fadd_rn(__fmul_rn(*t, s.c1), __fmul_rn(p_new, s.c2));   // _rn intrinsics: never contracted into an FMA
+}
+
+// SOFT = false ignores `soft`; SOFT = true also blends every parameter's target, the frozen prefix included (its
+// parameters do not move, so the blend reads them unchanged).
+template <bool SOFT>
 __global__ void __launch_bounds__(256) k_clip_rmsprop(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer,
                                                       float *grad, float *sq, const float *norm_part, int n_part,
                                                       float lr, float alpha, float eps, float clip, float *scalars,
-                                                      const float *denominator, int64_t n_frozen) {
+                                                      const float *denominator, int64_t n_frozen, SoftBlend soft) {
     __shared__ float s_red[8];
     __shared__ float s_coef;
     pdl_wait();
@@ -1072,22 +1088,30 @@ __global__ void __launch_bounds__(256) k_clip_rmsprop(float *agent, int64_t n_ag
     __syncthreads();
     const float coef = s_coef;
     const int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x;
-    if (p >= n_agent + n_mixer || p < n_frozen) return;   // frozen parameters: RMSprop skips them (p.grad is None)
+    if (p >= n_agent + n_mixer) return;
     float *param = p < n_agent ? agent + p : mixer + (p - n_agent);
+    if (p < n_frozen) {                                   // frozen parameters: RMSprop skips them (p.grad is None)
+        if constexpr (SOFT) soft_blend(soft, p, n_agent, *param);
+        return;
+    }
     const float gv = grad[p] * (denominator ? 1.0f / denominator[0] : 1.0f) * coef;
     grad[p] = gv;   // clip_grad_norm_ scales .grad in place
     const float v = alpha * sq[p] + (1.0f - alpha) * gv * gv;
     sq[p] = v;
-    *param = *param - lr * gv / (sqrtf(v) + eps);
+    const float pn = *param - lr * gv / (sqrtf(v) + eps);
+    *param = pn;
+    if constexpr (SOFT) soft_blend(soft, p, n_agent, pn);
 }
 
 // clip_grad_norm_ + torch.optim.Adam.step (amsgrad = False, maximize = False, L2 weight decay added to the gradient),
 // one pass over the flat buffers.  state = exp_avg[P] | exp_avg_sq[P] | step (f32) | ticket (u32).  The step counter
 // lives on the device so that a replayed CUDA graph advances it: every block reads the old step, then takes a ticket;
 // the last block to arrive (all others have read by then) re-arms the ticket and writes step + 1.
+template <bool SOFT>
 __global__ void __launch_bounds__(256) k_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer,
                                                    float *grad, float *state, const float *norm_part, int n_part,
-                                                   mal_adam_t h, float *scalars, const float *denominator, int64_t n_frozen) {
+                                                   mal_adam_t h, float *scalars, const float *denominator, int64_t n_frozen,
+                                                   SoftBlend soft) {
     __shared__ float s_red[8];
     __shared__ float s_coef, s_step_size, s_bc2_sqrt;
     pdl_wait();
@@ -1110,8 +1134,12 @@ __global__ void __launch_bounds__(256) k_clip_adam(float *agent, int64_t n_agent
     __syncthreads();
     const float coef = s_coef, step_size = s_step_size, bc2_sqrt = s_bc2_sqrt;
     const int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x;
-    if (p >= P || p < n_frozen) return;                           // frozen parameters: Adam skips them (p.grad is None)
+    if (p >= P) return;
     float *param = p < n_agent ? agent + p : mixer + (p - n_agent);
+    if (p < n_frozen) {                                           // frozen parameters: Adam skips them (p.grad is None)
+        if constexpr (SOFT) soft_blend(soft, p, n_agent, *param);
+        return;
+    }
     float g = grad[p] * (denominator ? 1.0f / denominator[0] : 1.0f) * coef;
     grad[p] = g;                                                  // clip_grad_norm_ scales .grad in place
     const float pv = *param;
@@ -1121,7 +1149,9 @@ __global__ void __launch_bounds__(256) k_clip_adam(float *agent, int64_t n_agent
     const float vn = v * (float)h.beta2 + (float)(1.0 - h.beta2) * g * g;  // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1 - beta2)
     state[p] = mn;
     state[P + p] = vn;
-    *param = pv + step_size * (mn / (sqrtf(vn) / bc2_sqrt + (float)h.eps));   // addcdiv_(exp_avg, denom, -step_size)
+    const float pn = pv + step_size * (mn / (sqrtf(vn) / bc2_sqrt + (float)h.eps));   // addcdiv_(exp_avg, denom, -step_size)
+    *param = pn;
+    if constexpr (SOFT) soft_blend(soft, p, n_agent, pn);
 }
 
 __global__ void __launch_bounds__(256) k_copy_f32(float *dst, const float *src, int64_t n) {

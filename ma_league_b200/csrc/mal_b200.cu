@@ -610,6 +610,8 @@ static int get_dims(const mal_batch_t *b, const mal_learner_cfg_t *c, Dims *d) {
     MAL_REQUIRE(c->returns == MAL_RETURNS_ONE_STEP || c->returns == MAL_RETURNS_TD_LAMBDA, "returns %d not recognised",
                 c->returns);
     MAL_REQUIRE(c->td_lambda >= 0.0f && c->td_lambda <= 1.0f, "td_lambda must be a number in [0, 1]");   // false for NaN
+    MAL_REQUIRE(c->target_tau == 0.0 || (c->target_tau > 0.0 && c->target_tau <= 1.0),
+                "target_tau must be 0 (no soft target update) or a number in (0, 1]");                // false for NaN
     d->B = b->B; d->TT = b->TT; d->T = b->TT - 1; d->N = b->N; d->A = b->A; d->OBS = b->OBS; d->S = b->S;
     MAL_REQUIRE(c->agent_kind == MAL_AGENT_RNN || c->agent_kind == MAL_AGENT_DQN, "agent kind %d not recognised", c->agent_kind);
     d->kind = c->agent_kind;
@@ -2023,29 +2025,63 @@ extern "C" int mal_mixer_backward(int32_t mixer, int32_t B, int32_t T, int32_t N
     return 0;
 }
 
+// mal_soft_target_t -> the SoftBlend of the SOFT optimiser instances; soft == NULL: no soft update (*out untouched)
+static int soft_blend_of(const char *who, const mal_soft_target_t *soft, int64_t n_mixer, SoftBlend *out) {
+    MAL_REQUIRE(soft, "%s: soft target update missing", who);
+    MAL_REQUIRE(soft->tau > 0.0 && soft->tau <= 1.0, "%s: tau must be a number in (0, 1]", who);   // false for NaN
+    MAL_REQUIRE(soft->target_agent && (n_mixer == 0 || soft->target_mixer), "%s: target buffer missing", who);
+    *out = SoftBlend{soft->target_agent, soft->target_mixer, (float)(1.0 - soft->tau), (float)soft->tau};
+    return 0;
+}
+
 static int launch_clip_rmsprop(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad,
                                float *sq, const float *norm_part, int n_part, float lr, float alpha, float eps,
-                               float clip, float *scalars, const float *denominator, int64_t n_frozen, cudaStream_t st, bool pdl = false) {
+                               float clip, float *scalars, const float *denominator, int64_t n_frozen, cudaStream_t st,
+                               const SoftBlend *soft, bool pdl = false) {
     const int64_t P = n_agent + n_mixer;
-    { ProfScope _ps("k_clip_rmsprop", st); launch_k(k_clip_rmsprop, dim3((unsigned)ceil_div64(P, 256)), dim3(256), 0, st, pdl, agent, n_agent, mixer, n_mixer, grad, sq, norm_part,
-                                                                n_part, lr, alpha, eps, clip, scalars, denominator, n_frozen); }
+    const dim3 grid((unsigned)ceil_div64(P, 256));
+    if (soft) {
+        { ProfScope _ps("k_clip_rmsprop_soft", st); launch_k(k_clip_rmsprop<true>, grid, dim3(256), 0, st, pdl, agent, n_agent, mixer, n_mixer, grad, sq, norm_part,
+                                                                         n_part, lr, alpha, eps, clip, scalars, denominator, n_frozen, *soft); }
+        MAL_LAUNCH_CHECK("k_clip_rmsprop_soft");
+        return 0;
+    }
+    { ProfScope _ps("k_clip_rmsprop", st); launch_k(k_clip_rmsprop<false>, grid, dim3(256), 0, st, pdl, agent, n_agent, mixer, n_mixer, grad, sq, norm_part,
+                                                                n_part, lr, alpha, eps, clip, scalars, denominator, n_frozen, SoftBlend{}); }
     MAL_LAUNCH_CHECK("k_clip_rmsprop");
     return 0;
 }
 
-extern "C" int mal_clip_rmsprop(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad,
-                                float *square_avg, float lr, float alpha, float eps, float clip, float *scalars,
-                                float *scratch, const float *denominator, int64_t n_frozen, void *stream) {
+static int clip_rmsprop(const char *who, float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad,
+                        float *square_avg, float lr, float alpha, float eps, float clip, float *scalars,
+                        float *scratch, const float *denominator, int64_t n_frozen, const SoftBlend *soft, void *stream) {
     MAL_REQUIRE(agent && grad && square_avg && scalars && scratch && n_agent > 0 && n_mixer >= 0,
-                "mal_clip_rmsprop: bad arguments (scratch needs ceil(P/256) floats)");
-    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "mal_clip_rmsprop: n_frozen out of range");
-    MAL_REQUIRE(n_mixer == 0 || mixer, "mal_clip_rmsprop: mixer buffer missing");
+                "%s: bad arguments (scratch needs ceil(P/256) floats)", who);
+    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "%s: n_frozen out of range", who);
+    MAL_REQUIRE(n_mixer == 0 || mixer, "%s: mixer buffer missing", who);
     const int64_t P = n_agent + n_mixer;
     const int nb = (int)ceil_div64(P, 256);
     { ProfScope _ps("k_sumsq", (cudaStream_t)stream); k_sumsq<<<nb, 256, 0, (cudaStream_t)stream>>>(grad, P, scratch, denominator, n_frozen); }
     MAL_LAUNCH_CHECK("k_sumsq");
     return launch_clip_rmsprop(agent, n_agent, mixer, n_mixer, grad, square_avg, scratch, nb, lr, alpha, eps, clip,
-                               scalars, denominator, n_frozen, (cudaStream_t)stream);
+                               scalars, denominator, n_frozen, (cudaStream_t)stream, soft);
+}
+
+extern "C" int mal_clip_rmsprop(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad,
+                                float *square_avg, float lr, float alpha, float eps, float clip, float *scalars,
+                                float *scratch, const float *denominator, int64_t n_frozen, void *stream) {
+    return clip_rmsprop("mal_clip_rmsprop", agent, n_agent, mixer, n_mixer, grad, square_avg, lr, alpha, eps, clip,
+                        scalars, scratch, denominator, n_frozen, nullptr, stream);
+}
+
+extern "C" int mal_clip_rmsprop_soft(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad,
+                                     float *square_avg, float lr, float alpha, float eps, float clip, float *scalars,
+                                     float *scratch, const float *denominator, int64_t n_frozen,
+                                     const mal_soft_target_t *soft, void *stream) {
+    SoftBlend sb;
+    if (int rc = soft_blend_of("mal_clip_rmsprop_soft", soft, n_mixer, &sb)) return rc;
+    return clip_rmsprop("mal_clip_rmsprop_soft", agent, n_agent, mixer, n_mixer, grad, square_avg, lr, alpha, eps, clip,
+                        scalars, scratch, denominator, n_frozen, &sb, stream);
 }
 
 // k_peer_allreduce_grad: rank-order sum of the peers' un-normalised halves into grad_out / tail_out, and the norm partials
@@ -2064,28 +2100,58 @@ static int peer_allreduce(const char *who, const void *const *peer_bufs, int32_t
     return 0;
 }
 
+static int peer_allreduce_clip_rmsprop(const char *who, const void *const *peer_bufs, int32_t world, float *agent,
+                                       int64_t n_agent, float *mixer, int64_t n_mixer, float *grad_out, float *tail_out,
+                                       int32_t tail, float *square_avg, float lr, float alpha, float eps, float clip,
+                                       float *scalars, float *scratch, int64_t n_frozen, const SoftBlend *soft,
+                                       void *stream) {
+    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "%s: n_frozen out of range", who);
+    MAL_REQUIRE(peer_bufs && world >= 1 && world <= PEER_MAX, "%s: world size must be in [1, %d]", who, PEER_MAX);
+    MAL_REQUIRE(agent && grad_out && tail_out && square_avg && scalars && scratch && n_agent > 0 && n_mixer >= 0 && tail >= 5 && tail <= 32,
+                "%s: bad arguments (scratch needs ceil(P/256) floats, tail >= 5)", who);
+    const int64_t P = n_agent + n_mixer;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = peer_allreduce(who, peer_bufs, world, P, grad_out, tail_out, tail, scratch, n_frozen, st)) return rc;
+    return launch_clip_rmsprop(agent, n_agent, mixer, n_mixer, grad_out, square_avg, scratch, (int)ceil_div64(P, 256), lr, alpha, eps, clip,
+                               scalars, nullptr, n_frozen, st, soft);
+}
+
 extern "C" int mal_peer_allreduce_clip_rmsprop(const void *const *peer_bufs, int32_t world, float *agent, int64_t n_agent,
                                                float *mixer, int64_t n_mixer, float *grad_out, float *tail_out, int32_t tail,
                                                float *square_avg, float lr, float alpha, float eps, float clip,
                                                float *scalars, float *scratch, int64_t n_frozen, void *stream) {
-    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "mal_peer_allreduce_clip_rmsprop: n_frozen out of range");
-    MAL_REQUIRE(peer_bufs && world >= 1 && world <= PEER_MAX, "mal_peer_allreduce_clip_rmsprop: world size must be in [1, %d]", PEER_MAX);
-    MAL_REQUIRE(agent && grad_out && tail_out && square_avg && scalars && scratch && n_agent > 0 && n_mixer >= 0 && tail >= 5 && tail <= 32,
-                "mal_peer_allreduce_clip_rmsprop: bad arguments (scratch needs ceil(P/256) floats, tail >= 5)");
-    const int64_t P = n_agent + n_mixer;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (int rc = peer_allreduce("mal_peer_allreduce_clip_rmsprop", peer_bufs, world, P, grad_out, tail_out, tail, scratch, n_frozen, st)) return rc;
-    return launch_clip_rmsprop(agent, n_agent, mixer, n_mixer, grad_out, square_avg, scratch, (int)ceil_div64(P, 256), lr, alpha, eps, clip,
-                               scalars, nullptr, n_frozen, st);
+    return peer_allreduce_clip_rmsprop("mal_peer_allreduce_clip_rmsprop", peer_bufs, world, agent, n_agent, mixer, n_mixer,
+                                       grad_out, tail_out, tail, square_avg, lr, alpha, eps, clip, scalars, scratch,
+                                       n_frozen, nullptr, stream);
+}
+
+extern "C" int mal_peer_allreduce_clip_rmsprop_soft(const void *const *peer_bufs, int32_t world, float *agent,
+                                                    int64_t n_agent, float *mixer, int64_t n_mixer, float *grad_out,
+                                                    float *tail_out, int32_t tail, float *square_avg, float lr,
+                                                    float alpha, float eps, float clip, float *scalars, float *scratch,
+                                                    int64_t n_frozen, const mal_soft_target_t *soft, void *stream) {
+    SoftBlend sb;
+    if (int rc = soft_blend_of("mal_peer_allreduce_clip_rmsprop_soft", soft, n_mixer, &sb)) return rc;
+    return peer_allreduce_clip_rmsprop("mal_peer_allreduce_clip_rmsprop_soft", peer_bufs, world, agent, n_agent, mixer,
+                                       n_mixer, grad_out, tail_out, tail, square_avg, lr, alpha, eps, clip, scalars,
+                                       scratch, n_frozen, &sb, stream);
 }
 
 // forward + backward of the fused step (mal_learner_step, mal_learner_step_adam); *norm_part / *n_part / *scalars are
-// the inputs of the optimiser kernel's clip prologue
+// the inputs of the optimiser kernel's clip prologue, *soft the soft target update of cfg->target_tau (*use_soft = false
+// when target_tau is 0)
 static int learner_step_fwd_bwd(const mal_batch_t *batch, const mal_learner_cfg_t *cfg, const mal_plan_t *plan,
                                 float *agent, const float *target_agent, float *mixer, const float *target_mixer,
                                 void *workspace, float *grad, void *stream, const float **norm_part, int *n_part,
-                                float **scalars) {
+                                float **scalars, SoftBlend *soft, bool *use_soft) {
     MAL_REQUIRE(!cfg || !cfg->unnormalized, "mal_learner_step: unnormalized (data-parallel) mode needs the split calls");
+    *use_soft = cfg && cfg->target_tau > 0.0;     // a target_tau out of range is rejected by the forward's checks
+    if (*use_soft) {
+        // the forward reads the targets; the optimiser kernel, last on the stream, rewrites them
+        MAL_REQUIRE(plan, "mal_learner_step: null plan");
+        const mal_soft_target_t st{cfg->target_tau, const_cast<float *>(target_agent), const_cast<float *>(target_mixer)};
+        if (int rc = soft_blend_of("mal_learner_step", &st, plan->n_mixer_params, soft)) return rc;
+    }
     g_defer_stats = true;
     const int rc_f = mal_learner_forward(batch, cfg, plan, agent, target_agent, mixer, target_mixer, workspace, stream);
     g_defer_stats = false;
@@ -2113,11 +2179,14 @@ extern "C" int mal_learner_step(const mal_batch_t *batch, const mal_learner_cfg_
     const float *norm_part;
     int n_part;
     float *scalars;
+    SoftBlend soft;
+    bool use_soft;
     if (int rc = learner_step_fwd_bwd(batch, cfg, plan, agent, target_agent, mixer, target_mixer, workspace, grad, stream,
-                                      &norm_part, &n_part, &scalars)) return rc;
+                                      &norm_part, &n_part, &scalars, &soft, &use_soft)) return rc;
     return launch_clip_rmsprop(agent, plan->n_agent_params, mixer, plan->n_mixer_params, grad, square_avg,
                                norm_part, n_part, cfg->lr, cfg->alpha, cfg->eps, cfg->clip, scalars,
-                               nullptr, cfg->freeze_agent ? plan->n_agent_params : 0, (cudaStream_t)stream, true);   // stream predecessor: k_grad_reduce
+                               nullptr, cfg->freeze_agent ? plan->n_agent_params : 0, (cudaStream_t)stream,
+                               use_soft ? &soft : nullptr, true);   // stream predecessor: k_grad_reduce
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2134,10 +2203,18 @@ static int check_adam(const char *who, const mal_adam_t *h, const float *state) 
 
 static int launch_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad, float *state,
                             const float *norm_part, int n_part, const mal_adam_t &h, float *scalars,
-                            const float *denominator, int64_t n_frozen, cudaStream_t st, bool pdl = false) {
+                            const float *denominator, int64_t n_frozen, cudaStream_t st, const SoftBlend *soft,
+                            bool pdl = false) {
     const int64_t P = n_agent + n_mixer;
-    { ProfScope _ps("k_clip_adam", st); launch_k(k_clip_adam, dim3((unsigned)ceil_div64(P, 256)), dim3(256), 0, st, pdl, agent, n_agent, mixer, n_mixer, grad, state,
-                                                             norm_part, n_part, h, scalars, denominator, n_frozen); }
+    const dim3 grid((unsigned)ceil_div64(P, 256));
+    if (soft) {
+        { ProfScope _ps("k_clip_adam_soft", st); launch_k(k_clip_adam<true>, grid, dim3(256), 0, st, pdl, agent, n_agent, mixer, n_mixer, grad, state,
+                                                                      norm_part, n_part, h, scalars, denominator, n_frozen, *soft); }
+        MAL_LAUNCH_CHECK("k_clip_adam_soft");
+        return 0;
+    }
+    { ProfScope _ps("k_clip_adam", st); launch_k(k_clip_adam<false>, grid, dim3(256), 0, st, pdl, agent, n_agent, mixer, n_mixer, grad, state,
+                                                             norm_part, n_part, h, scalars, denominator, n_frozen, SoftBlend{}); }
     MAL_LAUNCH_CHECK("k_clip_adam");
     return 0;
 }
@@ -2149,43 +2226,83 @@ extern "C" int mal_learner_step_adam(const mal_batch_t *batch, const mal_learner
     const float *norm_part;
     int n_part;
     float *scalars;
+    SoftBlend soft;
+    bool use_soft;
     if (int rc = learner_step_fwd_bwd(batch, cfg, plan, agent, target_agent, mixer, target_mixer, workspace, grad, stream,
-                                      &norm_part, &n_part, &scalars)) return rc;
+                                      &norm_part, &n_part, &scalars, &soft, &use_soft)) return rc;
     return launch_clip_adam(agent, plan->n_agent_params, mixer, plan->n_mixer_params, grad, adam_state, norm_part, n_part,
                             *adam, scalars, nullptr, cfg->freeze_agent ? plan->n_agent_params : 0, (cudaStream_t)stream,
-                            true);   // stream predecessor: k_grad_reduce
+                            use_soft ? &soft : nullptr, true);   // stream predecessor: k_grad_reduce
 }
 
-extern "C" int mal_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad, float *adam_state,
-                             const mal_adam_t *adam, float *scalars, float *scratch, const float *denominator,
-                             int64_t n_frozen, void *stream) {
-    if (int rc = check_adam("mal_clip_adam", adam, adam_state)) return rc;
+static int clip_adam(const char *who, float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad,
+                     float *adam_state, const mal_adam_t *adam, float *scalars, float *scratch, const float *denominator,
+                     int64_t n_frozen, const SoftBlend *soft, void *stream) {
+    if (int rc = check_adam(who, adam, adam_state)) return rc;
     MAL_REQUIRE(agent && grad && scalars && scratch && n_agent > 0 && n_mixer >= 0,
-                "mal_clip_adam: bad arguments (scratch needs ceil(P/256) floats)");
-    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "mal_clip_adam: n_frozen out of range");
-    MAL_REQUIRE(n_mixer == 0 || mixer, "mal_clip_adam: mixer buffer missing");
+                "%s: bad arguments (scratch needs ceil(P/256) floats)", who);
+    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "%s: n_frozen out of range", who);
+    MAL_REQUIRE(n_mixer == 0 || mixer, "%s: mixer buffer missing", who);
     const int64_t P = n_agent + n_mixer;
     const int nb = (int)ceil_div64(P, 256);
     { ProfScope _ps("k_sumsq", (cudaStream_t)stream); k_sumsq<<<nb, 256, 0, (cudaStream_t)stream>>>(grad, P, scratch, denominator, n_frozen); }
     MAL_LAUNCH_CHECK("k_sumsq");
     return launch_clip_adam(agent, n_agent, mixer, n_mixer, grad, adam_state, scratch, nb, *adam, scalars, denominator,
-                            n_frozen, (cudaStream_t)stream);
+                            n_frozen, (cudaStream_t)stream, soft);
+}
+
+extern "C" int mal_clip_adam(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad, float *adam_state,
+                             const mal_adam_t *adam, float *scalars, float *scratch, const float *denominator,
+                             int64_t n_frozen, void *stream) {
+    return clip_adam("mal_clip_adam", agent, n_agent, mixer, n_mixer, grad, adam_state, adam, scalars, scratch,
+                     denominator, n_frozen, nullptr, stream);
+}
+
+extern "C" int mal_clip_adam_soft(float *agent, int64_t n_agent, float *mixer, int64_t n_mixer, float *grad,
+                                  float *adam_state, const mal_adam_t *adam, float *scalars, float *scratch,
+                                  const float *denominator, int64_t n_frozen, const mal_soft_target_t *soft,
+                                  void *stream) {
+    SoftBlend sb;
+    if (int rc = soft_blend_of("mal_clip_adam_soft", soft, n_mixer, &sb)) return rc;
+    return clip_adam("mal_clip_adam_soft", agent, n_agent, mixer, n_mixer, grad, adam_state, adam, scalars, scratch,
+                     denominator, n_frozen, &sb, stream);
+}
+
+static int peer_allreduce_clip_adam(const char *who, const void *const *peer_bufs, int32_t world, float *agent,
+                                    int64_t n_agent, float *mixer, int64_t n_mixer, float *grad_out, float *tail_out,
+                                    int32_t tail, float *adam_state, const mal_adam_t *adam, float *scalars,
+                                    float *scratch, int64_t n_frozen, const SoftBlend *soft, void *stream) {
+    if (int rc = check_adam(who, adam, adam_state)) return rc;
+    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "%s: n_frozen out of range", who);
+    MAL_REQUIRE(agent && grad_out && tail_out && scalars && scratch && n_agent > 0 && n_mixer >= 0 && tail >= 5 && tail <= 32,
+                "%s: bad arguments (scratch needs ceil(P/256) floats, tail >= 5)", who);
+    MAL_REQUIRE(n_mixer == 0 || mixer, "%s: mixer buffer missing", who);
+    const int64_t P = n_agent + n_mixer;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = peer_allreduce(who, peer_bufs, world, P, grad_out, tail_out, tail, scratch, n_frozen, st)) return rc;
+    return launch_clip_adam(agent, n_agent, mixer, n_mixer, grad_out, adam_state, scratch, (int)ceil_div64(P, 256), *adam,
+                            scalars, nullptr, n_frozen, st, soft);
 }
 
 extern "C" int mal_peer_allreduce_clip_adam(const void *const *peer_bufs, int32_t world, float *agent, int64_t n_agent,
                                             float *mixer, int64_t n_mixer, float *grad_out, float *tail_out, int32_t tail,
                                             float *adam_state, const mal_adam_t *adam, float *scalars, float *scratch,
                                             int64_t n_frozen, void *stream) {
-    if (int rc = check_adam("mal_peer_allreduce_clip_adam", adam, adam_state)) return rc;
-    MAL_REQUIRE(n_frozen >= 0 && n_frozen <= n_agent + n_mixer, "mal_peer_allreduce_clip_adam: n_frozen out of range");
-    MAL_REQUIRE(agent && grad_out && tail_out && scalars && scratch && n_agent > 0 && n_mixer >= 0 && tail >= 5 && tail <= 32,
-                "mal_peer_allreduce_clip_adam: bad arguments (scratch needs ceil(P/256) floats, tail >= 5)");
-    MAL_REQUIRE(n_mixer == 0 || mixer, "mal_peer_allreduce_clip_adam: mixer buffer missing");
-    const int64_t P = n_agent + n_mixer;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (int rc = peer_allreduce("mal_peer_allreduce_clip_adam", peer_bufs, world, P, grad_out, tail_out, tail, scratch, n_frozen, st)) return rc;
-    return launch_clip_adam(agent, n_agent, mixer, n_mixer, grad_out, adam_state, scratch, (int)ceil_div64(P, 256), *adam,
-                            scalars, nullptr, n_frozen, st);
+    return peer_allreduce_clip_adam("mal_peer_allreduce_clip_adam", peer_bufs, world, agent, n_agent, mixer, n_mixer,
+                                    grad_out, tail_out, tail, adam_state, adam, scalars, scratch, n_frozen, nullptr,
+                                    stream);
+}
+
+extern "C" int mal_peer_allreduce_clip_adam_soft(const void *const *peer_bufs, int32_t world, float *agent,
+                                                 int64_t n_agent, float *mixer, int64_t n_mixer, float *grad_out,
+                                                 float *tail_out, int32_t tail, float *adam_state,
+                                                 const mal_adam_t *adam, float *scalars, float *scratch,
+                                                 int64_t n_frozen, const mal_soft_target_t *soft, void *stream) {
+    SoftBlend sb;
+    if (int rc = soft_blend_of("mal_peer_allreduce_clip_adam_soft", soft, n_mixer, &sb)) return rc;
+    return peer_allreduce_clip_adam("mal_peer_allreduce_clip_adam_soft", peer_bufs, world, agent, n_agent, mixer,
+                                    n_mixer, grad_out, tail_out, tail, adam_state, adam, scalars, scratch, n_frozen,
+                                    &sb, stream);
 }
 
 extern "C" int mal_copy_f32(float *dst, const float *src, int64_t n, void *stream) {

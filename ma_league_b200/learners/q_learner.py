@@ -6,9 +6,11 @@ double-Q target max, mixers, TD loss, full backward (mixer + BPTT), clip_grad_no
 `args.optimizer: "adam"` (`mal_learner_step_adam`).  The TD targets are
 the 1-step targets of q_learner.py:86, or lambda-returns when `args.td_lambda` is a number in [0, 1] (INTEGRATION.md).  Nothing is read
 back to the host except on log steps (the reference syncs every step through `.item()`, q_learner.py:113).
+`args.target_update_interval_or_tau` (EPyMARL) <= 1 blends the target networks softly inside the optimiser kernel.
 """
 import copy
 import ctypes as C
+import math
 import numbers
 
 import torch as th
@@ -95,7 +97,7 @@ class QLearner(Learner):
                               a.grad_norm_clip, int(self.save_q), int(self._dp_world() > 1), int(self._agent_frozen()),
                               getattr(self.mac.agent, "mal_kind", nat.AGENT_RNN),
                               nat.agent_input_flags(getattr(a, "obs_last_action", True), getattr(a, "obs_agent_id", True)),
-                              *self._returns())
+                              *self._returns(), self._target_update()[2])
 
     def _returns(self):
         """(mal_learner_cfg_t.returns, td_lambda) from `args.td_lambda`: absent or None is the 1-step target of
@@ -106,6 +108,21 @@ class QLearner(Learner):
         if isinstance(lam, bool) or not isinstance(lam, numbers.Real) or not 0.0 <= float(lam) <= 1.0:
             raise nat.MalError("args.td_lambda must be None or a number in [0, 1], got %r" % (lam,))
         return nat.RETURNS_TD_LAMBDA, float(lam)
+
+    def _target_update(self):
+        """(mode, interval, tau) from EPyMARL's `args.target_update_interval_or_tau`:
+        - absent or None: ("hard", None, 0.0), hard copies every `args.target_update_interval` episodes
+          (the reference rule; the interval is read where train() checks it, as the reference reads it);
+        - a number > 1: ("hard", that number, 0.0), the same rule with this interval;
+        - tau in (0, 1]: ("soft", None, tau), target = (1 - tau) target + tau param after every optimiser step, in the
+          optimiser kernel (mal_learner_cfg_t.target_tau, the *_soft entries), and no hard copy."""
+        v = getattr(self.args, "target_update_interval_or_tau", None)
+        if v is None:
+            return "hard", None, 0.0
+        if isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(v) or not v > 0:
+            raise nat.MalError("args.target_update_interval_or_tau must be None, an interval > 1 or a tau in (0, 1], "
+                               "got %r" % (v,))
+        return ("hard", v, 0.0) if v > 1 else ("soft", None, float(v))
 
     def _agent_frozen(self):
         """`freeze_agent_weights()` (multi_agent_controller.py:74-76, `args.freeze_native`): in the reference a frozen
@@ -236,9 +253,13 @@ class QLearner(Learner):
             if p.grad is not g:
                 p.grad = g
 
-        if (episode_num - self.last_target_update_episode) / self.args.target_update_interval >= 1.0:
-            self.update_targets()
-            self.last_target_update_episode = episode_num
+        mode, interval, _ = self._target_update()
+        if mode == "hard":
+            if interval is None:
+                interval = self.args.target_update_interval
+            if (episode_num - self.last_target_update_episode) / interval >= 1.0:
+                self.update_targets()
+                self.last_target_update_episode = episode_num
 
         sc = self.scalars()
         if dp:
@@ -361,22 +382,36 @@ class QLearner(Learner):
         denom = self._grad_store[n_total + 4:]            # global mask.sum()
         a = self.args
         n_frozen = self._plan.n_agent_params if cfg.freeze_agent else 0
+        soft = self._soft_target(cfg, f)
         with nat.on_device(dev):
             if adam is not None:
-                nat.check(lib.mal_clip_adam(nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
-                                            self._plan.n_mixer_params, nat.ptr(self._grad),
-                                            nat.ptr(self.optimiser.flat_state), C.byref(adam), nat.ptr(self.scalars()),
-                                            nat.ptr(self._dp_scratch), nat.ptr(denom), n_frozen, st), "mal_clip_adam")
+                args = (nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]), self._plan.n_mixer_params,
+                        nat.ptr(self._grad), nat.ptr(self.optimiser.flat_state), C.byref(adam), nat.ptr(self.scalars()),
+                        nat.ptr(self._dp_scratch), nat.ptr(denom), n_frozen)
+                if soft is None:
+                    nat.check(lib.mal_clip_adam(*args, st), "mal_clip_adam")
+                else:
+                    nat.check(lib.mal_clip_adam_soft(*args, C.byref(soft), st), "mal_clip_adam_soft")
             else:
-                nat.check(lib.mal_clip_rmsprop(nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
-                                               self._plan.n_mixer_params, nat.ptr(self._grad),
-                                               nat.ptr(self.optimiser.flat_sq), a.lr, a.optim_alpha, a.optim_eps,
-                                               a.grad_norm_clip, nat.ptr(self.scalars()), nat.ptr(self._dp_scratch),
-                                               nat.ptr(denom), n_frozen, st), "mal_clip_rmsprop")
+                args = (nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]), self._plan.n_mixer_params,
+                        nat.ptr(self._grad), nat.ptr(self.optimiser.flat_sq), a.lr, a.optim_alpha, a.optim_eps,
+                        a.grad_norm_clip, nat.ptr(self.scalars()), nat.ptr(self._dp_scratch), nat.ptr(denom), n_frozen)
+                if soft is None:
+                    nat.check(lib.mal_clip_rmsprop(*args, st), "mal_clip_rmsprop")
+                else:
+                    nat.check(lib.mal_clip_rmsprop_soft(*args, C.byref(soft), st), "mal_clip_rmsprop_soft")
         if self.dp_profile is not None:
             ev1 = th.cuda.Event(enable_timing=True)
             ev1.record()
             self.dp_profile.append((ev0, ev1))
+
+    @staticmethod
+    def _soft_target(cfg, f):
+        """The mal_soft_target_t of the data-parallel optimiser entries, or None without a soft target update (the
+        single-process step reads tau from the cfg)."""
+        if cfg.target_tau == 0.0:
+            return None
+        return nat.SoftTarget(cfg.target_tau, nat.ptr(f["tagent"]), nat.ptr(f["tmixer"]))
 
     # ---- fused exchange: peer-memory all-reduce inside the optimiser prologue (no NCCL call on the path)
     def _dp_symmetric(self, n_total, dev):
@@ -428,19 +463,26 @@ class QLearner(Learner):
         hdl.barrier(channel=0)                           # every rank's half h is complete (and half h^1 is free again)
         a = self.args
         n_frozen = self._plan.n_agent_params if cfg.freeze_agent else 0
+        soft = self._soft_target(cfg, f)
+        head = (ptrs[h], hdl.world_size, nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
+                self._plan.n_mixer_params, nat.ptr(self._grad), nat.ptr(self._grad_store[n_total:]), DP_TAIL)
         with nat.on_device(dev):
             if adam is not None:
-                nat.check(lib.mal_peer_allreduce_clip_adam(
-                    ptrs[h], hdl.world_size, nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
-                    self._plan.n_mixer_params, nat.ptr(self._grad), nat.ptr(self._grad_store[n_total:]), DP_TAIL,
-                    nat.ptr(self.optimiser.flat_state), C.byref(adam), nat.ptr(self.scalars()), nat.ptr(self._dp_scratch),
-                    n_frozen, st), "mal_peer_allreduce_clip_adam")
+                args = head + (nat.ptr(self.optimiser.flat_state), C.byref(adam), nat.ptr(self.scalars()),
+                               nat.ptr(self._dp_scratch), n_frozen)
+                if soft is None:
+                    nat.check(lib.mal_peer_allreduce_clip_adam(*args, st), "mal_peer_allreduce_clip_adam")
+                else:
+                    nat.check(lib.mal_peer_allreduce_clip_adam_soft(*args, C.byref(soft), st),
+                              "mal_peer_allreduce_clip_adam_soft")
             else:
-                nat.check(lib.mal_peer_allreduce_clip_rmsprop(
-                    ptrs[h], hdl.world_size, nat.ptr(f["agent"]), self._plan.n_agent_params, nat.ptr(f["mixer"]),
-                    self._plan.n_mixer_params, nat.ptr(self._grad), nat.ptr(self._grad_store[n_total:]), DP_TAIL,
-                    nat.ptr(self.optimiser.flat_sq), a.lr, a.optim_alpha, a.optim_eps, a.grad_norm_clip,
-                    nat.ptr(self.scalars()), nat.ptr(self._dp_scratch), n_frozen, st), "mal_peer_allreduce_clip_rmsprop")
+                args = head + (nat.ptr(self.optimiser.flat_sq), a.lr, a.optim_alpha, a.optim_eps, a.grad_norm_clip,
+                               nat.ptr(self.scalars()), nat.ptr(self._dp_scratch), n_frozen)
+                if soft is None:
+                    nat.check(lib.mal_peer_allreduce_clip_rmsprop(*args, st), "mal_peer_allreduce_clip_rmsprop")
+                else:
+                    nat.check(lib.mal_peer_allreduce_clip_rmsprop_soft(*args, C.byref(soft), st),
+                              "mal_peer_allreduce_clip_rmsprop_soft")
         if self.dp_profile is not None:
             ev1 = th.cuda.Event(enable_timing=True)
             ev1.record()
@@ -541,7 +583,8 @@ class QLearner(Learner):
         return out
 
     def update_targets(self):
-        """q_learner.py:127-131: online -> target copy (one flat device copy per network)."""
+        """q_learner.py:127-131: online -> target copy (one flat device copy per network).  train() calls it in hard
+        mode; with a soft `target_update_interval_or_tau` it is only the public hard copy."""
         pairs = [(ensure_flat(self.target_mac.agent), ensure_flat(self.mac.agent))]
         if self.mixer is not None:
             pairs.append((ensure_flat(self.target_mixer), ensure_flat(self.mixer)))
